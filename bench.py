@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- the five BASELINE.json configs through the C ABI of libeg_b200.so; config 2 is the headline and the default.
 
-    python bench.py [--config C] --gpus N --steps K --warmup W          (N > 1: launched under torchrun by the driver)
+    python bench.py [--config C] --gpus N --steps K --warmup W [--dump-outputs DIR]     (N > 1: launched under torchrun)
     python bench.py [--config C] --impl reference --gpus N --steps K --warmup W     (the CPU restatement of the same path)
 
     C = 1  encrypt_bool + RingProof verify of 10 000 Boolean ciphertexts (benches/basics.rs:60-82 shape; latency-bound at
@@ -22,7 +22,9 @@ the 128-byte NCCL id and the barriers of the timing protocol.  `--scaling strong
 
 Synthetic data: `--unique` distinct items are produced by the oracle's prover from the seeded ChaCha streams of SURVEY.md
 8(d) (1 % tampered with the reference's tamper patterns) and tiled to the batch size; cost does not depend on contents
-(uniform control flow); every timed batch's verdicts / tallies / values are checked against the oracle's.
+(uniform control flow); every timed batch's verdicts / tallies / values are checked against the oracle's.  With the same
+arguments the inputs are the same from run to run: `--dump-outputs DIR` writes what the last timed step returned as
+DIR/<name>.npy, so that two builds of the library can be compared output for output.
 """
 import argparse
 import json
@@ -31,6 +33,7 @@ import pathlib
 import random
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -64,7 +67,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ring-mode", type=int, default=-1, choices=[-1, 0, 1, 2, 3], help="-1: per config (2 = k_ring for the large batches)")
     ap.add_argument("--chunk", type=int, default=0, help="items per internal chunk (0 = library default)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 arm: the reference arm times the oracle on samples it does not keep")
+    return args
 
 
 # =============================================================================== workloads
@@ -90,6 +100,7 @@ class Workload:
     executed_field_ops_per_task = None
     has_tally = False
     options = 0
+    output_names = ("verdicts",)
 
     def make(self, unique, threads):      # -> None; fills self.inputs (list of unique arrays) and expectations
         raise NotImplementedError
@@ -97,7 +108,7 @@ class Workload:
     def setup(self, e):
         pass
 
-    def outputs(self, n):                 # [(shape, numpy dtype)]
+    def outputs(self, n):                 # [(shape, numpy dtype)], in the order of output_names
         raise NotImplementedError
 
     def step_dev(self, e, n, d_in, d_out):
@@ -168,6 +179,7 @@ class Choice(Workload):
     bytes_per_item = 5 * 64 + 11 * 32 + 64         # 736, SURVEY.md 8(a) a12
     ref_field_ops_per_item = 4956 * 11 + 280 * (34 + 10)      # 66 836
     has_tally = True
+    output_names = ("verdicts", "tally")
     # what k_ring executes per equation side of a two-equation ring (DESIGN.md 5): 2 x 1603 table build + 4 sides x (435 + 497
     # + 112) + 112 for [e a]G + 304 for encoding the first equation's pair
     executed_field_ops_per_task = (2 * 1603 + 4 * (435 + 497 + FIXED_TERM_OPS) + FIXED_TERM_OPS + 304) / 4
@@ -226,6 +238,7 @@ class Qv(Workload):
     options = 5
     ref_field_ops_per_item = 256e3
     has_tally = True
+    output_names = ("verdicts", "tally")
 
     def make(self, unique, threads):
         import numpy as np
@@ -346,6 +359,7 @@ class Shares(Workload):
     ref_field_ops_per_item = 27e3
     kernel = "k_msm"
     kernel_kind = 2
+    output_names = ("share_verdicts", "values", "found")
     # k_msm tasks per tally: 6 equation sides (3 shares x 2) + one 3-term recombination
     field_ops_per_task = (6 * FIELD_OPS_PER_SIDE + FIELD_OPS_3TERM_SUM) / 7
     USED = (0, 2, 4)
@@ -477,10 +491,12 @@ def int32_peak():
     """Measured INT32 multiply-add issue rate (lane-ops / s) of this GPU: tools/microbench/int_pipe_bench."""
     exe = ROOT / "tools" / "microbench" / "int_pipe_bench"
     try:
-        if not exe.exists():      # built by __graft_entry__.build(); rebuilt here if the binary did not travel
-            subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-o", str(exe),
-                            str(exe) + ".cu"], check=True, timeout=600)
-        out = subprocess.run([str(exe), "8192"], check=True, stdout=subprocess.PIPE, text=True, timeout=120).stdout
+        with tempfile.TemporaryDirectory() as tmp:
+            if not exe.exists():  # built by __graft_entry__.build(); otherwise compiled here, outside the tree
+                src, exe = str(exe) + ".cu", pathlib.Path(tmp) / exe.name
+                subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-o", str(exe),
+                                src], check=True, timeout=600)
+            out = subprocess.run([str(exe), "8192"], check=True, stdout=subprocess.PIPE, text=True, timeout=120).stdout
         return json.loads(out.strip().splitlines()[-1])
     except Exception as exc:      # the bench line then carries peak = None
         return {"error": repr(exc), "tests": {}}
@@ -517,6 +533,28 @@ def cpu_rates(wl, threads, target_s, sample_override=0):
     sample = sample_override or max(probe, int(single * threads * target_s) // 64 * 64)
     dt = wl.cpu(sample, threads)
     return sample / dt, single, sample, dt, threads
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(directory, names, arrays, n):
+    """DIR/<name>.npy for every output of a step over `n` items: float32 for bytes and flags, float64 for wider integers
+    (both exact).  When the files would exceed DUMP_BYTES in all, every per-item output keeps the same seeded sample of
+    items, whose indices go to DIR/sample_index.npy."""
+    import numpy as np
+    outs = {name: a.astype(np.float32 if a.dtype.itemsize == 1 else np.float64) for name, a in zip(names, arrays)}
+    per_item = [k for k, a in outs.items() if a.shape[0] == n]
+    total, budget = sum(a.nbytes for a in outs.values()), DUMP_BYTES - 4096       # 4096: room for the .npy headers
+    if total > budget:
+        fixed = total - sum(outs[k].nbytes for k in per_item)
+        row = sum(outs[k].nbytes for k in per_item) // n + 8                         # + its float64 sample index
+        idx = np.sort(np.random.default_rng(0).choice(n, (budget - fixed) // row, replace=False))
+        outs = {k: (a[idx] if k in per_item else a) for k, a in outs.items()}
+        outs["sample_index"] = idx.astype(np.float64)
+    directory.mkdir(parents=True, exist_ok=True)
+    for k, a in outs.items():
+        np.save(directory / f"{k}.npy", a)
 
 
 # =============================================================================== reference arm
@@ -575,15 +613,19 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if not eg_build.LIB.exists() and "EG_B200_LIB" not in os.environ:
-        # the CUDA library normally travels with the repo snapshot; compile it (nvcc, sm_100a) if it did not.  Rank 0
-        # of a node builds, the others wait for the file.  There is no other implementation to fall back to.
+        # __graft_entry__.build() leaves the CUDA library in the package.  Without it, compile it (nvcc, sm_100a) into the
+        # temporary directory, never into the tree, which may be read-only.  Rank 0 of a node builds, the others wait for
+        # an up-to-date file.  There is no other implementation to fall back to.
+        lib = pathlib.Path(tempfile.gettempdir()) / f"eg_b200_bench_{os.getuid()}" / eg_build.LIB.name
+        lib.parent.mkdir(exist_ok=True)
         if local_rank == 0:
-            eg_build.build()
+            eg_build.build(lib=lib)
         else:
             for _ in range(1200):
-                if eg_build.LIB.exists():
+                if not eg_build.needs_build(lib):
                     break
                 time.sleep(0.5)
+        os.environ["EG_B200_LIB"] = str(lib)
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the engine has no CPU fallback")
     torch.cuda.set_device(local_rank)
@@ -678,7 +720,10 @@ def main():
     # ---------------- correctness of what was timed
     def host_outs(tensors):
         return [x.cpu().numpy().view(np.dtype(dt)).reshape(shape) for x, (shape, dt) in zip(tensors, out_specs)]
-    wl.check(B, host_outs(d_out), world, unique)
+    last = host_outs(d_out)
+    wl.check(B, last, world, unique)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pathlib.Path(args.dump_outputs), wl.output_names, last, B)
 
     # ---------------- end-to-end through the host C ABI (`e2e`): host buffers, H2D + D2H inside, every step
     def e2e_run(h_arrays, h_outs, steps):
