@@ -115,6 +115,13 @@ PROTOTYPES = {
     "eg_prove_range_batch_seeded": (C.c_int32, [C.c_void_p, C.POINTER(Range), C.c_char_p, C.c_size_t, P8, P8, P8, C.c_uint64, P8, P8, P8]),
     "eg_qv_prover_draws": (C.c_size_t, [C.POINTER(QvParams)]),
     "eg_encrypt_qv_batch": (C.c_int32, [C.c_void_p, C.POINTER(QvParams), C.c_size_t, P8, P8, P8]),
+    "eg_decrypt_batch": (C.c_int32, [C.c_void_p, P8, C.c_size_t, P8, C.c_void_p, P8, P8, P8]),
+    "eg_decrypt_share_batch": (C.c_int32, [C.c_void_p, C.POINTER(KeySet), C.c_uint32, P8, C.c_size_t, P8, P8, P8, P8, P8]),
+    "eg_decrypt_share_batch_seeded": (C.c_int32, [C.c_void_p, C.POINTER(KeySet), C.c_uint32, P8, C.c_size_t, P8, P8, C.c_uint64, P8, P8, P8]),
+    "eg_decrypt_share_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(KeySet), C.c_uint32, P8, C.c_size_t, P8, P8, P8, C.c_uint64, P8, P8,
+                                               P8]),
+    "eg_prove_decryption_batch": (C.c_int32, [C.c_void_p, C.c_char_p, P8, C.c_size_t, P8, P8, P8, P8, P8]),
+    "eg_prove_decryption_batch_seeded": (C.c_int32, [C.c_void_p, C.c_char_p, P8, C.c_size_t, P8, P8, C.c_uint64, P8, P8, P8]),
     "eg_kernel_launch_count": (C.c_uint64, [C.c_void_p]),
     "eg_last_timings": (C.c_int32, [C.c_void_p, C.POINTER(C.c_float * 5)]),
     "eg_ctx_stream": (C.c_void_p, [C.c_void_p]),

@@ -70,6 +70,7 @@ struct eg_ctx {
     int prove_grid[3] = {0, 0, 0};
     int rprove_grid[3] = {0, 0, 0};
     int sumsq_prove_grid = 0, encrypt_grid = 0;
+    int decrypt_grid[4] = {0, 0, 0, 0};     // k_decrypt<op, ct>: index 2 op + ct
     dev_buf ring_scratch;
     // per-call narrow fixed-base tables of the participant keys of a key set (api_sharing.inc), cached by key bytes
     dev_buf xtab;
@@ -447,6 +448,39 @@ static eg_status launch_encrypt(eg_ctx *ctx, const encrypt_params &P) {
     }
     const unsigned grid = (unsigned)std::min<size_t>((size_t)ctx->encrypt_grid, (P.n + EG_RING_THREADS - 1) / EG_RING_THREADS);
     k_encrypt<<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P);
+#endif
+    ctx->launches++;
+    return EG_SUCCESS;
+}
+
+#ifndef EG_HOSTSIM
+template <int OP, bool CT>
+static eg_status launch_decrypt_t(eg_ctx *ctx, const decrypt_params &P) {
+    int &grid_cache = ctx->decrypt_grid[2 * OP + (CT ? 1 : 0)];
+    if (grid_cache == 0) {
+        int per_sm = 0, sms = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_decrypt<OP, CT>, EG_DECRYPT_THREADS, 0));
+        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
+        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_decrypt does not fit on an SM");
+        grid_cache = per_sm * sms;
+    }
+    const unsigned grid = (unsigned)std::min<size_t>((size_t)grid_cache, (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS);
+    k_decrypt<OP, CT><<<grid, EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
+    return EG_SUCCESS;
+}
+#endif
+
+static eg_status launch_decrypt(eg_ctx *ctx, int op, const decrypt_params &P) {
+    const bool ct = P.rnd.ct != 0;
+#ifdef EG_HOSTSIM
+    if (op == EG_DEC_PLAIN) {
+        if (ct) { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PLAIN, true>(P, tid))) } else { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PLAIN, false>(P, tid))) }
+    } else {
+        if (ct) { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PROOF, true>(P, tid))) } else { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PROOF, false>(P, tid))) }
+    }
+#else
+    if (op == EG_DEC_PLAIN) TRY((ct ? launch_decrypt_t<EG_DEC_PLAIN, true>(ctx, P) : launch_decrypt_t<EG_DEC_PLAIN, false>(ctx, P)));
+    else TRY((ct ? launch_decrypt_t<EG_DEC_PROOF, true>(ctx, P) : launch_decrypt_t<EG_DEC_PROOF, false>(ctx, P)));
 #endif
     ctx->launches++;
     return EG_SUCCESS;
@@ -1001,5 +1035,7 @@ extern "C" eg_status eg_ctx_set_blinding_base(eg_ctx *ctx, const uint8_t base[32
 #include "api_sigma.inc"
 
 #include "api_decrypt.inc"
+
+#include "api_decrypt_side.inc"
 
 #include "api_multi.inc"

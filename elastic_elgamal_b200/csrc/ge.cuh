@@ -654,6 +654,63 @@ EG_HD void ge_fixed_adds_ct(ge_ext &acc, ge_p1p1 &t, int nf, const uint32_t *fta
     }
 }
 
+// out = [a] P from the per-thread window table of P (ge_window_table), variable time: 252 doublings, an addition per non-zero
+// 4-bit digit.  For scalars whose digits are the same in every lane (a decryption key), the branches do not diverge.
+static EG_HD_NOINLINE void ge_var_mul(ge_ext &out, const ge_cached tbl[8], const sc &a) {
+    uint32_t ra[8];
+    sc_recode4(ra, a);
+    ge_ext acc = ge_identity();
+#pragma unroll 1
+    for (int i = 63; i >= 0; i--) {
+        if (i != 63) ge_hot_dbl(acc, 4);
+        const int d = sc_digit4(ra, i);
+        if (d != 0) ge_hot_add_cached(acc, (const uint32_t *)&tbl[(d < 0 ? -d : d) - 1], d < 0, i == 0);
+    }
+    out = acc;
+}
+
+// Constant-time variable-base multiplication for SECRET scalars (a decryption key, a proof nonce): 64 signed 4-bit windows
+// over the table [1..8] P; every window reads all eight entries and keeps one with masks, negates it with masks (swap
+// Y + X / Y - X, negate 2dT) and always adds (digit 0 adds the identity (1, 1, 1, 0)).  No branch and no address depends
+// on the scalar; 252 doublings and 64 additions.
+static EG_HD_NOINLINE void ge_var_mul_ct(ge_ext &out, const ge_cached tbl[8], const sc &a) {
+    uint32_t ra[8];
+    sc_recode4(ra, a);
+    ge_ext acc = ge_identity();
+    ge_p1p1 t;
+#pragma unroll 1
+    for (int i = 63; i >= 0; i--) {
+        if (i != 63) ge_hot_dbl(acc, 4);
+        const int d = sc_digit4(ra, i);                         // secret, in [-8, 7]
+        const uint32_t sign = (uint32_t)(d >> 31);              // all ones when negative
+        const uint32_t mag = ((uint32_t)d ^ sign) - sign;       // |d|
+        ge_cached e;
+        e.YpX = fe_one(); e.YmX = fe_one(); e.Z = fe_one(); e.T2d = fe_zero();
+#pragma unroll 1
+        for (uint32_t k = 1; k <= 8; k++) {
+            const uint32_t m = (uint32_t)0 - (uint32_t)((((mag ^ k) - 1u) >> 31) & 1u);      // all ones iff mag == k
+            const ge_cached &q = tbl[k - 1];
+            for (int w = 0; w < 8; w++) {
+                e.YpX.v[w] = (e.YpX.v[w] & ~m) | (q.YpX.v[w] & m);
+                e.YmX.v[w] = (e.YmX.v[w] & ~m) | (q.YmX.v[w] & m);
+                e.Z.v[w] = (e.Z.v[w] & ~m) | (q.Z.v[w] & m);
+                e.T2d.v[w] = (e.T2d.v[w] & ~m) | (q.T2d.v[w] & m);
+            }
+        }
+        fe nt;
+        fe_neg(nt, e.T2d);
+        for (int w = 0; w < 8; w++) {
+            const uint32_t p = e.YpX.v[w], q = e.YmX.v[w];
+            e.YpX.v[w] = (p & ~sign) | (q & sign);
+            e.YmX.v[w] = (q & ~sign) | (p & sign);
+            e.T2d.v[w] = (e.T2d.v[w] & ~sign) | (nt.v[w] & sign);
+        }
+        ge_add_cached_p1p1(t, acc, e, false);
+        ge_p1p1_to_ext(acc, t);
+    }
+    out = acc;
+}
+
 // fixed-base-only form (the provers' [x] G, [x] K + [y] G); ct selects the constant-time table walk for secret scalars
 static EG_HD_NOINLINE void ge_eval_fixed(ge_ext &out, int nf, const uint32_t *ftab0, const sc &b0, const uint32_t *ftab1, const sc &b1,
                                          bool ct = false) {
@@ -737,6 +794,34 @@ static EG_HD_NOINLINE void ge_double_compress2(uint32_t w0[8], uint32_t w1[8], c
     fe_select(i1, i1, fe_zero(), z1);
     ge_dc_finish(w0, s0, i0);
     ge_dc_finish(w1, s1, i1);
+}
+
+// w[k] = encode(2 Q[k]), k < N, with one inversion: Montgomery's trick over ge_dc_prepare's products, as k_terminal.  The
+// per-point states live in local arrays walked by rolled loops (N x 48 words would not stay in registers anyway).
+template <int N>
+static EG_HD_NOINLINE void ge_double_compress_n(uint32_t w[N][8], const ge_ext Q[N]) {
+    ge_dc_state st[N];
+    fe prefix[N], u[N];
+    bool z[N];
+    fe run = fe_one();
+#pragma unroll 1
+    for (int k = 0; k < N; k++) {
+        fe t;
+        ge_dc_prepare(st[k], t, Q[k]);
+        z[k] = fe_iszero(t);
+        fe_select(u[k], t, fe_one(), z[k]);
+        fe_mul(run, run, u[k]);
+        prefix[k] = run;
+    }
+    fe inv;
+    fe_invert(inv, run);
+#pragma unroll 1
+    for (int k = N - 1; k >= 0; k--) {
+        fe ik;
+        if (k) { fe_mul(ik, inv, prefix[k - 1]); fe_mul(inv, inv, u[k]); } else ik = inv;
+        fe_select(ik, ik, fe_zero(), z[k]);
+        ge_dc_finish(w[k], st[k], ik);
+    }
 }
 
 EG_HD void ge_double_compress1(uint32_t w[8], const ge_ext &Q) {

@@ -1751,6 +1751,19 @@ struct dlog_lookup_params {
     uint8_t *found;             // 1 found, 0 absent, 2 malformed input
 };
 
+// DiscreteLogTable::get (encryption.rs:287-297) on a non-identity element's encoding `w`: 1 and `value` when present, 0 absent
+EG_HD uint8_t dlog_probe(const uint32_t w[8], size_t cap, const uint32_t *keys, const unsigned long long *vals, unsigned long long &value) {
+    size_t slot = (size_t)dlog_hash(w) & (cap - 1);
+    for (;;) {
+        const unsigned long long v = vals[slot];
+        if (v == 0) { value = 0; return 0; }
+        bool eq = true;
+        for (int k = 0; k < 8; k++) eq = eq && (keys[slot * 8 + k] == w[k]);
+        if (eq) { value = v; return 1; }
+        slot = (slot + 1) & (cap - 1);
+    }
+}
+
 EG_HD void dlog_lookup_body(const dlog_lookup_params &P, size_t item) {
     if (P.flags[item] & 1u) { P.found[item] = 2; P.values[item] = 0; return; }
     ge_ext B, D, M;
@@ -1760,15 +1773,108 @@ EG_HD void dlog_lookup_body(const dlog_lookup_params &P, size_t item) {
     if (ge_is_identity(M)) { P.found[item] = 1; P.values[item] = 0; return; }
     uint32_t w[8];
     ge_encode(w, M);
-    size_t slot = (size_t)dlog_hash(w) & (P.cap - 1);
-    for (;;) {
-        unsigned long long v = P.vals[slot];
-        if (v == 0) { P.found[item] = 0; P.values[item] = 0; return; }
-        bool eq = true;
-        for (int k = 0; k < 8; k++) eq = eq && (P.keys[slot * 8 + k] == w[k]);
-        if (eq) { P.found[item] = 1; P.values[item] = v; return; }
-        slot = (slot + 1) & (P.cap - 1);
+    unsigned long long v = 0;
+    P.found[item] = dlog_probe(w, P.cap, P.keys, P.vals, v);
+    P.values[item] = v;
+}
+
+// ------------------------------------------------------------------ decryption side: the talliers' operations
+//
+// One thread per ciphertext, with the holder's secret key s (a canonical scalar, the same in every lane):
+//   EG_DEC_PLAIN  SecretKey::decrypt_to_element (keys/impls.rs:160-177): M = B - [s]R, encoded, then DiscreteLogTable::get
+//                 (encryption.rs:287-297) when a table is given.
+//   EG_DEC_PROOF  dh = [s]R with a LogEqualityProof over log base R (log_equality.rs:114-143): the share of
+//                 ActiveParticipant::decrypt_share (participant.rs:163-185) or VerifiableDecryption::new with a custom key
+//                 (decryption.rs:89-111) -- the two differ only in the transcript prefix and the public key, both host-made.
+//                 Nonce x = one 64-byte block; [x]G from the wide table of G, [s/2]R and [x/2]R share one window table of R,
+//                 the three encodings take one inversion (ge_double_compress_n on the half-scalar points); s = c s + x.
+// CT = true (eg_ctx_set_prover_mode 1): the key and the nonce go through ge_var_mul_ct / ge_fixed_adds_ct.
+#define EG_DEC_PLAIN 0
+#define EG_DEC_PROOF 1
+
+struct decrypt_params {
+    size_t n;
+    const uint8_t *cts;                  // n * 64
+    const uint8_t *wide;                 // EG_DEC_PROOF, caller-supplied blocks: n * 64
+    uint8_t *out;                        // n * 32: the element (plain, may be null) / dh (proof)
+    uint8_t *proofs;                     // EG_DEC_PROOF: n * 64 = c | s
+    unsigned long long *values;          // EG_DEC_PLAIN with a table: n
+    uint8_t *flags;                      // n: plain: found (1 / 0 / 2 = does not decode); proof: ok
+    uint32_t secret[8];                  // the key, by value (like rand_src's ChaCha seed)
+    uint32_t key_words[8];               // EG_DEC_PROOF: encoding of [s]G, "[r]G" of the transcript
+    transcript prefix;                   // EG_DEC_PROOF: up to and including start_proof("log_eq")
+    size_t cap;                          // EG_DEC_PLAIN: dlog table (keys == null: no table)
+    const uint32_t *keys;
+    const unsigned long long *vals;
+    const uint32_t *table_g;
+    rand_src rnd;
+};
+
+template <int OP, bool CT>
+EG_HD void decrypt_body(const decrypt_params &P, size_t item) {
+    uint32_t w[8], w2[8];
+    load32_bytes(w, P.cts + item * 64);
+    ge_ext R, B;
+    bool ok = ge_decode(R, w);
+    if (OP == EG_DEC_PLAIN) {
+        load32_bytes(w2, P.cts + item * 64 + 32);
+        ok = ge_decode(B, w2) && ok;
     }
+    if (!ok) {
+        for (int k = 0; k < 8; k++) w[k] = 0;
+        if (P.out) store32_bytes(P.out + item * 32, w);
+        if (OP == EG_DEC_PLAIN) {
+            P.flags[item] = 2;
+            if (P.values) P.values[item] = 0;
+        } else {
+            store32_bytes(P.proofs + item * 64, w);
+            store32_bytes(P.proofs + item * 64 + 32, w);
+            P.flags[item] = 0;
+        }
+        return;
+    }
+    EG_ALIGN16 ge_cached tbl[8];
+    ge_window_table(tbl, R);
+    sc s;
+    for (int k = 0; k < 8; k++) s.v[k] = P.secret[k];
+    if (OP == EG_DEC_PLAIN) {
+        ge_ext D, M;
+        if (CT) ge_var_mul_ct(D, tbl, s); else ge_var_mul(D, tbl, s);
+        ge_sub(M, B, D);
+        ge_encode(w, M);
+        if (P.out) store32_bytes(P.out + item * 32, w);
+        uint8_t f = 1;
+        if (P.keys) {
+            unsigned long long v = 0;
+            if (!ge_is_identity(M)) f = dlog_probe(w, P.cap, P.keys, P.vals, v);
+            P.values[item] = v;
+        }
+        P.flags[item] = f;
+        return;
+    }
+    uint32_t blk[16], enc[3][8];                             // dh | [x]G | [x]R
+    sc x, hs, hx, c, resp;
+    rand_block(blk, P.rnd, item, 0, P.wide + item * 64);
+    sc_from_wide_words(x, blk);
+    sc_half(hs, s);
+    sc_half(hx, x);
+    ge_ext q[3];
+    if (CT) { ge_var_mul_ct(q[0], tbl, hs); ge_var_mul_ct(q[2], tbl, hx); }
+    else { ge_var_mul(q[0], tbl, hs); ge_var_mul(q[2], tbl, hx); }
+    ge_eval_fixed(q[1], 1, P.table_g, hx, P.table_g, hx, CT);
+    ge_double_compress_n<3>(enc, q);
+    transcript t = P.prefix;
+    merlin_append_words(t, EG_LBL("K"), w, 8);                 // R's own bytes: canonical, as it decoded
+    merlin_append_words(t, EG_LBL("[r]G"), P.key_words, 8);
+    merlin_append_words(t, EG_LBL("[r]K"), enc[0], 8);
+    merlin_append_words(t, EG_LBL("[x]G"), enc[1], 8);
+    merlin_append_words(t, EG_LBL("[x]K"), enc[2], 8);
+    merlin_challenge_scalar(t, EG_LBL("c"), c);
+    sc_muladd(resp, c, s, x);
+    store32_bytes(P.out + item * 32, enc[0]);
+    store32_bytes(P.proofs + item * 64, c.v);
+    store32_bytes(P.proofs + item * 64 + 32, resp.v);
+    P.flags[item] = 1;
 }
 
 

@@ -461,7 +461,62 @@ class Engine:
                                                       _addr(values), _addr(found)))
         return values, found
 
+    # ---- decryption side (the holder's secret key; randomness as for encrypt_*: `wide_rand` blocks or `seed=`)
+    @staticmethod
+    def _secret(secret):
+        return _u8(np.frombuffer(bytes(secret), dtype=np.uint8), (32,))
+
+    def decrypt(self, secret, cts, table=None):
+        """SecretKey::decrypt_to_element / decrypt: (elements, values, found); values is None without a table, found as
+        eg_decrypt_batch (1 found / decoded, 0 absent from the table, 2 the ciphertext does not decode)."""
+        cts = _u8(cts, (-1, 64))
+        n = cts.shape[0]
+        elements, found = np.empty((n, 32), np.uint8), np.empty(n, np.uint8)
+        values = np.zeros(n, np.uint64) if table is not None else None
+        sec = self._secret(secret)
+        self._check(self.lib.eg_decrypt_batch(self.h, _addr(sec), n, _addr(cts), table.h if table is not None else None,
+                                              _addr(elements), _addr(values), _addr(found)))
+        return elements, values, found
+
+    def decrypt_share(self, keyset, index, secret, cts, wide_rand=None, seed=None, counter_base=0):
+        """ActiveParticipant::decrypt_share: (shares, proofs, ok) in the layouts verify_shares reads (one share per tally)."""
+        cts = _u8(cts, (-1, 64))
+        n = cts.shape[0]
+        shares, proofs, ok = np.empty((n, 32), np.uint8), np.empty((n, 64), np.uint8), np.empty(n, np.uint8)
+        sec = self._secret(secret)
+        if seed is not None:
+            seed = self._seed(seed)
+            self._check(self.lib.eg_decrypt_share_batch_seeded(self.h, C.byref(keyset), index, _addr(sec), n, _addr(cts),
+                                                               _addr(seed), counter_base, _addr(shares), _addr(proofs),
+                                                               _addr(ok)))
+        else:
+            wide_rand = _u8(wide_rand, (n, 64))
+            self._check(self.lib.eg_decrypt_share_batch(self.h, C.byref(keyset), index, _addr(sec), n, _addr(cts),
+                                                        _addr(wide_rand), _addr(shares), _addr(proofs), _addr(ok)))
+        return shares, proofs, ok.astype(bool)
+
+    def prove_decryption(self, label, secret, cts, wide_rand=None, seed=None, counter_base=0):
+        """VerifiableDecryption::new with the key pair (secret, [secret]G): (dh_elements, proofs, ok)."""
+        cts = _u8(cts, (-1, 64))
+        n = cts.shape[0]
+        dh, proofs, ok = np.empty((n, 32), np.uint8), np.empty((n, 64), np.uint8), np.empty(n, np.uint8)
+        sec = self._secret(secret)
+        if seed is not None:
+            seed = self._seed(seed)
+            self._check(self.lib.eg_prove_decryption_batch_seeded(self.h, label.encode(), _addr(sec), n, _addr(cts),
+                                                                  _addr(seed), counter_base, _addr(dh), _addr(proofs), _addr(ok)))
+        else:
+            wide_rand = _u8(wide_rand, (n, 64))
+            self._check(self.lib.eg_prove_decryption_batch(self.h, label.encode(), _addr(sec), n, _addr(cts),
+                                                           _addr(wide_rand), _addr(dh), _addr(proofs), _addr(ok)))
+        return dh, proofs, ok.astype(bool)
+
     # ---- device-pointer variants (ints are raw device addresses, e.g. torch.Tensor.data_ptr())
+    def decrypt_share_dev(self, keyset, index, secret, n, d_cts, d_shares, d_proofs, d_ok, d_wide_rand=None, seed=None, counter_base=0):
+        sec, seed = self._secret(secret), (self._seed(seed) if seed is not None else None)
+        self._check(self.lib.eg_decrypt_share_batch_dev(self.h, C.byref(keyset), index, _addr(sec), n, d_cts, d_wide_rand, _addr(seed),
+                                                        counter_base, d_shares, d_proofs, d_ok))
+
     def verify_bool_dev(self, n, d_cts, d_proofs, d_verdicts):
         self._check(self.lib.eg_verify_bool_batch_dev(self.h, n, d_cts, d_proofs, d_verdicts))
 

@@ -394,6 +394,46 @@ eg_status eg_encrypt_qv_batch_seeded(eg_ctx *ctx, const eg_qv_params *params, si
  * before a prover call returns.  Verification entry points only handle public data and stay variable-time. */
 eg_status eg_ctx_set_prover_mode(eg_ctx *ctx, int constant_time);
 
+/* ---- decryption side (the talliers' operations; they hold a secret) ------------------------------
+ * None of these needs a receiver key.  A secret that is not a canonical scalar is EG_ERR_INVALID_ARG.  The secret's digits
+ * follow eg_ctx_set_prover_mode like the nonces' (s = c secret + x: a leaked nonce reveals the key), the key travels by
+ * value in the kernel launch parameters, and the staging buffers are zeroed before a host-pointer call returns.  On a
+ * multi-device context the host forms shard the batch; item i keeps its own randomness either way. */
+
+/* SecretKey::decrypt_to_element / decrypt (src/keys/impls.rs:160-177) -> DiscreteLogTable::get (src/encryption.rs:287-297).
+ * elements (n*32, may be NULL): encode(B - [secret]R).  table may be NULL (then values may be NULL).
+ * found[i]: as eg_combine_decrypt_batch (1 found / identity -> 0, 0 absent, 2 ciphertext does not decode);
+ * without a table 1 = decoded, 2 = does not decode. */
+eg_status eg_decrypt_batch(eg_ctx *ctx, const uint8_t secret[32], size_t n, const uint8_t *cts /* n*64 */,
+                           const eg_dlog_table *table, uint8_t *elements, uint64_t *values, uint8_t *found /* n */);
+
+/* ActiveParticipant::decrypt_share (src/sharing/participant.rs:163-185): participant `index` of `keyset` with its secret
+ * share; one 64-byte block per item (the LogEqualityProof::new nonce, src/proofs/log_equality.rs:114-143).
+ * shares[i] / proofs[i] in the layouts eg_verify_shares_batch reads (one column of its n_tallies x n_shares arrays).
+ * ok[i] = 0 (outputs zeroed) when cts[i] does not decode.  index >= keyset->shares is EG_ERR_INVALID_ARG; the participant
+ * key is validated like PublicKey::from_bytes (EG_ERR_INVALID_ELEMENT); [secret_share]G != participant_keys[index] is
+ * EG_ERR_INVALID_ARG (the reference cannot build such an ActiveParticipant). */
+eg_status eg_decrypt_share_batch(eg_ctx *ctx, const eg_keyset *keyset, uint32_t index, const uint8_t secret_share[32], size_t n,
+                                 const uint8_t *cts /* n*64 */, const uint8_t *wide_rand /* n*64 */, uint8_t *shares /* n*32 */,
+                                 uint8_t *proofs /* n*64 */, uint8_t *ok /* n */);
+eg_status eg_decrypt_share_batch_seeded(eg_ctx *ctx, const eg_keyset *keyset, uint32_t index, const uint8_t secret_share[32], size_t n,
+                                        const uint8_t *cts, const uint8_t seed[32], uint64_t counter_base, uint8_t *shares,
+                                        uint8_t *proofs, uint8_t *ok);
+/* device pointers on a single-device context; seed == NULL -> one block per item at d_wide_rand (as eg_encrypt_*_batch_dev) */
+eg_status eg_decrypt_share_batch_dev(eg_ctx *ctx, const eg_keyset *keyset, uint32_t index, const uint8_t secret_share[32], size_t n,
+                                     const uint8_t *d_cts, const uint8_t *d_wide_rand, const uint8_t seed[32], uint64_t counter_base,
+                                     uint8_t *d_shares, uint8_t *d_proofs, uint8_t *d_ok);
+
+/* VerifiableDecryption::new with the key pair (secret, [secret]G) (src/decryption.rs:89-111), Transcript::new(label).
+ * One block per item (the proof nonce).  Outputs are what eg_verify_decryption_batch(label, [secret]G, ...) accepts;
+ * ok[i] = 0 (outputs zeroed) when cts[i] does not decode. */
+eg_status eg_prove_decryption_batch(eg_ctx *ctx, const char *transcript_label, const uint8_t secret[32], size_t n,
+                                    const uint8_t *cts /* n*64 */, const uint8_t *wide_rand /* n*64 */, uint8_t *dh_elements /* n*32 */,
+                                    uint8_t *proofs /* n*64 */, uint8_t *ok /* n */);
+eg_status eg_prove_decryption_batch_seeded(eg_ctx *ctx, const char *transcript_label, const uint8_t secret[32], size_t n,
+                                           const uint8_t *cts, const uint8_t seed[32], uint64_t counter_base, uint8_t *dh_elements,
+                                           uint8_t *proofs, uint8_t *ok);
+
 /* ---- device-pointer variants (inputs already resident in HBM; same semantics) ------------------- */
 eg_status eg_verify_bool_batch_dev(eg_ctx *ctx, size_t n, const uint8_t *d_cts, const uint8_t *d_proofs, uint8_t *d_verdicts);
 eg_status eg_verify_choice_batch_dev(eg_ctx *ctx, size_t n, uint32_t options, int single, const uint8_t *d_choices,

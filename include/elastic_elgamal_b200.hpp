@@ -281,6 +281,48 @@ class Engine {
         return out;
     }
 
+    // secret.decrypt(ct, &table) over a batch (keys/impls.rs:160-177); table == nullptr: decrypt_to_element only (found = decoded)
+    std::vector<DecryptedValue> decrypt_batch(const Scalar &secret, const std::vector<Ciphertext> &cts, const eg_dlog_table *table,
+                                              std::vector<Element> *elements = nullptr) {
+        const size_t n = cts.size();
+        std::vector<uint8_t> c, el(32 * n), found(n);
+        std::vector<uint64_t> values(n);
+        for (const auto &ct : cts) append(c, ct);
+        check(eg_decrypt_batch(ctx_, secret.data(), n, c.data(), table, el.data(), table ? values.data() : nullptr, found.data()));
+        if (elements) {
+            elements->assign(n, Element{});
+            for (size_t i = 0; i < n; i++) std::copy(el.begin() + 32 * i, el.begin() + 32 * (i + 1), (*elements)[i].begin());
+        }
+        std::vector<DecryptedValue> out(n);
+        for (size_t i = 0; i < n; i++) out[i] = DecryptedValue{found[i] == 1, values[i]};
+        return out;
+    }
+
+    // participant.decrypt_share(ct, rng) over a batch with in-kernel randomness (participant.rs:163-185): shares + proofs
+    std::pair<std::vector<Element>, std::vector<LogEqualityProof>> decrypt_share_batch(const PublicKeySet &ks, uint32_t index, const Scalar &secret_share,
+                                                                                       const std::vector<Ciphertext> &cts, const Seed &seed) {
+        if (ks.participant_keys.size() != ks.shares || ks.shares > 64) throw Error(EG_ERR_LEN_MISMATCH, "key set size mismatch");
+        eg_keyset k{};
+        k.shares = ks.shares; k.threshold = ks.threshold;
+        std::copy(ks.shared_key.bytes.begin(), ks.shared_key.bytes.end(), k.shared_key);
+        for (uint32_t i = 0; i < ks.shares; i++) std::copy(ks.participant_keys[i].bytes.begin(), ks.participant_keys[i].bytes.end(), k.participant_keys[i]);
+        const size_t n = cts.size();
+        std::vector<uint8_t> c, d(32 * n), p(64 * n), ok(n);
+        for (const auto &ct : cts) append(c, ct);
+        check(eg_decrypt_share_batch_seeded(ctx_, &k, index, secret_share.data(), n, c.data(), seed.key.data(), seed.counter_base, d.data(), p.data(), ok.data()));
+        return split_log_eq(d, p);
+    }
+
+    // VerifiableDecryption::new(ct, &(secret, [secret]G), &mut Transcript::new(label), rng) over a batch (decryption.rs:89-111)
+    std::pair<std::vector<Element>, std::vector<LogEqualityProof>> prove_decryption_batch(const Scalar &secret, const std::vector<Ciphertext> &cts,
+                                                                                          const std::string &label, const Seed &seed) {
+        const size_t n = cts.size();
+        std::vector<uint8_t> c, d(32 * n), p(64 * n), ok(n);
+        for (const auto &ct : cts) append(c, ct);
+        check(eg_prove_decryption_batch_seeded(ctx_, label.c_str(), secret.data(), n, c.data(), seed.key.data(), seed.counter_base, d.data(), p.data(), ok.data()));
+        return split_log_eq(d, p);
+    }
+
     // key.encrypt_bool(value, rng) over a batch with in-kernel randomness (keys/impls.rs:77-89)
     std::pair<std::vector<Ciphertext>, std::vector<RingProof>> encrypt_bool_batch(const std::vector<uint8_t> &values, const Seed &seed) {
         const size_t n = values.size();
@@ -337,6 +379,17 @@ class Engine {
             std::copy(t.begin() + 64 * k + 32, t.begin() + 64 * k + 64, out[k].blinded_element.begin());
         }
         return out;
+    }
+    static std::pair<std::vector<Element>, std::vector<LogEqualityProof>> split_log_eq(const std::vector<uint8_t> &d, const std::vector<uint8_t> &p) {
+        const size_t n = d.size() / 32;
+        std::vector<Element> el(n);
+        std::vector<LogEqualityProof> pr(n);
+        for (size_t i = 0; i < n; i++) {
+            std::copy(d.begin() + 32 * i, d.begin() + 32 * (i + 1), el[i].begin());
+            std::copy(p.begin() + 64 * i, p.begin() + 64 * i + 32, pr[i].challenge.begin());
+            std::copy(p.begin() + 64 * i + 32, p.begin() + 64 * (i + 1), pr[i].response.begin());
+        }
+        return {el, pr};
     }
     static RingProof ring_proof(const uint8_t *p, size_t responses) {
         RingProof out;

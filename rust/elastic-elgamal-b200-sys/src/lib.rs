@@ -186,6 +186,23 @@ extern "C" {
     pub fn eg_encrypt_qv_batch(ctx: *mut eg_ctx, params: *const eg_qv_params, n: usize, votes: *const u64,
                                wide_rand: *const u8, ballots: *mut u8) -> eg_status;
 
+    // decryption side (SecretKey::decrypt, ActiveParticipant::decrypt_share, VerifiableDecryption::new)
+    pub fn eg_decrypt_batch(ctx: *mut eg_ctx, secret: *const u8, n: usize, cts: *const u8, table: *const eg_dlog_table,
+                            elements: *mut u8, values: *mut u64, found: *mut u8) -> eg_status;
+    pub fn eg_decrypt_share_batch(ctx: *mut eg_ctx, keyset: *const eg_keyset, index: u32, secret_share: *const u8, n: usize,
+                                  cts: *const u8, wide_rand: *const u8, shares: *mut u8, proofs: *mut u8, ok: *mut u8) -> eg_status;
+    pub fn eg_decrypt_share_batch_seeded(ctx: *mut eg_ctx, keyset: *const eg_keyset, index: u32, secret_share: *const u8, n: usize,
+                                         cts: *const u8, seed: *const u8, counter_base: u64, shares: *mut u8, proofs: *mut u8,
+                                         ok: *mut u8) -> eg_status;
+    pub fn eg_decrypt_share_batch_dev(ctx: *mut eg_ctx, keyset: *const eg_keyset, index: u32, secret_share: *const u8, n: usize,
+                                      d_cts: *const u8, d_wide_rand: *const u8, seed: *const u8, counter_base: u64, d_shares: *mut u8,
+                                      d_proofs: *mut u8, d_ok: *mut u8) -> eg_status;
+    pub fn eg_prove_decryption_batch(ctx: *mut eg_ctx, transcript_label: *const c_char, secret: *const u8, n: usize, cts: *const u8,
+                                     wide_rand: *const u8, dh_elements: *mut u8, proofs: *mut u8, ok: *mut u8) -> eg_status;
+    pub fn eg_prove_decryption_batch_seeded(ctx: *mut eg_ctx, transcript_label: *const c_char, secret: *const u8, n: usize,
+                                            cts: *const u8, seed: *const u8, counter_base: u64, dh_elements: *mut u8, proofs: *mut u8,
+                                            ok: *mut u8) -> eg_status;
+
     pub fn eg_last_kernel_stats(ctx: *const eg_ctx, kind: c_int, launches: *mut u64, tasks: *mut u64, ms: *mut f32) -> eg_status;
     pub fn eg_kernel_launch_count(ctx: *const eg_ctx) -> u64;
     pub fn eg_last_timings(ctx: *const eg_ctx, out_ms: *mut f32) -> eg_status;

@@ -26,7 +26,7 @@ use elastic_elgamal::{
     group::{ElementOps, Ristretto, ScalarOps},
     sharing::{self, PublicKeySet},
     CandidateDecryption, Ciphertext, CommitmentEquivalenceProof, LogEqualityProof, ProofOfPossession, PublicKey,
-    RangeDecomposition, RangeProof, RingProof, SumOfSquaresProof, VerifiableDecryption, VerificationError,
+    RangeDecomposition, RangeProof, RingProof, SecretKey, SumOfSquaresProof, VerifiableDecryption, VerificationError,
 };
 use elastic_elgamal_b200_sys as sys;
 use serde::Serialize;
@@ -609,6 +609,112 @@ impl Engine {
             sys::eg_combine_decrypt_batch(self.ctx, t as u32, idx.as_ptr(), n, t as u32, c.as_ptr(), sh.as_ptr(), table.table, values.as_mut_ptr(), found.as_mut_ptr())
         })?;
         Ok(values.iter().zip(found).map(|(&v, f)| (f == 1).then_some(v)).collect())
+    }
+
+    // ------------------------------------------------------------------ decryption side (the holder's secret key)
+
+    fn secret_bytes(secret: &SecretKey<Ristretto>) -> [u8; 32] {
+        let mut b = [0_u8; 32];
+        Ristretto::serialize_scalar(secret.expose_scalar(), &mut b);
+        b
+    }
+
+    fn share_outputs(dh: &[u8], proofs: &[u8], ok: &[u8]) -> Vec<(VerifiableDecryption<Ristretto>, LogEqualityProof<Ristretto>)> {
+        debug_assert!(ok.iter().all(|&f| f == 1), "typed ciphertexts decode");
+        dh.chunks(32)
+            .zip(proofs.chunks(64))
+            .map(|(d, p)| {
+                let d = CandidateDecryption::from_bytes(d).expect("the engine emits canonical encodings").into_unchecked();
+                (d, LogEqualityProof::from_bytes(p).expect("the engine emits canonical scalars"))
+            })
+            .collect()
+    }
+
+    /// `secret.decrypt_to_element(ct)` over a batch (keys/impls.rs:160-163).
+    pub fn decrypt_to_elements(&self, secret: &SecretKey<Ristretto>, cts: &[Ciphertext<Ristretto>]) -> Result<Vec<Element>, EngineError> {
+        let n = cts.len();
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let (mut elements, mut found) = (vec![0_u8; n * 32], vec![0_u8; n]);
+        let key = Self::secret_bytes(secret);
+        self.check(unsafe {
+            sys::eg_decrypt_batch(self.ctx, key.as_ptr(), n, c.as_ptr(), ptr::null(), elements.as_mut_ptr(), ptr::null_mut(), found.as_mut_ptr())
+        })?;
+        Ok(elements.chunks(32).map(element).collect())
+    }
+
+    /// `secret.decrypt(ct, &table)` over a batch (keys/impls.rs:165-177): `Some(value)` or `None` outside the table.
+    pub fn decrypt(&self, secret: &SecretKey<Ristretto>, cts: &[Ciphertext<Ristretto>], table: &DlogTable<'_>) -> Result<Vec<Option<u64>>, EngineError> {
+        let n = cts.len();
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let (mut values, mut found) = (vec![0_u64; n], vec![0_u8; n]);
+        let key = Self::secret_bytes(secret);
+        self.check(unsafe {
+            sys::eg_decrypt_batch(self.ctx, key.as_ptr(), n, c.as_ptr(), table.table, ptr::null_mut(), values.as_mut_ptr(), found.as_mut_ptr())
+        })?;
+        Ok(values.iter().zip(found).map(|(&v, f)| (f == 1).then_some(v)).collect())
+    }
+
+    /// `participant.decrypt_share(ct, rng)` over a batch for participant `index` of `key_set` holding `secret_share`
+    /// (participant.rs:163-185); one randomness block per ciphertext.  A secret share that does not match
+    /// `key_set.participant_keys()[index]` is an `EngineError` (the reference cannot build that participant).
+    pub fn decrypt_shares(
+        &self,
+        key_set: &PublicKeySet<Ristretto>,
+        index: usize,
+        secret_share: &SecretKey<Ristretto>,
+        cts: &[Ciphertext<Ristretto>],
+        randomness: Randomness<'_>,
+    ) -> Result<Vec<(VerifiableDecryption<Ristretto>, LogEqualityProof<Ristretto>)>, EngineError> {
+        let n = cts.len();
+        assert!(key_set.params().shares <= 64);
+        let ks = Self::keyset(key_set);
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let (mut dh, mut proofs, mut ok) = (vec![0_u8; n * 32], vec![0_u8; n * 64], vec![0_u8; n]);
+        let key = Self::secret_bytes(secret_share);
+        self.check(match randomness {
+            Randomness::Blocks(wide) => {
+                assert_eq!(wide.len(), n * 64);
+                unsafe {
+                    sys::eg_decrypt_share_batch(self.ctx, &ks, index as u32, key.as_ptr(), n, c.as_ptr(), wide.as_ptr(), dh.as_mut_ptr(),
+                                                proofs.as_mut_ptr(), ok.as_mut_ptr())
+                }
+            }
+            Randomness::Seeded { seed, counter_base } => unsafe {
+                sys::eg_decrypt_share_batch_seeded(self.ctx, &ks, index as u32, key.as_ptr(), n, c.as_ptr(), seed.as_ptr(), counter_base,
+                                                   dh.as_mut_ptr(), proofs.as_mut_ptr(), ok.as_mut_ptr())
+            },
+        })?;
+        Ok(Self::share_outputs(&dh, &proofs, &ok))
+    }
+
+    /// `VerifiableDecryption::new(ct, &keypair, &mut Transcript::new(label), rng)` over a batch with the key pair
+    /// `(secret, [secret]G)` (decryption.rs:89-111); one randomness block per ciphertext.
+    pub fn prove_decryptions(
+        &self,
+        transcript_label: &str,
+        secret: &SecretKey<Ristretto>,
+        cts: &[Ciphertext<Ristretto>],
+        randomness: Randomness<'_>,
+    ) -> Result<Vec<(VerifiableDecryption<Ristretto>, LogEqualityProof<Ristretto>)>, EngineError> {
+        let n = cts.len();
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let label = CString::new(transcript_label).map_err(|_| EngineError { status: sys::EG_ERR_INVALID_ARG, message: "label contains NUL".into() })?;
+        let (mut dh, mut proofs, mut ok) = (vec![0_u8; n * 32], vec![0_u8; n * 64], vec![0_u8; n]);
+        let key = Self::secret_bytes(secret);
+        self.check(match randomness {
+            Randomness::Blocks(wide) => {
+                assert_eq!(wide.len(), n * 64);
+                unsafe {
+                    sys::eg_prove_decryption_batch(self.ctx, label.as_ptr(), key.as_ptr(), n, c.as_ptr(), wide.as_ptr(), dh.as_mut_ptr(),
+                                                   proofs.as_mut_ptr(), ok.as_mut_ptr())
+                }
+            }
+            Randomness::Seeded { seed, counter_base } => unsafe {
+                sys::eg_prove_decryption_batch_seeded(self.ctx, label.as_ptr(), key.as_ptr(), n, c.as_ptr(), seed.as_ptr(), counter_base,
+                                                      dh.as_mut_ptr(), proofs.as_mut_ptr(), ok.as_mut_ptr())
+            },
+        })?;
+        Ok(Self::share_outputs(&dh, &proofs, &ok))
     }
 
     // ------------------------------------------------------------------ ciphertext operators
