@@ -1705,7 +1705,7 @@ struct dlog_build_params {
 EG_HD void dlog_build_body(const dlog_build_params &P, size_t tid) {
     uint64_t v0 = P.lo + tid * P.per;
     if (v0 >= P.hi) return;
-    uint64_t v1 = v0 + P.per < P.hi ? v0 + P.per : P.hi;
+    uint64_t v1 = P.hi - v0 > P.per ? v0 + P.per : P.hi;      // v0 + per may wrap past 2^64 in the top slice
     ge_ext G = ge_generator(), acc = ge_identity();
     ge_cached cg;
     ge_to_cached(cg, G);
