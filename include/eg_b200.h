@@ -192,7 +192,12 @@ eg_status eg_verify_choice_batch(eg_ctx *ctx, size_t n, uint32_t options, int si
                                  uint8_t *tally /* options*64 or NULL */);
 
 /* RangeDecomposition (src/proofs/range.rs:106-108): rings listed as in `Display` (:110-124), most significant
- * first; ring i admits the values step[i] * {0, .., size[i]-1}. */
+ * first; ring i admits the values step[i] * {0, .., size[i]-1}.  The range is [0, upper bound) with upper bound
+ * 1 + sum (size[i] - 1) * step[i], taken without overflow: from 2^64 on, every uint64_t value is in it.  Every call that
+ * takes an eg_range returns EG_ERR_INVALID_ARG unless it has 1..64 rings, sizes in 1..4096 summing to at most 3500,
+ * non-zero steps, and no gaps: read from the last ring to the first, the step of each ring of size > 1 is at most the
+ * upper bound of the rings after it (1 for the last ring).  eg_range_optimal always produces such a decomposition, and
+ * with it every value below the upper bound is decomposed greedily, most significant ring first. */
 typedef struct {
     uint32_t n_rings;
     uint32_t reserved;

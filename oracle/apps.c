@@ -770,8 +770,8 @@ int eo_gen_range_batch(const uint8_t pkb[32], const eo_range *range, const char 
                        uint8_t *rings, int threads) {
     range_ctx c;
     if (eo_pk_from_bytes(&c.pk, pkb)) return -1;
-    uint64_t ub = eo_range_upper_bound(range);
-    for (size_t i = 0; i < n; i++) if (values[i] >= ub) return -1;
+    uint64_t max_value = eo_range_max_value(range);
+    for (size_t i = 0; i < n; i++) if (values[i] > max_value) return -1;
     if (eo_prepared_range_init(&c.pr, range)) return -1;
     c.label = label; c.seed = seed; c.first = first; c.values = values; c.cts = cts; c.partials = partials; c.rings = rings;
     parallel_for(gen_range_item, &c, n, threads);

@@ -157,7 +157,8 @@ typedef struct {
 } eo_range;
 
 int      eo_range_optimal(eo_range *out, uint64_t upper_bound);            /* range.rs:148-153 */
-uint64_t eo_range_upper_bound(const eo_range *r);                          /* range.rs:174-181 */
+uint64_t eo_range_upper_bound(const eo_range *r);                          /* range.rs:174-181 (wraps from 2^64 on) */
+uint64_t eo_range_max_value(const eo_range *r);                            /* upper bound - 1, saturated at 2^64 - 1 */
 uint64_t eo_range_rings_size(const eo_range *r);                           /* range.rs:183-186 */
 size_t   eo_range_display(const eo_range *r, char *buf, size_t cap);       /* range.rs:110-124 */
 

@@ -236,7 +236,7 @@ static void g_table_init(void) {
     g_naf8_ready = 1;
 }
 
-#define EO_MAX_TERMS 16
+#define EO_MAX_TERMS 17      /* SumOfSquaresProof::verify with 15 ciphertexts: 15 + 2 terms (proofs.c) */
 
 /* r = sum s_i P_i + g*G  (g may be NULL): Straus with shared doublings */
 static void straus(eo_pt *r, const eo_sc *scalars, const eo_pt *points, size_t n, const eo_sc *g) {
@@ -276,7 +276,11 @@ static void straus(eo_pt *r, const eo_sc *scalars, const eo_pt *points, size_t n
 }
 
 void eo_pt_multi_mul(eo_pt *r, const eo_sc *scalars, const eo_pt *points, size_t n) {
-    straus(r, scalars, points, n, NULL);
+    if (n <= EO_MAX_TERMS) { straus(r, scalars, points, n, NULL); return; }
+    eo_pt rest;                                    /* e.g. PublicKeySet::from_participants with a threshold above 17 */
+    straus(r, scalars, points, EO_MAX_TERMS, NULL);
+    eo_pt_multi_mul(&rest, scalars + EO_MAX_TERMS, points + EO_MAX_TERMS, n - EO_MAX_TERMS);
+    eo_pt_add(r, r, &rest);
 }
 
 void eo_pt_double_mul_generator(eo_pt *r, const eo_sc *a, const eo_pt *A, const eo_sc *b) {

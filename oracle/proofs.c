@@ -328,6 +328,13 @@ uint64_t eo_range_upper_bound(const eo_range *r) {                    /* range.r
     return s + 1;
 }
 
+/* upper bound - 1, with the sum taken in 128 bits: from an upper bound of 2^64 on, every u64 value is in the range */
+uint64_t eo_range_max_value(const eo_range *r) {
+    unsigned __int128 s = 0;
+    for (uint32_t i = 0; i < r->n_rings; i++) s += (unsigned __int128)(r->size[i] - 1) * r->step[i];
+    return s > UINT64_MAX ? UINT64_MAX : (uint64_t)s;
+}
+
 uint64_t eo_range_rings_size(const eo_range *r) {                     /* range.rs:183-186 */
     uint64_t s = 0;
     for (uint32_t i = 0; i < r->n_rings; i++) s += r->size[i];
@@ -382,7 +389,7 @@ int eo_range_prove_prepared(const eo_pk *pk, const eo_prepared_range *pr, uint64
                             const eo_sc *ct_random, eo_transcript *t, eo_rng *rng,
                             eo_ct *partial /* n_rings-1 */, eo_sc *common_challenge, eo_sc *responses) {
     const eo_range *range = &pr->range;
-    if (value >= eo_range_upper_bound(range)) return -1;
+    if (value > eo_range_max_value(range)) return -1;
     size_t indexes[EO_MAX_RINGS];
     char display[EO_MAX_RINGS * 48];
     range_decompose(range, indexes, value);

@@ -4,7 +4,7 @@
 
 #include "eg_oracle.h"
 
-#define EO_MAX_TERMS_SUMSQ 14
+#define EO_MAX_TERMS_SUMSQ 15      /* SumOfSquaresProof / QuadraticVotingBallot: the engine's 1..15 */
 
 typedef struct { eo_pt R, B; } eo_ct;     /* Ciphertext encryption.rs:96-101: (random_element, blinded_element) */
 
