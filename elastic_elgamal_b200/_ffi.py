@@ -122,6 +122,14 @@ PROTOTYPES = {
                                                P8]),
     "eg_prove_decryption_batch": (C.c_int32, [C.c_void_p, C.c_char_p, P8, C.c_size_t, P8, P8, P8, P8, P8]),
     "eg_prove_decryption_batch_seeded": (C.c_int32, [C.c_void_p, C.c_char_p, P8, C.c_size_t, P8, P8, C.c_uint64, P8, P8, P8]),
+    "eg_prove_commitment_equiv_batch": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_size_t, P8, P8, P8, P8, P8, P8, P8]),
+    "eg_prove_commitment_equiv_batch_seeded": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_size_t, P8, P8, P8, C.c_uint64, P8, P8, P8,
+                                                           P8]),
+    "eg_prove_sumsq_batch": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_uint32, C.c_size_t, P8, P8, P8, P8, P8, P8, P8]),
+    "eg_prove_sumsq_batch_seeded": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_uint32, C.c_size_t, P8, P8, P8, P8, P8, P8, C.c_uint64,
+                                                P8]),
+    "eg_prove_possession_batch": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_uint32, C.c_size_t, P8, P8, P8, P8]),
+    "eg_prove_possession_batch_seeded": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_uint32, C.c_size_t, P8, P8, C.c_uint64, P8, P8]),
     "eg_kernel_launch_count": (C.c_uint64, [C.c_void_p]),
     "eg_last_timings": (C.c_int32, [C.c_void_p, C.POINTER(C.c_float * 5)]),
     "eg_ctx_stream": (C.c_void_p, [C.c_void_p]),

@@ -71,6 +71,7 @@ struct eg_ctx {
     int rprove_grid[3] = {0, 0, 0};
     int sumsq_prove_grid = 0, encrypt_grid = 0;
     int decrypt_grid[4] = {0, 0, 0, 0};     // k_decrypt<op, ct>: index 2 op + ct
+    int ceq_prove_grid = 0, pop_prove_grid[2] = {0, 0};
     dev_buf ring_scratch;
     // per-call narrow fixed-base tables of the participant keys of a key set (api_sharing.inc), cached by key bytes
     dev_buf xtab;
@@ -502,6 +503,60 @@ static eg_status launch_sumsq_prove(eg_ctx *ctx, const sumsq_prove_params &P) {
     k_sumsq_prove<<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P);
 #endif
     ctx->launches++;
+    return EG_SUCCESS;
+}
+
+static eg_status launch_sumsq_stage(eg_ctx *ctx, const sumsq_stage_params &P) {
+#ifdef EG_HOSTSIM
+    EG_FOR_HOST(P.n, sumsq_stage_body(P, tid))
+#else
+    k_sumsq_stage<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
+#endif
+    ctx->launches++;
+    return EG_SUCCESS;
+}
+
+#ifndef EG_HOSTSIM
+// resident threads of a persistent grid of `kernel` (cached in `grid_cache`)
+template <class K>
+static eg_status persistent_grid(eg_ctx *ctx, K kernel, int threads, int &grid_cache, const char *name) {
+    if (grid_cache == 0) {
+        int per_sm = 0, sms = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0));
+        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
+        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, (std::string(name) + " does not fit on an SM").c_str());
+        grid_cache = per_sm * sms;
+    }
+    return EG_SUCCESS;
+}
+#endif
+
+static eg_status launch_ceq_prove(eg_ctx *ctx, const ceq_prove_params &P) {
+#ifdef EG_HOSTSIM
+    EG_FOR_HOST(P.n, ceq_prove_body(P, tid))
+#else
+    TRY(persistent_grid(ctx, k_ceq_prove, EG_DECRYPT_THREADS, ctx->ceq_prove_grid, "k_ceq_prove"));
+    const unsigned grid = (unsigned)std::min<size_t>((size_t)ctx->ceq_prove_grid, (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS);
+    k_ceq_prove<<<grid, EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
+#endif
+    ctx->launches++;
+    return EG_SUCCESS;
+}
+
+static eg_status launch_pop_prove(eg_ctx *ctx, const pop_prove_params &P) {
+#ifdef EG_HOSTSIM
+    EG_FOR_HOST(P.n * (size_t)P.k, pop_key_body(P, tid % P.n, (uint32_t)(tid / P.n)))
+    EG_FOR_HOST(P.n, pop_final_body(P, tid))
+#else
+    TRY(persistent_grid(ctx, k_pop_prove<0>, EG_DECRYPT_THREADS, ctx->pop_prove_grid[0], "k_pop_prove"));
+    TRY(persistent_grid(ctx, k_pop_prove<1>, EG_DECRYPT_THREADS, ctx->pop_prove_grid[1], "k_pop_prove"));
+    const size_t t0 = P.n * (size_t)P.k;
+    k_pop_prove<0><<<(unsigned)std::min<size_t>((size_t)ctx->pop_prove_grid[0], (t0 + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS),
+                     EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
+    k_pop_prove<1><<<(unsigned)std::min<size_t>((size_t)ctx->pop_prove_grid[1], (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS),
+                     EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
+#endif
+    ctx->launches += 2;
     return EG_SUCCESS;
 }
 
@@ -1037,5 +1092,7 @@ extern "C" eg_status eg_ctx_set_blinding_base(eg_ctx *ctx, const uint8_t base[32
 #include "api_decrypt.inc"
 
 #include "api_decrypt_side.inc"
+
+#include "api_sigma_provers.inc"
 
 #include "api_multi.inc"

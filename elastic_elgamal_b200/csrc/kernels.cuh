@@ -1877,6 +1877,197 @@ EG_HD void decrypt_body(const decrypt_params &P, size_t item) {
     P.flags[item] = 1;
 }
 
+// ------------------------------------------------------------------ proving side: CommitmentEquivalenceProof::new
+//
+// CommitmentEquivalenceProof::new (commitment.rs:126-196) for a ciphertext (R, B) = ([r]G, [v]G + [r]K) whose value v and
+// randomness r the caller holds.  Draws: the commitment blinding b (SecretKey::generate), then the nonces e_r, e_v, e_c.
+// Every point is fixed-base: R, B, C = [v]G + [b]H, [e_r]G, [e_v]G + [e_r]K, [e_v]G + [e_c]H; the six encodings share one
+// inversion (ge_double_compress_n on the half-scalar points).  R and B are always computed because the transcript absorbs
+// them; `cts` only decides whether they are written.  One thread per item.
+struct ceq_prove_params {
+    size_t n;
+    const uint64_t *values;              // n
+    const uint8_t *ct_r;                 // n * 32: canonical scalars (validated on the host)
+    const uint8_t *wide;                 // caller-supplied blocks: n * 4 * 64
+    uint8_t *cts;                        // n * 64 or null
+    uint8_t *commitments;                // n * 32
+    uint8_t *proofs;                     // n * 128 = c | s_r | s_v | s_c
+    uint8_t *blindings;                  // n * 32 (secret)
+    transcript prefix;                   // Transcript::new(label) + start_proof("commitment_equivalence") + "K"
+    const uint32_t *table_g, *table_k, *table_h;
+    rand_src rnd;
+};
+
+EG_HD void ceq_prove_body(const ceq_prove_params &P, size_t item) {
+    const bool ct = P.rnd.ct != 0;
+    uint32_t w[16];
+    sc r, b, er, ev, ec, s;
+    const sc v = sc_from_u64(P.values[item]);
+    load32_bytes(w, P.ct_r + item * 32);
+    if (!sc_from_words(r, w)) r = sc_zero();
+    const uint8_t *blk = P.wide + item * 4 * 64;
+    rand_block(w, P.rnd, item, 0, blk);
+    sc_from_wide_words(b, w);
+    rand_block(w, P.rnd, item, 1, blk + 64);
+    sc_from_wide_words(er, w);
+    rand_block(w, P.rnd, item, 2, blk + 128);
+    sc_from_wide_words(ev, w);
+    rand_block(w, P.rnd, item, 3, blk + 192);
+    sc_from_wide_words(ec, w);
+    ge_ext q[6];
+    {
+        sc hr, hv, hb;
+        sc_half(hr, r);
+        sc_half(hv, v);
+        sc_half(hb, b);
+        ge_eval_fixed(q[0], 1, P.table_g, hr, P.table_g, hr, ct);          // R = [r]G
+        ge_eval_fixed(q[1], 2, P.table_k, hr, P.table_g, hv, ct);          // B = [r]K + [v]G
+        ge_eval_fixed(q[2], 2, P.table_h, hb, P.table_g, hv, ct);          // C = [b]H + [v]G
+    }
+    {
+        sc her, hev, hec;
+        sc_half(her, er);
+        sc_half(hev, ev);
+        sc_half(hec, ec);
+        ge_eval_fixed(q[3], 1, P.table_g, her, P.table_g, her, ct);        // [e_r]G
+        ge_eval_fixed(q[4], 2, P.table_k, her, P.table_g, hev, ct);        // [e_v]G + [e_r]K
+        ge_eval_fixed(q[5], 2, P.table_h, hec, P.table_g, hev, ct);        // [e_v]G + [e_c]H
+    }
+    uint32_t enc[6][8];
+    ge_double_compress_n<6>(enc, q);
+    transcript t = P.prefix;
+    merlin_append_words(t, EG_LBL("R"), enc[0], 8);
+    merlin_append_words(t, EG_LBL("B"), enc[1], 8);
+    merlin_append_words(t, EG_LBL("C"), enc[2], 8);
+    merlin_append_words(t, EG_LBL("[e_r]G"), enc[3], 8);
+    merlin_append_words(t, EG_LBL("[e_v]G + [e_r]K"), enc[4], 8);
+    merlin_append_words(t, EG_LBL("[e_v]G + [e_c]H"), enc[5], 8);
+    sc c;
+    merlin_challenge_scalar(t, EG_LBL("c"), c);
+    uint8_t *out = P.proofs + item * 128;
+    store32_bytes(out, c.v);
+    sc_muladd(s, c, r, er);
+    store32_bytes(out + 32, s.v);
+    sc_muladd(s, c, v, ev);
+    store32_bytes(out + 64, s.v);
+    sc_muladd(s, c, b, ec);
+    store32_bytes(out + 96, s.v);
+    store32_bytes(P.commitments + item * 32, enc[2]);
+    store32_bytes(P.blindings + item * 32, b.v);
+    if (P.cts) {
+        store32_bytes(P.cts + item * 64, enc[0]);
+        store32_bytes(P.cts + item * 64 + 32, enc[1]);
+    }
+}
+
+// ------------------------------------------------------------------ proving side: Keypair::from + ProofOfPossession::from_keys
+//
+// possession.rs:93-130 over k key pairs per proof, the public keys derived here ([s_j]G, so a key cannot mismatch its secret).
+// One nonce draw x_j per key, in key order.  Phase 0, one thread per (item, key j): encode([s_j]G) into `keys`, encode([x_j]G)
+// into planar scratch (index j over n items).  Phase 1, one thread per item: transcript start_proof("multi_pop"), "K" x k,
+// "R" x k, challenge c; the responses c s_j + x_j re-draw x_j, so no nonce is ever stored.
+struct pop_prove_params {
+    size_t n;
+    uint32_t k;                          // keys per proof, 1..64
+    const uint8_t *secrets;              // n * k * 32: canonical scalars (validated on the host)
+    const uint8_t *wide;                 // caller-supplied blocks: n * k * 64
+    uint8_t *keys;                       // n * k * 32
+    uint8_t *proofs;                     // n * (1 + k) * 32 = c | s_0 .. s_{k-1}
+    uint32_t *enc;                       // planar encodings, index j over n items: [x_j]G
+    transcript prefix;                   // Transcript::new(label) + start_proof("multi_pop")
+    const uint32_t *table_g;
+    rand_src rnd;
+};
+
+EG_HD void pop_nonce(sc &x, const pop_prove_params &P, size_t item, uint32_t j) {
+    uint32_t w[16];
+    rand_block(w, P.rnd, item, j, P.wide + (item * P.k + j) * 64);
+    sc_from_wide_words(x, w);
+}
+
+EG_HD void pop_key_body(const pop_prove_params &P, size_t item, uint32_t j) {
+    const bool ct = P.rnd.ct != 0;
+    uint32_t w[8], enc[2][8];
+    sc s, x, hs, hx;
+    load32_bytes(w, P.secrets + (item * P.k + j) * 32);
+    if (!sc_from_words(s, w)) s = sc_zero();
+    pop_nonce(x, P, item, j);
+    sc_half(hs, s);
+    sc_half(hx, x);
+    ge_ext q[2];
+    ge_eval_fixed(q[0], 1, P.table_g, hs, P.table_g, hs, ct);
+    ge_eval_fixed(q[1], 1, P.table_g, hx, P.table_g, hx, ct);
+    ge_double_compress_n<2>(enc, q);
+    store32_bytes(P.keys + (item * P.k + j) * 32, enc[0]);
+    planar_store_words(P.enc, P.n, j, 8, item, enc[1]);
+}
+
+EG_HD void pop_final_body(const pop_prove_params &P, size_t item) {
+    transcript t = P.prefix;
+    uint32_t w[8];
+#pragma unroll 1
+    for (uint32_t j = 0; j < P.k; j++) {
+        load32_bytes(w, P.keys + (item * P.k + j) * 32);
+        merlin_append_words(t, EG_LBL("K"), w, 8);
+    }
+#pragma unroll 1
+    for (uint32_t j = 0; j < P.k; j++) {
+        planar_load_words(w, P.enc, P.n, j, 8, item);
+        merlin_append_words(t, EG_LBL("R"), w, 8);
+    }
+    sc c;
+    merlin_challenge_scalar(t, EG_LBL("c"), c);
+    uint8_t *out = P.proofs + item * (1 + (size_t)P.k) * 32;
+    store32_bytes(out, c.v);
+#pragma unroll 1
+    for (uint32_t j = 0; j < P.k; j++) {
+        sc s, x, resp;
+        load32_bytes(w, P.secrets + (item * P.k + j) * 32);
+        if (!sc_from_words(s, w)) s = sc_zero();
+        pop_nonce(x, P, item, j);
+        sc_muladd(resp, c, s, x);
+        store32_bytes(out + 32 * (1 + (size_t)j), resp.v);
+    }
+}
+
+// ------------------------------------------------------------------ SumOfSquaresProof::new on its own: input staging
+//
+// k_sumsq_prove reads an item's ciphertexts and sum ciphertext from one record (ct_stride apart) and the randomness as
+// planar scalars.  One thread per item packs the caller's flat arrays into that shape: records of (m + 1) * 64 B
+// (m ciphertexts, then the sum ciphertext), r_i planar over n * m items, r_z planar over n items.
+struct sumsq_stage_params {
+    size_t n;
+    uint32_t m;
+    const uint8_t *cts;                  // n * m * 64
+    const uint8_t *sum_cts;              // n * 64
+    const uint8_t *r;                    // n * m * 32
+    const uint8_t *r_sum;                // n * 32
+    uint8_t *records;                    // n * (m + 1) * 64
+    uint32_t *r_planar;                  // planar scalars over n * m items
+    uint32_t *r_sum_planar;              // planar scalars over n items
+};
+
+EG_HD void sumsq_stage_body(const sumsq_stage_params &P, size_t item) {
+    uint32_t w[8];
+    uint8_t *rec = P.records + item * (P.m + 1) * 64;
+#pragma unroll 1
+    for (uint32_t i = 0; i < P.m; i++) {
+        const size_t q = item * P.m + i;
+        load32_bytes(w, P.cts + q * 64);
+        store32_bytes(rec + 64 * (size_t)i, w);
+        load32_bytes(w, P.cts + q * 64 + 32);
+        store32_bytes(rec + 64 * (size_t)i + 32, w);
+        load32_bytes(w, P.r + q * 32);
+        planar_store_words(P.r_planar, P.n * P.m, 0, 8, q, w);
+    }
+    load32_bytes(w, P.sum_cts + item * 64);
+    store32_bytes(rec + 64 * (size_t)P.m, w);
+    load32_bytes(w, P.sum_cts + item * 64 + 32);
+    store32_bytes(rec + 64 * (size_t)P.m + 32, w);
+    load32_bytes(w, P.r_sum + item * 32);
+    planar_store_words(P.r_sum_planar, P.n, 0, 8, item, w);
+}
+
 
 // QuadraticVotingBallot::verify precedence (quadratic_voting.rs:291-329): malformed anywhere, then the first failing
 // vote range proof (Variant{i}), then the credit range proof, then the sum-of-squares proof.

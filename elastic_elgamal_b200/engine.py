@@ -511,6 +511,61 @@ class Engine:
                                                            _addr(wide_rand), _addr(dh), _addr(proofs), _addr(ok)))
         return dh, proofs, ok.astype(bool)
 
+    # ---- provers of the stand-alone sigma proofs (randomness: `wide_rand` blocks or `seed=`, as for encrypt_*)
+    def prove_commitment_equiv(self, label, values, ct_randomness, wide_rand=None, seed=None, counter_base=0, want_cts=True):
+        """CommitmentEquivalenceProof::new on existing ciphertexts: (cts or None, commitments, proofs, blindings).  Four
+        blocks per item (blinding, e_r, e_v, e_c); blindings are secret."""
+        values = np.ascontiguousarray(values, dtype=np.uint64).reshape(-1)
+        n = values.shape[0]
+        ct_randomness = _u8(ct_randomness, (n, 32))
+        cts = np.empty((n, 64), np.uint8) if want_cts else None
+        commitments, proofs, blindings = np.empty((n, 32), np.uint8), np.empty((n, 128), np.uint8), np.empty((n, 32), np.uint8)
+        if seed is not None:
+            self._check(self.lib.eg_prove_commitment_equiv_batch_seeded(self.h, label.encode(), n, _addr(values), _addr(ct_randomness),
+                                                                        _addr(self._seed(seed)), counter_base, _addr(cts),
+                                                                        _addr(commitments), _addr(proofs), _addr(blindings)))
+        else:
+            wide_rand = _u8(wide_rand, (n, 4, 64))
+            self._check(self.lib.eg_prove_commitment_equiv_batch(self.h, label.encode(), n, _addr(values), _addr(ct_randomness),
+                                                                 _addr(wide_rand), _addr(cts), _addr(commitments), _addr(proofs),
+                                                                 _addr(blindings)))
+        return cts, commitments, proofs, blindings
+
+    def prove_sumsq(self, label, cts, values, randomness, sum_cts, sum_randomness, wide_rand=None, seed=None, counter_base=0):
+        """SumOfSquaresProof::new: cts (n, count, 64) with their values (n, count) and randomness (n, count, 32); sum_cts (n, 64)
+        with sum_randomness (n, 32).  Returns the proofs (n, 2 count + 2, 32)."""
+        cts = _u8(cts)
+        n, m = cts.shape[0], cts.shape[1]
+        cts = cts.reshape(n, m, 64)
+        values = np.ascontiguousarray(values, dtype=np.uint64).reshape(n, m)
+        randomness, sum_cts, sum_randomness = _u8(randomness, (n, m, 32)), _u8(sum_cts, (n, 64)), _u8(sum_randomness, (n, 32))
+        proofs = np.empty((n, 2 * m + 2, 32), np.uint8)
+        if seed is not None:
+            self._check(self.lib.eg_prove_sumsq_batch_seeded(self.h, label.encode(), m, n, _addr(cts), _addr(values), _addr(randomness),
+                                                             _addr(sum_cts), _addr(sum_randomness), _addr(self._seed(seed)),
+                                                             counter_base, _addr(proofs)))
+        else:
+            wide_rand = _u8(wide_rand, (n, 1 + 2 * m, 64))
+            self._check(self.lib.eg_prove_sumsq_batch(self.h, label.encode(), m, n, _addr(cts), _addr(values), _addr(randomness),
+                                                      _addr(sum_cts), _addr(sum_randomness), _addr(wide_rand), _addr(proofs)))
+        return proofs
+
+    def prove_possession(self, label, secrets, wide_rand=None, seed=None, counter_base=0):
+        """Keypair::from + ProofOfPossession::from_keys: secrets (n, k, 32) -> (keys (n, k, 32), proofs (n, 1 + k, 32)).
+        One block per key."""
+        secrets = _u8(secrets)
+        n, k = secrets.shape[0], secrets.shape[1]
+        secrets = secrets.reshape(n, k, 32)
+        keys, proofs = np.empty((n, k, 32), np.uint8), np.empty((n, 1 + k, 32), np.uint8)
+        if seed is not None:
+            self._check(self.lib.eg_prove_possession_batch_seeded(self.h, label.encode(), k, n, _addr(secrets), _addr(self._seed(seed)),
+                                                                  counter_base, _addr(keys), _addr(proofs)))
+        else:
+            wide_rand = _u8(wide_rand, (n, k, 64))
+            self._check(self.lib.eg_prove_possession_batch(self.h, label.encode(), k, n, _addr(secrets), _addr(wide_rand), _addr(keys),
+                                                           _addr(proofs)))
+        return keys, proofs
+
     # ---- device-pointer variants (ints are raw device addresses, e.g. torch.Tensor.data_ptr())
     def decrypt_share_dev(self, keyset, index, secret, n, d_cts, d_shares, d_proofs, d_ok, d_wide_rand=None, seed=None, counter_base=0):
         sec, seed = self._secret(secret), (self._seed(seed) if seed is not None else None)

@@ -439,6 +439,56 @@ eg_status eg_prove_decryption_batch_seeded(eg_ctx *ctx, const char *transcript_l
                                            const uint8_t *cts, const uint8_t seed[32], uint64_t counter_base, uint8_t *dh_elements,
                                            uint8_t *proofs, uint8_t *ok);
 
+/* ---- provers of the stand-alone sigma proofs -------------------------------------------------------
+ * Both randomness forms, as for the encryption side: caller-supplied 64-byte blocks in the draw order given below, or
+ * `_seeded`, where item i's draw k is the ChaCha20 block counter_base + (i << 20) + k.  Each block is reduced as
+ * Ristretto::generate_scalar does; both forms give identical bytes for identical blocks.  The secret scalars (values,
+ * randomness, blindings, nonces, possession secrets) follow eg_ctx_set_prover_mode, outputs are byte-identical in both modes,
+ * and every device buffer that held one of them, or a secret output, is zeroed before the call returns.  A scalar input that
+ * is not canonical is EG_ERR_INVALID_ARG, checked before any work.  On a multi-device context the batch is sharded; item i
+ * keeps its own randomness either way. */
+
+/* CommitmentEquivalenceProof::new (src/proofs/commitment.rs:126-196) on ciphertexts that exist already (CiphertextWithValue:
+ * cts[i] = ([r]G, [v]G + [r]K) with v = values[i], r = ct_randomness[i]), with `Transcript::new(label)`.  Four blocks per
+ * item: the commitment blinding b, then the nonces e_r, e_v, e_c.  commitments[i] = [v]G + [b]H (H: eg_ctx_set_blinding_base),
+ * proofs[i] = challenge | c r + e_r | c v + e_v | c b + e_c (the layout eg_verify_commitment_equiv_batch reads), blindings[i]
+ * = b, the SecretKey that `new` returns (a SECRET output).  cts (optional, may be NULL) receives the re-encryption ([r]G,
+ * [v]G + [r]K) for checking.  Needs the receiver key and the blinding base (EG_ERR_NO_RECEIVER otherwise). */
+eg_status eg_prove_commitment_equiv_batch(eg_ctx *ctx, const char *transcript_label, size_t n, const uint64_t *values /* n */,
+                                          const uint8_t *ct_randomness /* n*32 */, const uint8_t *wide_rand /* n*4*64 */,
+                                          uint8_t *cts /* n*64 or NULL */, uint8_t *commitments /* n*32 */,
+                                          uint8_t *proofs /* n*128 */, uint8_t *blindings /* n*32 */);
+eg_status eg_prove_commitment_equiv_batch_seeded(eg_ctx *ctx, const char *transcript_label, size_t n, const uint64_t *values,
+                                                 const uint8_t *ct_randomness, const uint8_t seed[32], uint64_t counter_base,
+                                                 uint8_t *cts /* or NULL */, uint8_t *commitments, uint8_t *proofs, uint8_t *blindings);
+
+/* SumOfSquaresProof::new (src/proofs/mul.rs:107-181) on its own, with `Transcript::new(label)` and the receiver key: item i
+ * proves that sum_cts[i] (randomness sum_randomness[i]) encrypts the sum of the squares of the values encrypted by its
+ * `count` ciphertexts (1..15; cts[i*count + j] with value values[i*count + j] and randomness randomness[i*count + j]).
+ * 1 + 2 count blocks per item: e_z, then (e_r,j, e_x,j) per ciphertext.  Proof layout as eg_verify_sumsq_batch reads:
+ * challenge | (r_resp, x_resp) x count | sum_resp.  As in the reference, the prover does not check that the ciphertexts match
+ * the values and randomness: an inconsistent item yields a proof that the verifiers reject. */
+eg_status eg_prove_sumsq_batch(eg_ctx *ctx, const char *transcript_label, uint32_t count, size_t n,
+                               const uint8_t *cts /* n*count*64 */, const uint64_t *values /* n*count */,
+                               const uint8_t *randomness /* n*count*32 */, const uint8_t *sum_cts /* n*64 */,
+                               const uint8_t *sum_randomness /* n*32 */, const uint8_t *wide_rand /* n*(1+2*count)*64 */,
+                               uint8_t *proofs /* n*(2*count+2)*32 */);
+eg_status eg_prove_sumsq_batch_seeded(eg_ctx *ctx, const char *transcript_label, uint32_t count, size_t n, const uint8_t *cts,
+                                      const uint64_t *values, const uint8_t *randomness, const uint8_t *sum_cts,
+                                      const uint8_t *sum_randomness, const uint8_t seed[32], uint64_t counter_base, uint8_t *proofs);
+
+/* Keypair::from(secret) for each of `keys_per_proof` (1..64) secrets, then ProofOfPossession::from_keys
+ * (src/proofs/possession.rs:93-130) with `Transcript::new(label)`.  keys[i*k + j] = encode([secrets[i*k + j]]G), computed on
+ * the device, so a key cannot mismatch its secret.  One block per key (its nonce), in key order; proofs[i] = challenge |
+ * responses, the layout eg_verify_possession_batch reads.  A zero secret gives what the reference gives: the identity
+ * encoding as the key, and a proof that the verifier refuses as EG_V_MALFORMED.  Needs no receiver key. */
+eg_status eg_prove_possession_batch(eg_ctx *ctx, const char *transcript_label, uint32_t keys_per_proof, size_t n,
+                                    const uint8_t *secrets /* n*k*32 */, const uint8_t *wide_rand /* n*k*64 */,
+                                    uint8_t *keys /* n*k*32 */, uint8_t *proofs /* n*(1+k)*32 */);
+eg_status eg_prove_possession_batch_seeded(eg_ctx *ctx, const char *transcript_label, uint32_t keys_per_proof, size_t n,
+                                           const uint8_t *secrets, const uint8_t seed[32], uint64_t counter_base, uint8_t *keys,
+                                           uint8_t *proofs);
+
 /* ---- device-pointer variants (inputs already resident in HBM; same semantics) ------------------- */
 eg_status eg_verify_bool_batch_dev(eg_ctx *ctx, size_t n, const uint8_t *d_cts, const uint8_t *d_proofs, uint8_t *d_verdicts);
 eg_status eg_verify_choice_batch_dev(eg_ctx *ctx, size_t n, uint32_t options, int single, const uint8_t *d_choices,

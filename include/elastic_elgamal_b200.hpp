@@ -323,6 +323,79 @@ class Engine {
         return split_log_eq(d, p);
     }
 
+    // CommitmentEquivalenceProof::new over a batch of existing ciphertexts of values[i] with randomness ct_randomness[i]
+    // (commitment.rs:126-196), in-kernel randomness.  Needs the receiver key and the blinding base; blindings are secret.
+    struct CommitmentEquivalence { Ciphertext ciphertext; CommitmentEquivalenceProof proof; Element commitment; Scalar blinding; };
+    std::vector<CommitmentEquivalence> prove_commitment_equiv_batch(const std::vector<uint64_t> &values, const std::vector<Scalar> &ct_randomness,
+                                                                    const std::string &label, const Seed &seed) {
+        const size_t n = values.size();
+        if (ct_randomness.size() != n) throw Error(EG_ERR_LEN_MISMATCH, "one randomness per value");
+        std::vector<uint8_t> r, c(64 * n), m(32 * n), p(128 * n), b(32 * n);
+        for (const auto &s : ct_randomness) r.insert(r.end(), s.begin(), s.end());
+        check(eg_prove_commitment_equiv_batch_seeded(ctx_, label.c_str(), n, values.data(), r.data(), seed.key.data(), seed.counter_base, c.data(),
+                                                     m.data(), p.data(), b.data()));
+        std::vector<CommitmentEquivalence> out(n);
+        for (size_t i = 0; i < n; i++) {
+            std::copy_n(&c[64 * i], 32, out[i].ciphertext.random_element.begin());
+            std::copy_n(&c[64 * i + 32], 32, out[i].ciphertext.blinded_element.begin());
+            Scalar *f[4] = {&out[i].proof.challenge, &out[i].proof.randomness_response, &out[i].proof.value_response, &out[i].proof.commitment_response};
+            for (int k = 0; k < 4; k++) std::copy_n(&p[128 * i + 32 * k], 32, f[k]->begin());
+            std::copy_n(&m[32 * i], 32, out[i].commitment.begin());
+            std::copy_n(&b[32 * i], 32, out[i].blinding.begin());
+        }
+        std::fill(b.begin(), b.end(), 0);
+        return out;
+    }
+
+    // SumOfSquaresProof::new over a batch (mul.rs:107-181): item i has `count` ciphertexts cts[i*count..] of values with
+    // randomness, and the sum ciphertext sum_cts[i] with sum_randomness[i]; in-kernel randomness.
+    std::vector<SumOfSquaresProof> prove_sumsq_batch(uint32_t count, const std::vector<Ciphertext> &cts, const std::vector<uint64_t> &values,
+                                                     const std::vector<Scalar> &randomness, const std::vector<Ciphertext> &sum_cts,
+                                                     const std::vector<Scalar> &sum_randomness, const std::string &label, const Seed &seed) {
+        const size_t n = sum_cts.size();
+        if (cts.size() != n * count || values.size() != n * count || randomness.size() != n * count || sum_randomness.size() != n)
+            throw Error(EG_ERR_LEN_MISMATCH, "count ciphertexts, values and randomness per sum ciphertext");
+        std::vector<uint8_t> c, s, r, sr, p(32 * (2 * (size_t)count + 2) * n);
+        for (const auto &ct : cts) append(c, ct);
+        for (const auto &ct : sum_cts) append(s, ct);
+        for (const auto &x : randomness) r.insert(r.end(), x.begin(), x.end());
+        for (const auto &x : sum_randomness) sr.insert(sr.end(), x.begin(), x.end());
+        check(eg_prove_sumsq_batch_seeded(ctx_, label.c_str(), count, n, c.data(), values.data(), r.data(), s.data(), sr.data(), seed.key.data(),
+                                          seed.counter_base, p.data()));
+        std::vector<SumOfSquaresProof> out(n);
+        const uint8_t *q = p.data();
+        for (auto &proof : out) {
+            std::copy_n(q, 32, proof.challenge.begin()); q += 32;
+            proof.ciphertext_responses.resize(2 * (size_t)count);
+            for (auto &x : proof.ciphertext_responses) { std::copy_n(q, 32, x.begin()); q += 32; }
+            std::copy_n(q, 32, proof.sum_response.begin()); q += 32;
+        }
+        return out;
+    }
+
+    // Keypair::from(secret) for keys_per_proof secrets per item, then ProofOfPossession::from_keys (possession.rs:93-130);
+    // in-kernel randomness.  Returns the public keys (item-major) and the proofs.
+    std::pair<std::vector<PublicKey>, std::vector<ProofOfPossession>> prove_possession_batch(uint32_t keys_per_proof, const std::vector<Scalar> &secrets,
+                                                                                          const std::string &label, const Seed &seed) {
+        const size_t k = keys_per_proof;
+        if (k == 0 || secrets.size() % k) throw Error(EG_ERR_LEN_MISMATCH, "keys_per_proof secrets per proof");
+        const size_t n = secrets.size() / k;
+        std::vector<uint8_t> s, keys(32 * k * n), p(32 * (1 + k) * n);
+        for (const auto &x : secrets) s.insert(s.end(), x.begin(), x.end());
+        check(eg_prove_possession_batch_seeded(ctx_, label.c_str(), keys_per_proof, n, s.data(), seed.key.data(), seed.counter_base, keys.data(), p.data()));
+        std::fill(s.begin(), s.end(), 0);
+        std::vector<PublicKey> pks(k * n);
+        for (size_t j = 0; j < k * n; j++) std::copy_n(&keys[32 * j], 32, pks[j].bytes.begin());
+        std::vector<ProofOfPossession> proofs(n);
+        for (size_t i = 0; i < n; i++) {
+            const uint8_t *q = &p[32 * (1 + k) * i];
+            std::copy_n(q, 32, proofs[i].challenge.begin());
+            proofs[i].responses.resize(k);
+            for (size_t j = 0; j < k; j++) std::copy_n(q + 32 * (1 + j), 32, proofs[i].responses[j].begin());
+        }
+        return {pks, proofs};
+    }
+
     // key.encrypt_bool(value, rng) over a batch with in-kernel randomness (keys/impls.rs:77-89)
     std::pair<std::vector<Ciphertext>, std::vector<RingProof>> encrypt_bool_batch(const std::vector<uint8_t> &values, const Seed &seed) {
         const size_t n = values.size();

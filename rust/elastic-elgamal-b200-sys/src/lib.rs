@@ -202,6 +202,23 @@ extern "C" {
     pub fn eg_prove_decryption_batch_seeded(ctx: *mut eg_ctx, transcript_label: *const c_char, secret: *const u8, n: usize,
                                             cts: *const u8, seed: *const u8, counter_base: u64, dh_elements: *mut u8, proofs: *mut u8,
                                             ok: *mut u8) -> eg_status;
+    pub fn eg_prove_commitment_equiv_batch(ctx: *mut eg_ctx, transcript_label: *const c_char, n: usize, values: *const u64,
+                                           ct_randomness: *const u8, wide_rand: *const u8, cts: *mut u8, commitments: *mut u8,
+                                           proofs: *mut u8, blindings: *mut u8) -> eg_status;
+    pub fn eg_prove_commitment_equiv_batch_seeded(ctx: *mut eg_ctx, transcript_label: *const c_char, n: usize, values: *const u64,
+                                                  ct_randomness: *const u8, seed: *const u8, counter_base: u64, cts: *mut u8,
+                                                  commitments: *mut u8, proofs: *mut u8, blindings: *mut u8) -> eg_status;
+    pub fn eg_prove_sumsq_batch(ctx: *mut eg_ctx, transcript_label: *const c_char, count: u32, n: usize, cts: *const u8, values: *const u64,
+                                randomness: *const u8, sum_cts: *const u8, sum_randomness: *const u8, wide_rand: *const u8,
+                                proofs: *mut u8) -> eg_status;
+    pub fn eg_prove_sumsq_batch_seeded(ctx: *mut eg_ctx, transcript_label: *const c_char, count: u32, n: usize, cts: *const u8,
+                                       values: *const u64, randomness: *const u8, sum_cts: *const u8, sum_randomness: *const u8,
+                                       seed: *const u8, counter_base: u64, proofs: *mut u8) -> eg_status;
+    pub fn eg_prove_possession_batch(ctx: *mut eg_ctx, transcript_label: *const c_char, keys_per_proof: u32, n: usize, secrets: *const u8,
+                                     wide_rand: *const u8, keys: *mut u8, proofs: *mut u8) -> eg_status;
+    pub fn eg_prove_possession_batch_seeded(ctx: *mut eg_ctx, transcript_label: *const c_char, keys_per_proof: u32, n: usize,
+                                            secrets: *const u8, seed: *const u8, counter_base: u64, keys: *mut u8, proofs: *mut u8)
+                                            -> eg_status;
 
     pub fn eg_last_kernel_stats(ctx: *const eg_ctx, kind: c_int, launches: *mut u64, tasks: *mut u64, ms: *mut f32) -> eg_status;
     pub fn eg_kernel_launch_count(ctx: *const eg_ctx) -> u64;

@@ -888,6 +888,132 @@ impl Engine {
         ballots.chunks(size).map(|b| Ok(flat::from_flat(b, &lens)?)).collect()
     }
 
+    // ------------------------------------------------------------------ stand-alone sigma provers
+
+    fn scalar_bytes(secrets: &[SecretKey<Ristretto>]) -> Vec<u8> {
+        secrets.iter().flat_map(Self::secret_bytes).collect()
+    }
+
+    fn secret_key(bytes: &[u8]) -> SecretKey<Ristretto> {
+        SecretKey::new(Ristretto::deserialize_scalar(bytes).expect("the engine emits canonical scalars"))
+    }
+
+    /// `CommitmentEquivalenceProof::new(ciphertext_with_value, receiver, blinding_base, &mut Transcript::new(label), rng)`
+    /// over a batch (commitment.rs:126-196) for ciphertexts of `values[i]` with randomness `ct_randomness[i]`; four randomness
+    /// blocks per item (blinding, e_r, e_v, e_c).  Returns the re-encrypted ciphertext, the proof, the commitment
+    /// `[v]G + [b]H` and the blinding `b` (secret).  Needs the receiver key and the blinding base.
+    pub fn prove_commitment_equivalences(
+        &self,
+        transcript_label: &str,
+        values: &[u64],
+        ct_randomness: &[SecretKey<Ristretto>],
+        randomness: Randomness<'_>,
+    ) -> Result<Vec<(Ciphertext<Ristretto>, CommitmentEquivalenceProof<Ristretto>, Element, SecretKey<Ristretto>)>, EngineError> {
+        let n = values.len();
+        assert_eq!(ct_randomness.len(), n);
+        let r = Self::scalar_bytes(ct_randomness);
+        let label = CString::new(transcript_label).map_err(|_| EngineError { status: sys::EG_ERR_INVALID_ARG, message: "label contains NUL".into() })?;
+        let (mut cts, mut coms, mut proofs, mut blind) = (vec![0_u8; n * 64], vec![0_u8; n * 32], vec![0_u8; n * 128], vec![0_u8; n * 32]);
+        self.check(match randomness {
+            Randomness::Blocks(wide) => {
+                assert_eq!(wide.len(), n * 4 * 64);
+                unsafe {
+                    sys::eg_prove_commitment_equiv_batch(self.ctx, label.as_ptr(), n, values.as_ptr(), r.as_ptr(), wide.as_ptr(), cts.as_mut_ptr(),
+                                                         coms.as_mut_ptr(), proofs.as_mut_ptr(), blind.as_mut_ptr())
+                }
+            }
+            Randomness::Seeded { seed, counter_base } => unsafe {
+                sys::eg_prove_commitment_equiv_batch_seeded(self.ctx, label.as_ptr(), n, values.as_ptr(), r.as_ptr(), seed.as_ptr(), counter_base,
+                                                            cts.as_mut_ptr(), coms.as_mut_ptr(), proofs.as_mut_ptr(), blind.as_mut_ptr())
+            },
+        })?;
+        let out = ciphertexts(&cts)
+            .into_iter()
+            .zip(proofs.chunks(128).zip(coms.chunks(32)).zip(blind.chunks(32)))
+            .map(|(ct, ((p, c), b))| Ok((ct, flat::from_flat(p, &[])?, element(c), Self::secret_key(b))))
+            .collect();
+        blind.iter_mut().for_each(|x| *x = 0);
+        out
+    }
+
+    /// `SumOfSquaresProof::new(ciphertexts, sum_of_squares, receiver, &mut Transcript::new(label), rng)` over a batch
+    /// (mul.rs:107-181): item `i` has the `count` ciphertexts `cts[i * count..]` of `values` with `ct_randomness`, and the sum
+    /// ciphertext `sum_cts[i]` with `sum_randomness[i]`; `1 + 2 count` randomness blocks per item.  As in the reference, the
+    /// inputs are not checked against each other: an inconsistent item yields a proof that does not verify.
+    #[allow(clippy::too_many_arguments)]
+    pub fn prove_sums_of_squares(
+        &self,
+        transcript_label: &str,
+        count: usize,
+        cts: &[Ciphertext<Ristretto>],
+        values: &[u64],
+        ct_randomness: &[SecretKey<Ristretto>],
+        sum_cts: &[Ciphertext<Ristretto>],
+        sum_randomness: &[SecretKey<Ristretto>],
+        randomness: Randomness<'_>,
+    ) -> Result<Vec<SumOfSquaresProof<Ristretto>>, EngineError> {
+        let n = sum_cts.len();
+        assert!(cts.len() == n * count && values.len() == n * count && ct_randomness.len() == n * count && sum_randomness.len() == n);
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let s: Vec<u8> = sum_cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let (r, sr) = (Self::scalar_bytes(ct_randomness), Self::scalar_bytes(sum_randomness));
+        let label = CString::new(transcript_label).map_err(|_| EngineError { status: sys::EG_ERR_INVALID_ARG, message: "label contains NUL".into() })?;
+        let stride = 32 * (2 * count + 2);
+        let mut proofs = vec![0_u8; n * stride];
+        self.check(match randomness {
+            Randomness::Blocks(wide) => {
+                assert_eq!(wide.len(), n * (1 + 2 * count) * 64);
+                unsafe {
+                    sys::eg_prove_sumsq_batch(self.ctx, label.as_ptr(), count as u32, n, c.as_ptr(), values.as_ptr(), r.as_ptr(), s.as_ptr(),
+                                              sr.as_ptr(), wide.as_ptr(), proofs.as_mut_ptr())
+                }
+            }
+            Randomness::Seeded { seed, counter_base } => unsafe {
+                sys::eg_prove_sumsq_batch_seeded(self.ctx, label.as_ptr(), count as u32, n, c.as_ptr(), values.as_ptr(), r.as_ptr(), s.as_ptr(),
+                                                 sr.as_ptr(), seed.as_ptr(), counter_base, proofs.as_mut_ptr())
+            },
+        })?;
+        // SumOfSquaresProof { challenge, ciphertext_responses: Vec<Scalar>, sum_response }
+        proofs.chunks(stride).map(|p| Ok(flat::from_flat(p, &[2 * count])?)).collect()
+    }
+
+    /// `Keypair::from(secret)` for each of `keys_per_proof` secrets, then `ProofOfPossession::from_keys(keypairs,
+    /// &mut Transcript::new(label), rng)` (possession.rs:93-130), over a batch; one randomness block per key.  The public keys
+    /// are computed on the device.
+    pub fn prove_possessions(
+        &self,
+        transcript_label: &str,
+        keys_per_proof: usize,
+        secrets: &[SecretKey<Ristretto>],
+        randomness: Randomness<'_>,
+    ) -> Result<Vec<(Vec<PublicKey<Ristretto>>, ProofOfPossession<Ristretto>)>, EngineError> {
+        let k = keys_per_proof;
+        assert!(k > 0 && secrets.len() % k == 0);
+        let n = secrets.len() / k;
+        let s = Self::scalar_bytes(secrets);
+        let label = CString::new(transcript_label).map_err(|_| EngineError { status: sys::EG_ERR_INVALID_ARG, message: "label contains NUL".into() })?;
+        let (mut keys, mut proofs) = (vec![0_u8; n * k * 32], vec![0_u8; n * (1 + k) * 32]);
+        self.check(match randomness {
+            Randomness::Blocks(wide) => {
+                assert_eq!(wide.len(), n * k * 64);
+                unsafe { sys::eg_prove_possession_batch(self.ctx, label.as_ptr(), k as u32, n, s.as_ptr(), wide.as_ptr(), keys.as_mut_ptr(), proofs.as_mut_ptr()) }
+            }
+            Randomness::Seeded { seed, counter_base } => unsafe {
+                sys::eg_prove_possession_batch_seeded(self.ctx, label.as_ptr(), k as u32, n, s.as_ptr(), seed.as_ptr(), counter_base,
+                                                      keys.as_mut_ptr(), proofs.as_mut_ptr())
+            },
+        })?;
+        keys.chunks(32 * k)
+            .zip(proofs.chunks(32 * (1 + k)))
+            .zip(secrets.chunks(k))
+            .map(|((ks, p), sec)| {
+                // a zero secret's key is the identity, which PublicKey::from_bytes refuses: take Keypair::from's key then
+                let keys = ks.chunks(32).zip(sec).map(|(b, s)| PublicKey::from_bytes(b).unwrap_or_else(|_| PublicKey::from(s))).collect();
+                Ok((keys, flat::from_flat(p, &[k])?))
+            })
+            .collect()
+    }
+
     /// Raw pass-through for objects a caller already holds in the flat layouts (e.g. straight from storage).
     pub fn raw(&self) -> *mut sys::eg_ctx {
         self.ctx
