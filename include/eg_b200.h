@@ -211,7 +211,8 @@ eg_status eg_range_optimal(uint64_t upper_bound, eg_range *out);
 size_t    eg_range_display(const eg_range *range, char *buf, size_t cap);
 
 /* PublicKey::verify_range (src/keys/impls.rs:143-151) -> RangeProof::verify (src/proofs/range.rs:547-577);
- * `transcript_label` is the Transcript::new label ("ciphertext_range" for verify_range). */
+ * `transcript_label` is the Transcript::new label ("ciphertext_range" for verify_range).  Here and in every other entry
+ * point that takes one, a transcript label is a NUL-terminated string of 1..255 bytes; anything else is EG_ERR_INVALID_ARG. */
 eg_status eg_verify_range_batch(eg_ctx *ctx, const eg_range *range, const char *transcript_label, size_t n,
                                 const uint8_t *cts /* n*64 */, const uint8_t *partial_cts /* n*(n_rings-1)*64 */,
                                 const uint8_t *ring_proofs /* n*(1+sum(size))*32 */, uint8_t *verdicts /* n */);
