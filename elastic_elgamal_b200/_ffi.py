@@ -89,6 +89,8 @@ PROTOTYPES = {
     "eg_keysets_validate_batch": (C.c_int32, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, P8, P8, P8]),
     "eg_dlog_table_create": (C.c_int32, [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_void_p)]),
     "eg_dlog_table_destroy": (None, [C.c_void_p]),
+    "eg_dlog_table_create_bsgs": (C.c_int32, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(C.c_void_p)]),
+    "eg_dlog_lookup_batch": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_size_t, P8, P8, P8]),
     "eg_combine_decrypt_batch": (C.c_int32, [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_size_t, C.c_uint32, P8, P8, C.c_void_p, P8, P8]),
     "eg_verify_qv_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(QvParams), C.c_size_t, P8, P8, P8]),
     "eg_verify_shares_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(KeySet), C.c_size_t, C.c_uint32, C.POINTER(C.c_uint32), P8, P8, P8, P8]),

@@ -92,7 +92,10 @@ struct eg_ctx {
 
 struct eg_dlog_table {
     eg_ctx *ctx;
-    uint64_t lo, hi;
+    uint64_t lo, hi;      // the whole range [lo, hi)
+    uint64_t m;           // baby steps: the device table holds [lo, lo + min(m, hi - lo))
+    uint64_t giants;      // ceil((hi - lo) / m); 1: a range table, no giant-step walk
+    uint32_t step[24];    // giants > 1: -[m/2]G in affine Niels form (dlog_walk_params::step)
     size_t cap;
     uint32_t *d_keys;     // cap * 8 words
     uint64_t *d_vals;     // cap
@@ -827,6 +830,51 @@ static void launch_dlog_lookup(eg_ctx *ctx, const dlog_lookup_params &P) {
     EG_FOR_HOST(P.n, dlog_lookup_body(P, tid))
 #else
     k_dlog_lookup<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
+#endif
+    ctx->launches++;
+}
+
+static void launch_dlog_get(eg_ctx *ctx, const dlog_get_params &P) {
+#ifdef EG_HOSTSIM
+    EG_FOR_HOST(P.n, dlog_get_body(P, tid))
+#else
+    k_dlog_get<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
+#endif
+    ctx->launches++;
+}
+
+// Giant-step walk of a BSGS table (giants > 1) over the items that the probe of giant step 0 left at found 0.  Each item gets
+// `segs` threads of seg_steps consecutive steps: enough threads in all to fill the GPU when the batch is small (one element
+// spreads over the whole device), one per item when the batch alone fills it, and never fewer than EG_WALK_MIN_STEPS steps
+// per thread, which keep the cost of a thread's start ([1/2]M and one fixed-base product, about 3 000 field operations)
+// small against its walk.
+#ifdef EG_HOSTSIM
+#define EG_WALK_MIN_STEPS 16           // the CPU harness: short segments, so that small tables cross segment boundaries
+#define EG_WALK_TARGET_THREADS 64
+#else
+#define EG_WALK_MIN_STEPS 2048
+#define EG_WALK_TARGET_THREADS (1u << 18)
+#endif
+static void launch_dlog_walk(eg_ctx *ctx, const eg_dlog_table *t, size_t n, const uint8_t *enc, uint64_t *values, uint8_t *found) {
+    if (t->giants <= 1 || n == 0) return;
+    dlog_walk_params P;
+    memset(&P, 0, sizeof P);
+    const uint64_t steps = t->giants - 1;
+    const uint64_t max_segs = (steps + EG_WALK_MIN_STEPS - 1) / EG_WALK_MIN_STEPS;
+    const uint64_t want = std::max<uint64_t>(1, (EG_WALK_TARGET_THREADS + n - 1) / n);
+    uint64_t segs = std::max<uint64_t>(1, std::min(max_segs, want));
+    P.seg_steps = (steps + segs - 1) / segs;
+    P.seg_steps = (P.seg_steps + EG_WALK_BLOCK - 1) / EG_WALK_BLOCK * EG_WALK_BLOCK;
+    segs = (steps + P.seg_steps - 1) / P.seg_steps;
+    P.n = n; P.enc = enc; P.found = found; P.values = (unsigned long long *)values;
+    P.lo = t->lo; P.hi = t->hi; P.m = t->m; P.giants = t->giants; P.segs = (uint32_t)segs;
+    P.cap = t->cap; P.keys = t->d_keys; P.vals = (const unsigned long long *)t->d_vals; P.table_g = ctx->d_table_g;
+    for (int w = 0; w < 24; w++) P.step[w] = t->step[w];
+    const size_t total = n * (size_t)segs;
+#ifdef EG_HOSTSIM
+    EG_FOR_HOST(total, dlog_walk_body(P, tid))
+#else
+    k_dlog_walk<<<grid_for(total, EG_DECRYPT_THREADS), EG_DECRYPT_THREADS, 0, ctx->stream>>>(P, total);
 #endif
     ctx->launches++;
 }

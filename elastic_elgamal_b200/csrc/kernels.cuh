@@ -1749,6 +1749,7 @@ struct dlog_lookup_params {
     const uint32_t *flags;      // malformed inputs
     unsigned long long *values;
     uint8_t *found;             // 1 found, 0 absent, 2 malformed input
+    uint8_t *enc;               // n * 32 or null: the encoding of M (read by the giant-step walk of a BSGS table)
 };
 
 // DiscreteLogTable::get (encryption.rs:287-297) on a non-identity element's encoding `w`: 1 and `value` when present, 0 absent
@@ -1773,9 +1774,115 @@ EG_HD void dlog_lookup_body(const dlog_lookup_params &P, size_t item) {
     if (ge_is_identity(M)) { P.found[item] = 1; P.values[item] = 0; return; }
     uint32_t w[8];
     ge_encode(w, M);
+    if (P.enc) store32_bytes(P.enc + item * 32, w);
     unsigned long long v = 0;
     P.found[item] = dlog_probe(w, P.cap, P.keys, P.vals, v);
     P.values[item] = v;
+}
+
+// DiscreteLogTable::get (encryption.rs:287-297) on caller-supplied element encodings: 2 when the encoding does not decode,
+// 1 / 0 for the identity, else the table probe
+struct dlog_get_params {
+    size_t n;
+    const uint8_t *enc;         // n * 32
+    size_t cap;
+    const uint32_t *keys;
+    const unsigned long long *vals;
+    unsigned long long *values;
+    uint8_t *found;
+};
+
+EG_HD void dlog_get_body(const dlog_get_params &P, size_t item) {
+    uint32_t w[8];
+    load32_bytes(w, P.enc + item * 32);
+    ge_ext M;
+    unsigned long long v = 0;
+    uint8_t f = 1;
+    if (!ge_decode(M, w)) f = 2;
+    else if (!ge_is_identity(M)) f = dlog_probe(w, P.cap, P.keys, P.vals, v);
+    P.found[item] = f;
+    P.values[item] = v;
+}
+
+// DiscreteLogTable::get over [lo, hi) by baby-step giant-step:the table holds the baby steps [lo, lo + m) and
+// v = u + j m (u in [lo, lo + m), j < giants) is found by probing P_j = M - [j m]G.  Giant step 0 is the ordinary probe
+// (dlog_lookup_body / decrypt_body); this walk takes the items it left at found 0 (decoded, absent) through j = 1 .. giants - 1.
+// Thread (item, seg) walks j in [1 + seg * seg_steps, ...) on the half points Q_j = [1/2] P_j, so a block of
+// EG_WALK_BLOCK steps is encoded with one inversion and no square root (ge_double_compress_n: encode(2 Q_j) = encode(P_j)).
+// A hit sets found[item] = 1, which the item's other segments poll once per block to stop early.  Only one (u, j) can
+// match (v < 2^64 < l), so any thread that finds it may write the result.
+#define EG_WALK_BLOCK 8
+struct dlog_walk_params {
+    size_t n;
+    const uint8_t *enc;         // n * 32: encodings of M (items at found != 0 are not read)
+    uint8_t *found;             // n: 0 = unresolved so far; set to 1 on a hit
+    unsigned long long *values; // n
+    uint64_t lo, hi, m, giants; // giants = ceil((hi - lo) / m) >= 2
+    uint64_t seg_steps;         // giant steps per thread (a multiple of EG_WALK_BLOCK)
+    uint32_t segs;              // threads per item
+    size_t cap;
+    const uint32_t *keys;
+    const unsigned long long *vals;
+    const uint32_t *table_g;    // wide fixed-base table of G
+    uint32_t step[24];          // -[m/2]G, affine Niels form
+};
+
+EG_HD uint8_t dlog_walk_poll(const uint8_t *found, size_t item) { return *(const volatile uint8_t *)(found + item); }
+
+EG_HD void dlog_walk_body(const dlog_walk_params &P, size_t tid) {
+    const size_t item = tid % P.n;
+    const uint64_t seg = tid / P.n;
+    const uint64_t j0 = 1 + seg * P.seg_steps;
+    if (j0 >= P.giants || dlog_walk_poll(P.found, item) != 0) return;
+    const uint64_t j1 = P.giants - j0 > P.seg_steps ? j0 + P.seg_steps : P.giants;
+    uint32_t w[8];
+    load32_bytes(w, P.enc + item * 32);
+    ge_ext M, H, X, Q;
+    ge_decode(M, w);                                            // decoded before (found 0, not 2)
+    EG_ALIGN16 ge_cached tbl[8];
+    ge_window_table(tbl, M);
+    sc half;
+    sc_half(half, sc_from_u64(1));
+    ge_var_mul(H, tbl, half);                                   // [1/2] M
+    sc c;
+    sc_half(c, sc_from_u64(j0 * P.m));                          // j0 m < 2^32 * 2^28
+    ge_eval_fixed(X, 1, P.table_g, c, P.table_g, c);
+    ge_sub(Q, H, X);                                            // Q_j0 = [1/2] (M - [j0 m]G)
+    ge_niels step;
+    ge_niels_load(step, P.step, 0);
+#pragma unroll 1
+    for (uint64_t jb = j0; jb < j1; jb += EG_WALK_BLOCK) {
+        if (jb != j0 && dlog_walk_poll(P.found, item) != 0) return;
+        ge_ext q[EG_WALK_BLOCK];
+        uint32_t e[EG_WALK_BLOCK][8];
+#pragma unroll 1
+        for (int k = 0; k < EG_WALK_BLOCK; k++) {
+            q[k] = Q;
+            ge_p1p1 t;
+            ge_add_niels_p1p1(t, Q, step, false);
+            ge_p1p1_to_ext(Q, t);
+        }
+        ge_double_compress_n<EG_WALK_BLOCK>(e, q);
+#pragma unroll 1
+        for (int k = 0; k < EG_WALK_BLOCK && jb + k < j1; k++) {
+            const uint64_t jm = (jb + k) * P.m;
+            bool zero = true;
+            for (int i = 0; i < 8; i++) zero = zero && e[k][i] == 0;
+            unsigned long long u = 0;
+            bool hit;
+            if (zero) hit = P.lo == 0;                              // P_j = [0]G: u = 0, never stored in the table
+            else hit = dlog_probe(e[k], P.cap, P.keys, P.vals, u) != 0;
+            const uint64_t v = (uint64_t)u + jm;
+            if (hit && v >= jm && v < P.hi) {                       // v >= jm: u + j m did not pass 2^64
+                P.values[item] = v;
+#if defined(__CUDA_ARCH__)
+                __threadfence();
+#endif
+                *(volatile uint8_t *)(P.found + item) = 1;
+                return;
+            }
+        }
+    }
 }
 
 // ------------------------------------------------------------------ decryption side: the talliers' operations

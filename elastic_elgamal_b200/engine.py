@@ -447,8 +447,19 @@ class Engine:
         self._check(self.lib.eg_keysets_validate_batch(self.h, shares, threshold, n, _addr(keys), _addr(shared), _addr(v)))
         return shared, v
 
-    def dlog_table(self, lo, hi):
-        return DlogTable(self, lo, hi)
+    def dlog_table(self, lo, hi, baby_steps=None):
+        """DiscreteLogTable::new(lo..hi).  baby_steps=None: the range table of every value (hi - lo <= 2^28);
+        baby_steps=m: baby-step giant-step, a table of m values and up to ceil((hi - lo) / m) giant steps per lookup."""
+        return DlogTable(self, lo, hi, baby_steps)
+
+    def dlog_lookup(self, table, elements):
+        """DiscreteLogTable::get over 32-byte element encodings: (values, found), found 1 / 0 / 2 = present / absent /
+        does not decode (the identity is found with value 0)."""
+        elements = _u8(elements, (-1, 32))
+        n = elements.shape[0]
+        values, found = np.zeros(n, np.uint64), np.zeros(n, np.uint8)
+        self._check(self.lib.eg_dlog_lookup_batch(self.h, table.h, n, _addr(elements), _addr(values), _addr(found)))
+        return values, found
 
     def combine_decrypt(self, indexes, cts, shares, table):
         t = len(indexes)
@@ -584,12 +595,15 @@ class Engine:
 
 
 class DlogTable:
-    """DiscreteLogTable::new(lo..hi) resident on the engine's GPU."""
+    """DiscreteLogTable::new(lo..hi) resident on the engine's GPU (a range table, or baby-step giant-step)."""
 
-    def __init__(self, engine, lo, hi):
+    def __init__(self, engine, lo, hi, baby_steps=None):
         self.engine = engine
         h = C.c_void_p()
-        engine._check(engine.lib.eg_dlog_table_create(engine.h, lo, hi, C.byref(h)))
+        if baby_steps is None:
+            engine._check(engine.lib.eg_dlog_table_create(engine.h, lo, hi, C.byref(h)))
+        else:
+            engine._check(engine.lib.eg_dlog_table_create_bsgs(engine.h, lo, hi, baby_steps, C.byref(h)))
         self.h = h
 
     def close(self):

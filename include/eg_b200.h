@@ -296,6 +296,23 @@ eg_status eg_keysets_validate_batch(eg_ctx *ctx, uint32_t shares, uint32_t thres
 eg_status eg_dlog_table_create(eg_ctx *ctx, uint64_t lo, uint64_t hi, eg_dlog_table **out);
 void      eg_dlog_table_destroy(eg_dlog_table *table);
 
+/* DiscreteLogTable::new(lo..hi) (src/encryption.rs:267-284) for ranges too large to tabulate: baby-step giant-step.
+ * The device holds the range table of [lo, lo + baby_steps) (exactly what eg_dlog_table_create(lo, lo + baby_steps)
+ * builds: cap = the power of two >= 2 * baby_steps + 2 slots of 40 B, so baby_steps = 2^k - 1 fills it best).  A lookup
+ * that misses it walks up to J = ceil((hi - lo) / baby_steps) giant steps.  Every lookup returns exactly what
+ * eg_dlog_table_create(lo, hi) would return if it could be built.  When hi - lo <= baby_steps, the result is that range
+ * table and no walk ever runs.
+ * EG_ERR_INVALID_ARG unless hi >= lo, 256 <= baby_steps <= 2^28 and J <= 2^32.  The table is accepted wherever an
+ * eg_dlog_table is: eg_decrypt_batch, eg_combine_decrypt_batch(_dev), eg_dlog_lookup_batch, single- and multi-device
+ * contexts (one replica per device), eg_dlog_table_destroy.  A lookup's time depends on the value it finds. */
+eg_status eg_dlog_table_create_bsgs(eg_ctx *ctx, uint64_t lo, uint64_t hi, uint64_t baby_steps, eg_dlog_table **out);
+
+/* DiscreteLogTable::get (src/encryption.rs:287-297) over a batch of 32-byte element encodings, for either kind of table:
+ * found[i] = 1 and values[i] = v when elements[i] = [v]G with v in the table's range; found 1 / value 0 for the identity
+ * (whatever the range); found 0 / value 0 otherwise; found 2 / value 0 when the encoding does not decode. */
+eg_status eg_dlog_lookup_batch(eg_ctx *ctx, const eg_dlog_table *table, size_t n, const uint8_t *elements /* n*32 */,
+                               uint64_t *values /* n */, uint8_t *found /* n */);
+
 /* Params::combine_shares (src/sharing/mod.rs:302-325) on the first `threshold` shares of every tally, then
  * VerifiableDecryption::decrypt (src/decryption.rs:138-144) through DiscreteLogTable::get (src/encryption.rs:287-297).
  * found[i] = 1 and values[i] set when the decrypted element is in the table (identity -> 0), found[i] = 0 when it

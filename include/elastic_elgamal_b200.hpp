@@ -266,6 +266,27 @@ class Engine {
         return t;
     }
 
+    // DiscreteLogTable::new(lo..hi) by baby-step giant-step (baby_steps values on the device, up to 2^32 giant steps per
+    // lookup); owned by the engine
+    eg_dlog_table *dlog_table_bsgs(uint64_t lo, uint64_t hi, uint64_t baby_steps) {
+        eg_dlog_table *t = nullptr;
+        check(eg_dlog_table_create_bsgs(ctx_, lo, hi, baby_steps, &t));
+        tables_.push_back(t);
+        return t;
+    }
+
+    // DiscreteLogTable::get over a batch of elements (encryption.rs:287-297); the identity is found with value 0
+    std::vector<DecryptedValue> dlog_lookup_batch(const eg_dlog_table *table, const std::vector<Element> &elements) {
+        const size_t n = elements.size();
+        std::vector<uint8_t> el, found(n);
+        std::vector<uint64_t> values(n);
+        for (const auto &e : elements) el.insert(el.end(), e.begin(), e.end());
+        check(eg_dlog_lookup_batch(ctx_, table, n, el.data(), values.data(), found.data()));
+        std::vector<DecryptedValue> out(n);
+        for (size_t i = 0; i < n; i++) out[i] = DecryptedValue{found[i] == 1, values[i]};
+        return out;
+    }
+
     // params.combine_shares(..) + decrypt(ct, &table) per tally (sharing/mod.rs:302-325, decryption.rs:138-144)
     std::vector<DecryptedValue> combine_decrypt_batch(const std::vector<uint32_t> &indexes, const std::vector<Ciphertext> &cts,
                                                       const std::vector<Element> &shares, const eg_dlog_table *table) {

@@ -120,6 +120,9 @@ extern "C" {
                                      shared_keys: *mut u8, verdicts: *mut u8) -> eg_status;
     pub fn eg_dlog_table_create(ctx: *mut eg_ctx, lo: u64, hi: u64, out: *mut *mut eg_dlog_table) -> eg_status;
     pub fn eg_dlog_table_destroy(table: *mut eg_dlog_table);
+    pub fn eg_dlog_table_create_bsgs(ctx: *mut eg_ctx, lo: u64, hi: u64, baby_steps: u64, out: *mut *mut eg_dlog_table) -> eg_status;
+    pub fn eg_dlog_lookup_batch(ctx: *mut eg_ctx, table: *const eg_dlog_table, n: usize, elements: *const u8, values: *mut u64,
+                                found: *mut u8) -> eg_status;
     pub fn eg_combine_decrypt_batch(ctx: *mut eg_ctx, threshold: u32, indexes: *const u32, n_tallies: usize,
                                     share_stride: u32, cts: *const u8, shares: *const u8, table: *const eg_dlog_table,
                                     values: *mut u64, found: *mut u8) -> eg_status;

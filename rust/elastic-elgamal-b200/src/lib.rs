@@ -92,6 +92,23 @@ pub struct DlogTable<'e> {
     table: *mut sys::eg_dlog_table,
 }
 
+impl DlogTable<'_> {
+    /// `DiscreteLogTable::get` (encryption.rs:287-297) over a batch of elements: `Some(value)` when the element is `[value]G`
+    /// with `value` in the table's range (the identity is `Some(0)`), else `None`.
+    pub fn get_batch(&self, elements: &[<Ristretto as elastic_elgamal::group::ElementOps>::Element]) -> Result<Vec<Option<u64>>, EngineError> {
+        let n = elements.len();
+        let mut bytes = vec![0_u8; 32 * n];
+        for (el, chunk) in elements.iter().zip(bytes.chunks_mut(32)) {
+            Ristretto::serialize_element(el, chunk);
+        }
+        let (mut values, mut found) = (vec![0_u64; n], vec![0_u8; n]);
+        self.engine.check(unsafe {
+            sys::eg_dlog_lookup_batch(self.engine.ctx, self.table, n, bytes.as_ptr(), values.as_mut_ptr(), found.as_mut_ptr())
+        })?;
+        Ok(values.iter().zip(found).map(|(&v, f)| (f == 1).then_some(v)).collect())
+    }
+}
+
 impl Drop for DlogTable<'_> {
     fn drop(&mut self) {
         let _ = self.engine;
@@ -587,6 +604,14 @@ impl Engine {
     pub fn dlog_table(&self, lo: u64, hi: u64) -> Result<DlogTable<'_>, EngineError> {
         let mut table = ptr::null_mut();
         self.check(unsafe { sys::eg_dlog_table_create(self.ctx, lo, hi, &mut table) })?;
+        Ok(DlogTable { engine: self, table })
+    }
+
+    /// `DiscreteLogTable::new(lo..hi)` for ranges too large to tabulate: a table of `baby_steps` values and up to
+    /// `ceil((hi - lo) / baby_steps)` (<= 2^32) giant steps per lookup; the same answers as a table of every value.
+    pub fn dlog_table_bsgs(&self, lo: u64, hi: u64, baby_steps: u64) -> Result<DlogTable<'_>, EngineError> {
+        let mut table = ptr::null_mut();
+        self.check(unsafe { sys::eg_dlog_table_create_bsgs(self.ctx, lo, hi, baby_steps, &mut table) })?;
         Ok(DlogTable { engine: self, table })
     }
 
