@@ -6,6 +6,29 @@
 // the kernels below; there is no CPU path (eg_ctx_create fails without a device).
 #ifdef EG_HOSTSIM
 #include "hostsim_cuda.h"      // test-only stand-in for the CUDA runtime (tests/hostsim): malloc/memcpy, no device
+// Kernels in the test harness: launch() runs a __global__ function once per (block, thread), one after the other, with the
+// built-in indices set first.  The pretend device has one SM that holds one CTA of any kernel, so a persistent grid is a
+// single CTA.
+#define __global__
+#define __launch_bounds__(...)
+struct dim3 {
+    unsigned x, y, z;
+    dim3(unsigned x_ = 1, unsigned y_ = 1, unsigned z_ = 1) : x(x_), y(y_), z(z_) {}
+};
+static thread_local dim3 blockIdx, threadIdx, blockDim, gridDim;
+template <class K, class... A> static void hs_launch(K kernel, dim3 grid, dim3 block, const A &...args) {
+    gridDim = grid; blockDim = block;
+    for (unsigned b = 0; b < grid.x * grid.y * grid.z; b++) {
+        blockIdx = dim3(b % grid.x, b / grid.x % grid.y, b / (grid.x * grid.y));
+        for (unsigned t = 0; t < block.x * block.y * block.z; t++) {
+            threadIdx = dim3(t % block.x, t / block.x % block.y, t / (block.x * block.y));
+            kernel(args...);
+        }
+    }
+}
+enum cudaDeviceAttr { cudaDevAttrMultiProcessorCount = 16 };
+static cudaError_t cudaDeviceGetAttribute(int *v, cudaDeviceAttr, int) { *v = 1; return cudaSuccess; }
+template <class K> static cudaError_t cudaOccupancyMaxActiveBlocksPerMultiprocessor(int *n, K, int, size_t) { *n = 1; return cudaSuccess; }
 #else
 #include <cuda_runtime.h>
 #endif
@@ -43,13 +66,12 @@ struct eg_ctx {
     uint8_t blinding_base[32];
     uint32_t *d_table_g = nullptr, *d_table_k = nullptr, *d_table_h = nullptr, *d_status = nullptr;
     std::string err;
-    uint64_t launches = 0, commit_launches = 0, commit_tasks = 0;
+    uint64_t launches = 0;
     float timings[5] = {0, 0, 0, 0, 0};
     cudaEvent_t ev[8];
     std::vector<cudaEvent_t> commit_ev;     // pairs (start, stop) around every k_commit / k_ring launch of the current call
     std::vector<uint8_t> commit_ev_kind;    // per pair: 0 = k_commit, 1 = k_ring, 2 = k_msm, 3 = k_ring_pair
     size_t commit_ev_used = 0;
-    uint64_t call_commit_tasks = 0, call_commit_launches = 0;
     uint64_t kind_tasks[EG_STAT_KINDS] = {0, 0, 0, 0}, kind_launches[EG_STAT_KINDS] = {0, 0, 0, 0};   // per kind, current call
     float kind_ms[EG_STAT_KINDS] = {0, 0, 0, 0};
     // grow-only scratch
@@ -66,12 +88,7 @@ struct eg_ctx {
     int ring_mode = 0;        // 2: k_ring (one thread per ring, chunked tables); 1: k_commit / k_ring_hash launches per equation;
                               // 0: chosen per chunk (1 when the chunk cannot fill the persistent k_ring grid, run_ring_job)
     int prover_ct = 0;        // eg_ctx_set_prover_mode: constant-time fixed-base arithmetic for the provers' secret scalars
-    int ring_grid[2] = {0, 0};   // resident CTAs of the two k_ring shapes (queried once)
-    int prove_grid[3] = {0, 0, 0};
-    int rprove_grid[3] = {0, 0, 0};
-    int sumsq_prove_grid = 0, encrypt_grid = 0;
-    int decrypt_grid[4] = {0, 0, 0, 0};     // k_decrypt<op, ct>: index 2 op + ct
-    int ceq_prove_grid = 0, pop_prove_grid[2] = {0, 0};
+    std::map<const void *, int> resident;   // resident CTAs of each persistent-grid kernel (resident_ctas)
     dev_buf ring_scratch;
     // per-call narrow fixed-base tables of the participant keys of a key set (api_sharing.inc), cached by key bytes
     dev_buf xtab;
@@ -134,12 +151,11 @@ static eg_status ensure(eg_ctx *ctx, dev_buf &b, size_t bytes) {
 
 static inline unsigned grid_for(size_t threads, unsigned block) { return (unsigned)((threads + block - 1) / block); }
 
-// Per-call statistics of the equation-evaluation kernels: one CUDA event pair around every launch of kind `kind`
-// (EG_STAT_KINDS), `tasks` = what the launch evaluates (equation sides for k_commit / k_ring, multi-scalar sums for k_msm).
+// Per-call statistics of the equation-evaluation kernels (eg_last_kernel_stats): stat_begin / stat_end put one CUDA event
+// pair around a launch of kind `kind` (EG_STAT_KINDS) and count it, `tasks` = what the launch evaluates (equation sides for
+// k_commit / k_ring / k_ring_pair, multi-scalar sums for k_msm).
 static void reset_call_stats(eg_ctx *ctx) {
     ctx->commit_ev_used = 0;
-    ctx->call_commit_tasks = 0;
-    ctx->call_commit_launches = 0;
     for (int q = 0; q < EG_STAT_KINDS; q++) { ctx->kind_tasks[q] = 0; ctx->kind_launches[q] = 0; ctx->kind_ms[q] = 0; }
     for (float &t : ctx->timings) t = 0;
 }
@@ -156,96 +172,93 @@ static eg_status drain_on_error(eg_ctx *ctx, eg_status st) {
     return st;
 }
 
-static cudaEvent_t stat_begin(eg_ctx *ctx, int kind, size_t tasks) {
+static void stat_begin(eg_ctx *ctx, int kind, size_t tasks) {
     if (ctx->commit_ev_used + 2 > ctx->commit_ev.size()) {
         cudaEvent_t a = nullptr, b = nullptr;
         cudaEventCreate(&a); cudaEventCreate(&b);
         ctx->commit_ev.push_back(a); ctx->commit_ev.push_back(b);
     }
-    cudaEvent_t e_start = ctx->commit_ev[ctx->commit_ev_used], e_stop = ctx->commit_ev[ctx->commit_ev_used + 1];
     if (ctx->commit_ev_kind.size() < ctx->commit_ev.size() / 2) ctx->commit_ev_kind.resize(ctx->commit_ev.size() / 2);
     ctx->commit_ev_kind[ctx->commit_ev_used / 2] = (uint8_t)kind;
     ctx->kind_tasks[kind] += tasks; ctx->kind_launches[kind]++;
+    cudaEventRecord(ctx->commit_ev[ctx->commit_ev_used], ctx->stream);
     ctx->commit_ev_used += 2;
-    cudaEventRecord(e_start, ctx->stream);
-    return e_stop;
 }
 
-// ------------------------------------------------------------------- launchers (the only kernel start sites)
+static void stat_end(eg_ctx *ctx) { cudaEventRecord(ctx->commit_ev[ctx->commit_ev_used - 1], ctx->stream); }
 
-#ifdef EG_HOSTSIM
-#define EG_FOR_HOST(total, stmt) for (size_t tid = 0; tid < (size_t)(total); tid++) { stmt; }
-#endif
+// ------------------------------------------------------------------- kernel launches
 
-static void launch_decode(eg_ctx *ctx, const decode_params &P) {
-    size_t total = P.n * (size_t)P.n_slots;
+// The only kernel start site.  The test harness (EG_HOSTSIM) runs the same __global__ function on the CPU once per
+// (block, thread), so that its tests cover the index mapping the GPU runs.
+template <class... KP, class... A>
+static void launch(eg_ctx *ctx, void (*kernel)(KP...), dim3 grid, unsigned block, const A &...args) {
 #ifdef EG_HOSTSIM
-    EG_FOR_HOST(total, decode_body(P, tid % P.n, (int)(tid / P.n)))
+    hs_launch(kernel, grid, dim3(block), args...);
 #else
-    k_decode<<<grid_for(total, 256), 256, 0, ctx->stream>>>(P);
+    kernel<<<grid, block, 0, ctx->stream>>>(args...);
 #endif
     ctx->launches++;
 }
 
-static void launch_scalars(eg_ctx *ctx, const scalars_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, scalars_body(P, tid))
-#else
-    k_scalars<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
+// one thread per task: ceil(total / block) CTAs of `block` threads
+template <class... KP, class... A>
+static void launch_flat(eg_ctx *ctx, void (*kernel)(KP...), size_t total, unsigned block, const A &...args) {
+    launch(ctx, kernel, grid_for(total, block), block, args...);
 }
 
-static void launch_commit(eg_ctx *ctx, const commit_params &P) {
-    size_t total = P.n * (size_t)P.n_slots;
-    cudaEvent_t e_stop = stat_begin(ctx, 0, total);
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(total, commit_body(P, tid % P.n, (int)(tid / P.n), P.table_g, P.table_k))
-#else
-    k_commit<<<grid_for(total, EG_COMMIT_THREADS), EG_COMMIT_THREADS, 0, ctx->stream>>>(P);
-#endif
-    cudaEventRecord(e_stop, ctx->stream);
-    ctx->launches++;
-    ctx->commit_launches++;
-    ctx->commit_tasks += total;
-    ctx->call_commit_tasks += total;
-    ctx->call_commit_launches++;
-}
-
-static void launch_terminal(eg_ctx *ctx, const terminal_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, terminal_body(P, tid))
-#else
-    k_terminal<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
-
-// One launch evaluates every equation of every ring of the chunk.  Accounted like k_commit: tasks = equation sides.
-#ifndef EG_HOSTSIM
-// resident CTAs of the persistent k_ring grid (shape 1: rings of <= 2 equations, shape 0: longer rings), cached per context
-static eg_status ring_grid_size(eg_ctx *ctx, int shape) {
-    if (ctx->ring_grid[shape] == 0) {
+// CTAs of `kernel` (at `threads` per CTA) that the device holds at once, queried once per context
+template <class K>
+static eg_status resident_ctas(eg_ctx *ctx, K kernel, unsigned threads, size_t &ctas) {
+    int &cached = ctx->resident[reinterpret_cast<const void *>(kernel)];
+    if (cached == 0) {
         int per_sm = 0, sms = 0;
-        if (shape) CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ring<EG_RING2_THREADS, EG_RING2_MINBLOCKS, EG_VCHUNKS_SHORT>, EG_RING2_THREADS, 0));
-        else CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_ring<EG_RING_THREADS, EG_RING_MINBLOCKS, EG_VCHUNKS_LONG>, EG_RING_THREADS, 0));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, (int)threads, 0));
         CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_ring does not fit on an SM");
-        ctx->ring_grid[shape] = per_sm * sms;
+        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "a persistent kernel does not fit on an SM");
+        cached = per_sm * sms;
     }
+    ctas = (size_t)cached;
     return EG_SUCCESS;
 }
-#endif
+
+// Persistent grid: at most one wave of resident CTAs, whose threads stride over the `total` tasks.
+template <class... KP, class... A>
+static eg_status launch_persistent(eg_ctx *ctx, void (*kernel)(KP...), unsigned threads, size_t total, const A &...args) {
+    size_t ctas = 0;
+    TRY(resident_ctas(ctx, kernel, threads, ctas));
+    launch(ctx, kernel, (unsigned)std::min<size_t>(ctas, (total + threads - 1) / threads), threads, args...);
+    return EG_SUCCESS;
+}
+
+// k_ring's two shapes (device_kernels.inc): rings of <= 2 equations run one CTA of 512 threads per SM with 4-chunk
+// tables, longer rings 2 CTAs of 256 threads
+struct ring_shape {
+    void (*kernel)(ring_params);
+    unsigned threads;
+};
+static ring_shape ring_shape_for(bool short_rings) {
+    if (short_rings) return {k_ring<EG_RING2_THREADS, EG_RING2_MINBLOCKS, EG_VCHUNKS_SHORT>, EG_RING2_THREADS};
+    return {k_ring<EG_RING_THREADS, EG_RING_MINBLOCKS, EG_VCHUNKS_LONG>, EG_RING_THREADS};
+}
+
+// resident threads of the persistent k_ring grid of one shape
+static eg_status ring_resident_threads(eg_ctx *ctx, bool short_rings, size_t &threads) {
+    const ring_shape s = ring_shape_for(short_rings);
+    size_t ctas = 0;
+    TRY(resident_ctas(ctx, s.kernel, s.threads, ctas));
+    threads = ctas * s.threads;
+    return EG_SUCCESS;
+}
 
 // Chunk size rounded down to a whole number of waves of the persistent k_ring grid: a chunk of `chunk` items starts
 // chunk x rings_per_item ring threads, and a last partial wave costs as much as a full one (47 662 range proofs x 8 rings
 // are 5.03 waves of 75 776 threads).  Explicit chunk sizes (eg_ctx_set_chunk_items) are left alone.
 static size_t wave_chunk(eg_ctx *ctx, size_t chunk, size_t rings_per_item, bool short_rings) {
 #if !defined(EG_HOSTSIM) && !defined(EG_NO_WAVE_CHUNK)
+    size_t resident = 0;
     if (ctx->chunk_items || rings_per_item == 0) return chunk;
-    const int shape = short_rings ? 1 : 0;
-    if (ring_grid_size(ctx, shape) != EG_SUCCESS) return chunk;
-    const size_t resident = (size_t)ctx->ring_grid[shape] * (shape ? EG_RING2_THREADS : EG_RING_THREADS);
+    if (ring_resident_threads(ctx, short_rings, resident) != EG_SUCCESS) return chunk;
     const size_t waves = chunk * rings_per_item / resident;
     if (waves >= 2) chunk = waves * resident / rings_per_item;
 #else
@@ -297,38 +310,39 @@ static eg_status pipeline_chunks(eg_ctx *ctx, size_t n_chunks, In stage_in, Run 
     return drain_on_error(ctx, pipeline_chunks_impl(ctx, n_chunks, stage_in, compute, stage_out));
 }
 
-static eg_status launch_ring(eg_ctx *ctx, ring_params &P) {
+static void launch_decode(eg_ctx *ctx, const decode_params &P) { launch_flat(ctx, k_decode, P.n * (size_t)P.n_slots, 256, P); }
+
+static void launch_scalars(eg_ctx *ctx, const scalars_params &P) { launch_flat(ctx, k_scalars, P.n, 256, P); }
+
+static void launch_commit(eg_ctx *ctx, const commit_params &P) {
+    const size_t total = P.n * (size_t)P.n_slots;
+    stat_begin(ctx, 0, total);
+    launch_flat(ctx, k_commit, total, EG_COMMIT_THREADS, P);
+    stat_end(ctx);
+}
+
+static void launch_terminal(eg_ctx *ctx, const terminal_params &P) { launch_flat(ctx, k_terminal, P.n, 128, P); }
+
+// equation sides of a ring job (tasks of k_ring / k_ring_pair), and whether all its rings have <= 2 equations
+static size_t ring_sides(const ring_params &P, bool &short_rings) {
     size_t sides = 0;
-    for (uint32_t r = 0; r < P.n_rings; r++) sides += 2 * (size_t)P.sizes[r];
-    sides *= P.n;
-    const size_t total = P.n * (size_t)P.n_rings;
-    bool short_rings = true;                // rings of <= 2 equations: 4-chunk tables, one CTA of 512 threads per SM
-    for (uint32_t r = 0; r < P.n_rings; r++) short_rings = short_rings && P.sizes[r] <= 2;
-#ifdef EG_HOSTSIM
-    TRY(ensure(ctx, ctx->ring_scratch, 2 * EG_VTAB_WORDS * 4));
+    short_rings = true;
+    for (uint32_t r = 0; r < P.n_rings; r++) { sides += 2 * (size_t)P.sizes[r]; short_rings = short_rings && P.sizes[r] <= 2; }
+    return sides * P.n;
+}
+
+// One launch evaluates every equation of every ring of the chunk.  Accounted like k_commit: tasks = equation sides.
+static eg_status launch_ring(eg_ctx *ctx, ring_params &P) {
+    bool short_rings = true;
+    const size_t sides = ring_sides(P, short_rings);
+    const ring_shape s = ring_shape_for(short_rings);
+    size_t resident = 0;
+    TRY(ring_resident_threads(ctx, short_rings, resident));
+    TRY(ensure(ctx, ctx->ring_scratch, resident * 2 * EG_VTAB_WORDS * 4));
     P.scratch = (uint32_t *)ctx->ring_scratch.p;
-    cudaEvent_t e_stop = stat_begin(ctx, 1, sides);
-    if (short_rings) { EG_FOR_HOST(total, ring_body<EG_VCHUNKS_SHORT>(P, tid % P.n, (uint32_t)(tid / P.n), P.scratch, P.table_g, P.table_k)) }
-    else { EG_FOR_HOST(total, ring_body<EG_VCHUNKS_LONG>(P, tid % P.n, (uint32_t)(tid / P.n), P.scratch, P.table_g, P.table_k)) }
-#else
-    const size_t smem = 0;
-    const int shape = short_rings ? 1 : 0;
-    const int threads = shape ? EG_RING2_THREADS : EG_RING_THREADS;
-    TRY(ring_grid_size(ctx, shape));
-    const size_t resident = (size_t)ctx->ring_grid[shape];
-    const unsigned grid = (unsigned)std::min<size_t>(resident, (total + threads - 1) / threads);
-    TRY(ensure(ctx, ctx->ring_scratch, resident * threads * 2 * EG_VTAB_WORDS * 4));
-    P.scratch = (uint32_t *)ctx->ring_scratch.p;
-    cudaEvent_t e_stop = stat_begin(ctx, 1, sides);
-    if (shape) k_ring<EG_RING2_THREADS, EG_RING2_MINBLOCKS, EG_VCHUNKS_SHORT><<<grid, threads, smem, ctx->stream>>>(P);
-    else k_ring<EG_RING_THREADS, EG_RING_MINBLOCKS, EG_VCHUNKS_LONG><<<grid, threads, smem, ctx->stream>>>(P);
-#endif
-    cudaEventRecord(e_stop, ctx->stream);
-    ctx->launches++;
-    ctx->commit_launches++;
-    ctx->commit_tasks += sides;
-    ctx->call_commit_tasks += sides;
-    ctx->call_commit_launches++;
+    stat_begin(ctx, 1, sides);
+    TRY(launch_persistent(ctx, s.kernel, s.threads, P.n * (size_t)P.n_rings, P));
+    stat_end(ctx);
     return EG_SUCCESS;
 }
 
@@ -336,286 +350,81 @@ static eg_status launch_ring(eg_ctx *ctx, ring_params &P) {
 // equation sides (X.n_slots > 0: the sum proof of an EncryptedChoice) ride along as further lanes of the same launch, so the
 // longest chain of the launch stays the ring's.  Accounted like k_ring (tasks = equation sides), under its own kind (3).
 static eg_status launch_ring_pair(eg_ctx *ctx, ring_params &P, const commit_params &X) {
-    size_t sides = 0;
-    for (uint32_t r = 0; r < P.n_rings; r++) sides += 2 * (size_t)P.sizes[r];
-    sides *= P.n;
-    const size_t total = P.n * (size_t)P.n_rings, extra = P.n * (size_t)X.n_slots;
     bool short_rings = true;
-    for (uint32_t r = 0; r < P.n_rings; r++) short_rings = short_rings && P.sizes[r] <= 2;
-#ifdef EG_HOSTSIM
-    TRY(ensure(ctx, ctx->ring_scratch, 2 * EG_VTAB_WORDS * 4));
+    const size_t sides = ring_sides(P, short_rings), lanes = 2 * P.n * (size_t)P.n_rings, extra = P.n * (size_t)X.n_slots;
+    TRY(ensure(ctx, ctx->ring_scratch, lanes * EG_VTAB_WORDS * 4));
     P.scratch = (uint32_t *)ctx->ring_scratch.p;
-    cudaEvent_t e_stop = stat_begin(ctx, 3, sides + extra);
-    if (short_rings) { EG_FOR_HOST(total, ring_pair_host<EG_VCHUNKS_SHORT>(P, tid % P.n, (uint32_t)(tid / P.n), P.scratch, P.table_g, P.table_k)) }
-    else { EG_FOR_HOST(total, ring_pair_host<EG_VCHUNKS_LONG>(P, tid % P.n, (uint32_t)(tid / P.n), P.scratch, P.table_g, P.table_k)) }
-    EG_FOR_HOST(extra, commit_body(X, tid % X.n, (int)(tid / X.n), X.table_g, X.table_k))
-#else
-    TRY(ensure(ctx, ctx->ring_scratch, 2 * total * EG_VTAB_WORDS * 4));
-    P.scratch = (uint32_t *)ctx->ring_scratch.p;
-    cudaEvent_t e_stop = stat_begin(ctx, 3, sides + extra);
-    const unsigned grid = grid_for(2 * total + extra, EG_PAIR_THREADS);
-    if (short_rings) k_ring_pair<EG_VCHUNKS_SHORT><<<grid, EG_PAIR_THREADS, 0, ctx->stream>>>(P, X);
-    else k_ring_pair<EG_VCHUNKS_LONG><<<grid, EG_PAIR_THREADS, 0, ctx->stream>>>(P, X);
-#endif
-    cudaEventRecord(e_stop, ctx->stream);
-    ctx->launches++;
-    ctx->commit_launches++;
-    ctx->commit_tasks += sides + extra;
-    ctx->call_commit_tasks += sides + extra;
-    ctx->call_commit_launches++;
+    stat_begin(ctx, 3, sides + extra);
+    launch_flat(ctx, short_rings ? k_ring_pair<EG_VCHUNKS_SHORT> : k_ring_pair<EG_VCHUNKS_LONG>, lanes + extra, EG_PAIR_THREADS, P, X);
+    stat_end(ctx);
     return EG_SUCCESS;
 }
 
-#ifndef EG_HOSTSIM
-template <int PHASE>
-static eg_status launch_prove_phase(eg_ctx *ctx, const prove_params &P, int &grid_cache) {
-    const size_t smem = 0;
-    if (grid_cache == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_prove<PHASE>, EG_RING_THREADS, smem));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_prove does not fit on an SM");
-        grid_cache = per_sm * sms;
-    }
-    const size_t total = PHASE == 1 ? P.n : P.n * (size_t)P.options;
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)grid_cache, (total + EG_RING_THREADS - 1) / EG_RING_THREADS);
-    TRY(ensure(ctx, ctx->ring_scratch, (size_t)grid_cache * EG_RING_THREADS * 2 * EG_VTAB_WORDS * 4));
-    k_prove<PHASE><<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P, (uint32_t *)ctx->ring_scratch.p);
-    ctx->launches++;
-    return EG_SUCCESS;
+// one phase of a prover (k_prove, k_rprove): persistent grid, 2 EG_VTAB_WORDS words of window-table scratch per thread
+template <class Params>
+static eg_status launch_prover_phase(eg_ctx *ctx, void (*kernel)(Params, uint32_t *), const Params &P, size_t total) {
+    size_t ctas = 0;
+    TRY(resident_ctas(ctx, kernel, EG_RING_THREADS, ctas));
+    TRY(ensure(ctx, ctx->ring_scratch, ctas * EG_RING_THREADS * 2 * EG_VTAB_WORDS * 4));
+    return launch_persistent(ctx, kernel, EG_RING_THREADS, total, P, (uint32_t *)ctx->ring_scratch.p);
 }
-#endif
 
 static eg_status launch_prove(eg_ctx *ctx, const prove_params &P) {
-#ifdef EG_HOSTSIM
-    TRY(ensure(ctx, ctx->ring_scratch, 2 * EG_VTAB_WORDS * 4));
-    uint32_t *scratch = (uint32_t *)ctx->ring_scratch.p;
-    EG_FOR_HOST(P.n * (size_t)P.options, prove_ring1_body(P, tid % P.n, (uint32_t)(tid / P.n), scratch, P.table_g, P.table_k))
-    EG_FOR_HOST(P.n, prove_common_body(P, tid, P.table_g, P.table_k))
-    EG_FOR_HOST(P.n * (size_t)P.options, prove_ring2_body(P, tid % P.n, (uint32_t)(tid / P.n), scratch, P.table_g, P.table_k))
-    ctx->launches += 3;
-#else
-    TRY(launch_prove_phase<0>(ctx, P, ctx->prove_grid[0]));
-    TRY(launch_prove_phase<1>(ctx, P, ctx->prove_grid[1]));
-    TRY(launch_prove_phase<2>(ctx, P, ctx->prove_grid[2]));
-#endif
-    return EG_SUCCESS;
+    TRY(launch_prover_phase(ctx, k_prove<0>, P, P.n * (size_t)P.options));
+    TRY(launch_prover_phase(ctx, k_prove<1>, P, P.n));
+    return launch_prover_phase(ctx, k_prove<2>, P, P.n * (size_t)P.options);
 }
-
-#ifndef EG_HOSTSIM
-template <int PHASE>
-static eg_status launch_rprove_phase(eg_ctx *ctx, const rprove_params &P, int &grid_cache) {
-    const size_t smem = 0;
-    if (grid_cache == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_rprove<PHASE>, EG_RING_THREADS, smem));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_rprove does not fit on an SM");
-        grid_cache = per_sm * sms;
-    }
-    const size_t total = P.n * (size_t)(PHASE == 0 ? P.n_rings + 1 : (PHASE == 1 ? 1 : P.n_rings));
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)grid_cache, (total + EG_RING_THREADS - 1) / EG_RING_THREADS);
-    TRY(ensure(ctx, ctx->ring_scratch, (size_t)grid_cache * EG_RING_THREADS * 2 * EG_VTAB_WORDS * 4));
-    k_rprove<PHASE><<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P, (uint32_t *)ctx->ring_scratch.p);
-    ctx->launches++;
-    return EG_SUCCESS;
-}
-#endif
 
 static eg_status launch_rprove(eg_ctx *ctx, const rprove_params &P) {
-#ifdef EG_HOSTSIM
-    TRY(ensure(ctx, ctx->ring_scratch, 2 * EG_VTAB_WORDS * 4));
-    uint32_t *scratch = (uint32_t *)ctx->ring_scratch.p;
-    EG_FOR_HOST(P.n * (size_t)(P.n_rings + 1), rprove_ring1_body(P, tid % P.n, (uint32_t)(tid / P.n), scratch, P.table_g, P.table_k))
-    EG_FOR_HOST(P.n, rprove_common_body(P, tid))
-    EG_FOR_HOST(P.n * (size_t)P.n_rings, rprove_ring2_body(P, tid % P.n, (uint32_t)(tid / P.n), scratch, P.table_g, P.table_k))
-    ctx->launches += 3;
-#else
-    TRY(launch_rprove_phase<0>(ctx, P, ctx->rprove_grid[0]));
-    TRY(launch_rprove_phase<1>(ctx, P, ctx->rprove_grid[1]));
-    TRY(launch_rprove_phase<2>(ctx, P, ctx->rprove_grid[2]));
-#endif
-    return EG_SUCCESS;
+    TRY(launch_prover_phase(ctx, k_rprove<0>, P, P.n * (size_t)(P.n_rings + 1)));
+    TRY(launch_prover_phase(ctx, k_rprove<1>, P, P.n));
+    return launch_prover_phase(ctx, k_rprove<2>, P, P.n * (size_t)P.n_rings);
 }
 
-static eg_status launch_encrypt(eg_ctx *ctx, const encrypt_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, encrypt_body(P, tid, P.table_g, P.table_k))
-#else
-    const size_t smem = 0;
-    if (ctx->encrypt_grid == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_encrypt, EG_RING_THREADS, smem));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_encrypt does not fit on an SM");
-        ctx->encrypt_grid = per_sm * sms;
-    }
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)ctx->encrypt_grid, (P.n + EG_RING_THREADS - 1) / EG_RING_THREADS);
-    k_encrypt<<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-    return EG_SUCCESS;
-}
-
-#ifndef EG_HOSTSIM
-template <int OP, bool CT>
-static eg_status launch_decrypt_t(eg_ctx *ctx, const decrypt_params &P) {
-    int &grid_cache = ctx->decrypt_grid[2 * OP + (CT ? 1 : 0)];
-    if (grid_cache == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_decrypt<OP, CT>, EG_DECRYPT_THREADS, 0));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_decrypt does not fit on an SM");
-        grid_cache = per_sm * sms;
-    }
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)grid_cache, (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS);
-    k_decrypt<OP, CT><<<grid, EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
-    return EG_SUCCESS;
-}
-#endif
+static eg_status launch_encrypt(eg_ctx *ctx, const encrypt_params &P) { return launch_persistent(ctx, k_encrypt, EG_RING_THREADS, P.n, P); }
 
 static eg_status launch_decrypt(eg_ctx *ctx, int op, const decrypt_params &P) {
     const bool ct = P.rnd.ct != 0;
-#ifdef EG_HOSTSIM
-    if (op == EG_DEC_PLAIN) {
-        if (ct) { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PLAIN, true>(P, tid))) } else { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PLAIN, false>(P, tid))) }
-    } else {
-        if (ct) { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PROOF, true>(P, tid))) } else { EG_FOR_HOST(P.n, (decrypt_body<EG_DEC_PROOF, false>(P, tid))) }
-    }
-#else
-    if (op == EG_DEC_PLAIN) TRY((ct ? launch_decrypt_t<EG_DEC_PLAIN, true>(ctx, P) : launch_decrypt_t<EG_DEC_PLAIN, false>(ctx, P)));
-    else TRY((ct ? launch_decrypt_t<EG_DEC_PROOF, true>(ctx, P) : launch_decrypt_t<EG_DEC_PROOF, false>(ctx, P)));
-#endif
-    ctx->launches++;
-    return EG_SUCCESS;
+    void (*kernel)(decrypt_params) = op == EG_DEC_PLAIN ? (ct ? k_decrypt<EG_DEC_PLAIN, true> : k_decrypt<EG_DEC_PLAIN, false>)
+                                                        : (ct ? k_decrypt<EG_DEC_PROOF, true> : k_decrypt<EG_DEC_PROOF, false>);
+    return launch_persistent(ctx, kernel, EG_DECRYPT_THREADS, P.n, P);
 }
 
 static eg_status launch_sumsq_prove(eg_ctx *ctx, const sumsq_prove_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, sumsq_prove_body(P, tid, P.table_g, P.table_k))
-#else
-    const size_t smem = 0;
-    if (ctx->sumsq_prove_grid == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sumsq_prove, EG_RING_THREADS, smem));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, "k_sumsq_prove does not fit on an SM");
-        ctx->sumsq_prove_grid = per_sm * sms;
-    }
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)ctx->sumsq_prove_grid, (P.n + EG_RING_THREADS - 1) / EG_RING_THREADS);
-    k_sumsq_prove<<<grid, EG_RING_THREADS, smem, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-    return EG_SUCCESS;
+    return launch_persistent(ctx, k_sumsq_prove, EG_RING_THREADS, P.n, P);
 }
 
 static eg_status launch_sumsq_stage(eg_ctx *ctx, const sumsq_stage_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, sumsq_stage_body(P, tid))
-#else
-    k_sumsq_stage<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_sumsq_stage, P.n, 256, P);
     return EG_SUCCESS;
 }
-
-#ifndef EG_HOSTSIM
-// resident threads of a persistent grid of `kernel` (cached in `grid_cache`)
-template <class K>
-static eg_status persistent_grid(eg_ctx *ctx, K kernel, int threads, int &grid_cache, const char *name) {
-    if (grid_cache == 0) {
-        int per_sm = 0, sms = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0));
-        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-        if (per_sm < 1) return fail(ctx, EG_ERR_CUDA, (std::string(name) + " does not fit on an SM").c_str());
-        grid_cache = per_sm * sms;
-    }
-    return EG_SUCCESS;
-}
-#endif
 
 static eg_status launch_ceq_prove(eg_ctx *ctx, const ceq_prove_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, ceq_prove_body(P, tid))
-#else
-    TRY(persistent_grid(ctx, k_ceq_prove, EG_DECRYPT_THREADS, ctx->ceq_prove_grid, "k_ceq_prove"));
-    const unsigned grid = (unsigned)std::min<size_t>((size_t)ctx->ceq_prove_grid, (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS);
-    k_ceq_prove<<<grid, EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-    return EG_SUCCESS;
+    return launch_persistent(ctx, k_ceq_prove, EG_DECRYPT_THREADS, P.n, P);
 }
 
 static eg_status launch_pop_prove(eg_ctx *ctx, const pop_prove_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n * (size_t)P.k, pop_key_body(P, tid % P.n, (uint32_t)(tid / P.n)))
-    EG_FOR_HOST(P.n, pop_final_body(P, tid))
-#else
-    TRY(persistent_grid(ctx, k_pop_prove<0>, EG_DECRYPT_THREADS, ctx->pop_prove_grid[0], "k_pop_prove"));
-    TRY(persistent_grid(ctx, k_pop_prove<1>, EG_DECRYPT_THREADS, ctx->pop_prove_grid[1], "k_pop_prove"));
-    const size_t t0 = P.n * (size_t)P.k;
-    k_pop_prove<0><<<(unsigned)std::min<size_t>((size_t)ctx->pop_prove_grid[0], (t0 + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS),
-                     EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
-    k_pop_prove<1><<<(unsigned)std::min<size_t>((size_t)ctx->pop_prove_grid[1], (P.n + EG_DECRYPT_THREADS - 1) / EG_DECRYPT_THREADS),
-                     EG_DECRYPT_THREADS, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches += 2;
-    return EG_SUCCESS;
+    TRY(launch_persistent(ctx, k_pop_prove<0>, EG_DECRYPT_THREADS, P.n * (size_t)P.k, P));
+    return launch_persistent(ctx, k_pop_prove<1>, EG_DECRYPT_THREADS, P.n, P);
 }
 
-static void launch_ring_hash(eg_ctx *ctx, const ring_hash_params &P) {
-    size_t total = P.n * (size_t)P.n_slots;
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(total, ring_hash_body(P, tid % P.n, (int)(tid / P.n)))
-#else
-    k_ring_hash<<<grid_for(total, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_ring_hash(eg_ctx *ctx, const ring_hash_params &P) { launch_flat(ctx, k_ring_hash, P.n * (size_t)P.n_slots, 128, P); }
 
-static void launch_ring_final(eg_ctx *ctx, const ring_final_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, ring_final_body(P, tid))
-#else
-    k_ring_final<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_ring_final(eg_ctx *ctx, const ring_final_params &P) { launch_flat(ctx, k_ring_final, P.n, 128, P); }
 
-static void launch_logeq_final(eg_ctx *ctx, const logeq_final_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, logeq_final_body(P, tid))
-#else
-    k_logeq_final<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_logeq_final(eg_ctx *ctx, const logeq_final_params &P) { launch_flat(ctx, k_logeq_final, P.n, 128, P); }
 
-static void launch_choice_sum(eg_ctx *ctx, const choice_sum_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(2 * P.n, choice_sum_body(P, tid % P.n, (int)(tid / P.n)))
-#else
-    k_choice_sum<<<grid_for(2 * P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_choice_sum(eg_ctx *ctx, const choice_sum_params &P) { launch_flat(ctx, k_choice_sum, 2 * P.n, 128, P); }
 
-static void launch_range_last(eg_ctx *ctx, const range_last_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(2 * P.n, range_last_body(P, tid % P.n, (int)(tid / P.n)))
-#else
-    k_range_last<<<grid_for(2 * P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_range_last(eg_ctx *ctx, const range_last_params &P) { launch_flat(ctx, k_range_last, 2 * P.n, 128, P); }
 
-static void launch_verdict(eg_ctx *ctx, const verdict_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, verdict_body(P, tid))
-#else
-    k_verdict<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
+static void launch_verdict(eg_ctx *ctx, const verdict_params &P) { launch_flat(ctx, k_verdict, P.n, 256, P); }
+
+static void launch_qv_verdict(eg_ctx *ctx, const qv_verdict_params &P) { launch_flat(ctx, k_qv_verdict, P.n, 256, P); }
+
+static void launch_share_verdict(eg_ctx *ctx, const share_verdict_params &P) {
+    const size_t total = P.n * (size_t)P.n_shares;
+    launch_flat(ctx, k_share_verdict, total, 256, P, total);
 }
 
 // wide fixed-base table of one base (ge.cuh): EG_WIDE_TABLE_WORDS words, followed by EG_WIDE_SCRATCH_WORDS of window bases
@@ -623,15 +432,8 @@ static void launch_verdict(eg_ctx *ctx, const verdict_params &P) {
 template <int BITS>
 static void launch_build_table_b(eg_ctx *ctx, const uint32_t *enc_words, int use_generator, uint32_t *table, uint32_t *status) {
     uint32_t *bases = table + EG_BITS_TABLE_WORDS(BITS);
-    const size_t fill = (size_t)EG_BITS_WINDOWS(BITS) * (EG_BITS_ENTRIES(BITS) / EG_WIDE_BLOCK);
-#ifdef EG_HOSTSIM
-    wide_bases_body<BITS>(enc_words, use_generator, bases, status);
-    EG_FOR_HOST(fill, wide_fill_body<BITS>(tid, bases, table))
-#else
-    k_wide_bases<BITS><<<1, 1, 0, ctx->stream>>>(enc_words, use_generator, bases, status);
-    k_wide_fill<BITS><<<grid_for(fill, 64), 64, 0, ctx->stream>>>(bases, table);
-#endif
-    ctx->launches += 2;
+    launch(ctx, k_wide_bases<BITS>, 1, 1, enc_words, use_generator, bases, status);
+    launch_flat(ctx, k_wide_fill<BITS>, (size_t)EG_BITS_WINDOWS(BITS) * (EG_BITS_ENTRIES(BITS) / EG_WIDE_BLOCK), 64, bases, table);
 }
 static void launch_build_table(eg_ctx *ctx, const uint32_t *enc_words, int use_generator, uint32_t *table, uint32_t *status) {
     launch_build_table_b<EG_WIDE_BITS>(ctx, enc_words, use_generator, table, status);
@@ -642,122 +444,47 @@ static void launch_build_narrow_table(eg_ctx *ctx, const uint32_t *enc_words, ui
 }
 
 static void launch_admissible(eg_ctx *ctx, const uint64_t *values, int count, uint32_t *adm) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(count, admissible_body((int)tid, values, adm))
-#else
-    k_admissible<<<grid_for(count, 64), 64, 0, ctx->stream>>>(values, count, adm);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_admissible, count, 64, values, count, adm);
 }
 
 // per-slot masked sums of planar points into `partial` (blocks per slot returned)
 static int launch_tally_partial(eg_ctx *ctx, const uint32_t *pts, size_t n, int n_slots, const uint8_t *verdicts, uint32_t *partial) {
     const int blocks = (int)std::max<size_t>(1, std::min<size_t>(EG_TALLY_BLOCKS, (n + EG_TALLY_THREADS - 1) / EG_TALLY_THREADS));
-#ifdef EG_HOSTSIM
-    for (int slot = 0; slot < n_slots; slot++)
-        for (int b = 0; b < blocks; b++) {
-            ge_ext acc = ge_identity(), q;
-            for (size_t i = (size_t)b; i < n; i += (size_t)blocks)
-                if (verdicts[i] == 0) { planar_load_point(q, pts, n, slot, i); ge_add(acc, acc, q); }
-            point_to_words32(partial + ((size_t)slot * blocks + b) * 32, acc);
-        }
-#else
-    dim3 grid(blocks, n_slots);
-    k_tally_partial<<<grid, EG_TALLY_THREADS, 0, ctx->stream>>>(pts, n, verdicts, partial);
-#endif
-    ctx->launches++;
+    launch(ctx, k_tally_partial, dim3(blocks, n_slots), EG_TALLY_THREADS, pts, n, verdicts, partial);
     return blocks;
 }
 
 static void launch_tally_final(eg_ctx *ctx, const uint32_t *partial, int count, int n_slots, uint32_t *running, int accumulate,
                                uint8_t *encode_out) {
-#ifdef EG_HOSTSIM
-    for (int slot = 0; slot < n_slots; slot++) {
-        ge_ext acc = ge_identity(), q;
-        for (int i = 0; i < count; i++) { point_from_words32(q, partial + ((size_t)slot * count + i) * 32); ge_add(acc, acc, q); }
-        uint32_t *r = running + (size_t)slot * 32;
-        if (accumulate) { point_from_words32(q, r); ge_add(acc, acc, q); }
-        point_to_words32(r, acc);
-        if (encode_out) { uint32_t w[8]; ge_encode(w, acc); store32_bytes(encode_out + 32 * slot, w); }
-    }
-#else
-    k_tally_final<<<n_slots, 32, 0, ctx->stream>>>(partial, count, running, accumulate, encode_out);
-#endif
-    ctx->launches++;
+    launch(ctx, k_tally_final, n_slots, 32, partial, count, running, accumulate, encode_out);
 }
 
 static void launch_elements_validate(eg_ctx *ctx, const uint8_t *enc, size_t n, uint8_t *ok) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(n, elements_validate_body(tid, enc, ok))
-#else
-    k_elements_validate<<<grid_for(n, 128), 128, 0, ctx->stream>>>(enc, n, ok);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_elements_validate, n, 128, enc, n, ok);
 }
 
 static void launch_scalars_validate(eg_ctx *ctx, const uint8_t *sc_in, size_t n, uint8_t *ok) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(n, scalars_validate_body(tid, sc_in, ok))
-#else
-    k_scalars_validate<<<grid_for(n, 256), 256, 0, ctx->stream>>>(sc_in, n, ok);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_scalars_validate, n, 256, sc_in, n, ok);
 }
 
-static void launch_keyset_verdict(eg_ctx *ctx, const keyset_verdict_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, keyset_verdict_body(P, tid))
-#else
-    k_keyset_verdict<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_keyset_verdict(eg_ctx *ctx, const keyset_verdict_params &P) { launch_flat(ctx, k_keyset_verdict, P.n, 256, P); }
 
-static void launch_unpack(eg_ctx *ctx, const unpack_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, unpack_body(P, tid))
-#else
-    k_unpack<<<grid_for(P.n, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_unpack(eg_ctx *ctx, const unpack_params &P) { launch_flat(ctx, k_unpack, P.n, 256, P); }
 
 static void launch_b64url(eg_ctx *ctx, const b64_params &P, bool encode) {
-    const size_t total = P.n * (size_t)P.groups;
-#ifdef EG_HOSTSIM
-    if (encode) { EG_FOR_HOST(total, b64url_encode_body(P, tid)) } else { EG_FOR_HOST(total, b64url_decode_body(P, tid)) }
-#else
-    if (encode) k_b64url<1><<<grid_for(total, 256), 256, 0, ctx->stream>>>(P);
-    else k_b64url<0><<<grid_for(total, 256), 256, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, encode ? k_b64url<1> : k_b64url<0>, P.n * (size_t)P.groups, 256, P);
 }
 
 static void launch_scalars_from_wide(eg_ctx *ctx, const uint8_t *wide, size_t n, uint8_t *out) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(n, scalars_from_wide_body(tid, wide, out))
-#else
-    k_scalars_from_wide<<<grid_for(n, 256), 256, 0, ctx->stream>>>(wide, n, out);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_scalars_from_wide, n, 256, wide, n, out);
 }
 
 static void launch_double_mul(eg_ctx *ctx, const uint8_t *a, const uint8_t *A, const uint8_t *b, size_t n, int mode, uint8_t *out, uint8_t *okv) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(n, double_mul_body(tid, a, A, b, mode, ctx->d_table_g, out, okv))
-#else
-    k_double_mul<<<grid_for(n, EG_COMMIT_THREADS), EG_COMMIT_THREADS, 0, ctx->stream>>>(a, A, b, n, mode, ctx->d_table_g, out, okv);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_double_mul, n, EG_COMMIT_THREADS, a, A, b, n, mode, ctx->d_table_g, out, okv);
 }
 
 static void launch_ciphertexts_sum(eg_ctx *ctx, const uint8_t *parts, size_t n_parts, size_t n_cts, uint8_t *out, uint32_t *bad) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(2 * n_cts, ciphertexts_sum_body(tid, parts, n_parts, n_cts, out, bad))
-#else
-    k_ciphertexts_sum<<<grid_for(2 * n_cts, 64), 64, 0, ctx->stream>>>(parts, n_parts, n_cts, out, bad);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_ciphertexts_sum, 2 * n_cts, 64, parts, n_parts, n_cts, out, bad);
 }
 
 // k_msm over the slot table uploaded last; slots whose encoding was deferred by upload_slots are encoded together by
@@ -769,15 +496,10 @@ static eg_status launch_msm(eg_ctx *ctx, const msm_params &P0) {
         TRY(ensure(ctx, ctx->term, P.n * (size_t)n_term * 128));
         P.term_pts = (uint32_t *)ctx->term.p;
     }
-    size_t total = P.n * (size_t)P.n_slots;
-    cudaEvent_t e_stop = stat_begin(ctx, 2, total);
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(total, msm_body(P, tid % P.n, (int)(tid / P.n), P.table_g, P.table_k, P.table_h))
-#else
-    k_msm<<<grid_for(total, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    cudaEventRecord(e_stop, ctx->stream);
-    ctx->launches++;
+    const size_t total = P.n * (size_t)P.n_slots;
+    stat_begin(ctx, 2, total);
+    launch_flat(ctx, k_msm, total, 128, P);
+    stat_end(ctx);
     if (n_term) {
         terminal_params tp = ctx->term_plan;
         tp.n = P.n; tp.term_pts = P.term_pts; tp.commit = P.commit;
@@ -786,62 +508,22 @@ static eg_status launch_msm(eg_ctx *ctx, const msm_params &P0) {
     return EG_SUCCESS;
 }
 
-static void launch_sigma_final(eg_ctx *ctx, const sigma_final_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, sigma_final_body(P, tid))
-#else
-    k_sigma_final<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_sigma_final(eg_ctx *ctx, const sigma_final_params &P) { launch_flat(ctx, k_sigma_final, P.n, 128, P); }
 
-static void launch_sumsq_final(eg_ctx *ctx, const sumsq_final_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, sumsq_final_body(P, tid))
-#else
-    k_sumsq_final<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_sumsq_final(eg_ctx *ctx, const sumsq_final_params &P) { launch_flat(ctx, k_sumsq_final, P.n, 128, P); }
 
 // `P` lives in host memory; the device copy `d_P` is what the kernel reads (the struct exceeds the 4 KB launch limit)
 static void launch_share_final(eg_ctx *ctx, const share_final_params &P, const share_final_params *d_P) {
-    size_t total = P.n * (size_t)P.n_shares;
-#ifdef EG_HOSTSIM
-    (void)d_P;
-    EG_FOR_HOST(total, share_final_body(P, tid % P.n, (int)(tid / P.n)))
-#else
-    k_share_final<<<grid_for(total, 128), 128, 0, ctx->stream>>>(d_P);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_share_final, P.n * (size_t)P.n_shares, 128, d_P);
 }
 
 static void launch_dlog_build(eg_ctx *ctx, const dlog_build_params &P, size_t threads) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(threads, dlog_build_body(P, tid))
-#else
-    k_dlog_build<<<grid_for(threads, 128), 128, 0, ctx->stream>>>(P, threads);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_dlog_build, threads, 128, P, threads);
 }
 
-static void launch_dlog_lookup(eg_ctx *ctx, const dlog_lookup_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, dlog_lookup_body(P, tid))
-#else
-    k_dlog_lookup<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_dlog_lookup(eg_ctx *ctx, const dlog_lookup_params &P) { launch_flat(ctx, k_dlog_lookup, P.n, 128, P); }
 
-static void launch_dlog_get(eg_ctx *ctx, const dlog_get_params &P) {
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(P.n, dlog_get_body(P, tid))
-#else
-    k_dlog_get<<<grid_for(P.n, 128), 128, 0, ctx->stream>>>(P);
-#endif
-    ctx->launches++;
-}
+static void launch_dlog_get(eg_ctx *ctx, const dlog_get_params &P) { launch_flat(ctx, k_dlog_get, P.n, 128, P); }
 
 // Giant-step walk of a BSGS table (giants > 1) over the items that the probe of giant step 0 left at found 0.  Each item gets
 // `segs` threads of seg_steps consecutive steps: enough threads in all to fill the GPU when the batch is small (one element
@@ -871,12 +553,7 @@ static void launch_dlog_walk(eg_ctx *ctx, const eg_dlog_table *t, size_t n, cons
     P.cap = t->cap; P.keys = t->d_keys; P.vals = (const unsigned long long *)t->d_vals; P.table_g = ctx->d_table_g;
     for (int w = 0; w < 24; w++) P.step[w] = t->step[w];
     const size_t total = n * (size_t)segs;
-#ifdef EG_HOSTSIM
-    EG_FOR_HOST(total, dlog_walk_body(P, tid))
-#else
-    k_dlog_walk<<<grid_for(total, EG_DECRYPT_THREADS), EG_DECRYPT_THREADS, 0, ctx->stream>>>(P, total);
-#endif
-    ctx->launches++;
+    launch_flat(ctx, k_dlog_walk, total, EG_DECRYPT_THREADS, P, total);
 }
 
 #include "comm.inc"
@@ -899,19 +576,20 @@ extern "C" uint64_t eg_kernel_launch_count(const eg_ctx *ctx) {
 
 extern "C" void *eg_ctx_stream(const eg_ctx *ctx) { return ctx ? (void *)ctx_first(const_cast<eg_ctx *>(ctx))->stream : nullptr; }
 
+// the ring-proof equation kernels: kinds 0 (k_commit), 1 (k_ring) and 3 (k_ring_pair) of eg_last_kernel_stats
 extern "C" eg_status eg_last_commit_stats(const eg_ctx *ctx, uint64_t *launches, uint64_t *tasks, float *ms) {
     if (!ctx) return EG_ERR_INVALID_ARG;
-    if (ctx_is_multi(ctx)) {            // launches / tasks summed over the devices, time = the slowest device
-        uint64_t l = 0, t = 0; float m = 0;
-        for (const eg_ctx *c : ctx->children) { l += c->call_commit_launches; t += c->call_commit_tasks; m = std::max(m, c->timings[2]); }
-        if (launches) *launches = l;
-        if (tasks) *tasks = t;
-        if (ms) *ms = m;
-        return EG_SUCCESS;
+    uint64_t l = 0, t = 0;
+    for (int kind : {0, 1, 3}) {
+        uint64_t kl = 0, kt = 0;
+        eg_last_kernel_stats(ctx, kind, &kl, &kt, nullptr);
+        l += kl; t += kt;
     }
-    if (launches) *launches = ctx->call_commit_launches;
-    if (tasks) *tasks = ctx->call_commit_tasks;
-    if (ms) *ms = ctx->timings[2];
+    float m = ctx->timings[2];          // on a multi-device context: the slowest device
+    if (ctx_is_multi(ctx)) { m = 0; for (const eg_ctx *c : ctx->children) m = std::max(m, c->timings[2]); }
+    if (launches) *launches = l;
+    if (tasks) *tasks = t;
+    if (ms) *ms = m;
     return EG_SUCCESS;
 }
 
@@ -959,8 +637,7 @@ extern "C" eg_status eg_selftest_field(eg_ctx *ctx, size_t n, uint64_t seed, uin
 #ifndef EG_HOSTSIM
     unsigned long long *d = (unsigned long long *)(ctx->d_status + 64);
     CU(cudaMemsetAsync(d, 0, 8, ctx->stream));
-    k_selftest_field<<<grid_for(n, 128), 128, 0, ctx->stream>>>(n, seed, d);
-    ctx->launches++;
+    launch_flat(ctx, k_selftest_field, n, 128, n, seed, d);
     unsigned long long h = 0;
     CU(cudaMemcpyAsync(&h, d, 8, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
