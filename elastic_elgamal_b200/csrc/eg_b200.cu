@@ -44,6 +44,7 @@ template <class K> static cudaError_t cudaOccupancyMaxActiveBlocksPerMultiproces
 
 #include "../../include/eg_b200.h"
 #include "kernels.cuh"
+#include "weighted_sum.cuh"
 
 using namespace eg;
 
@@ -105,6 +106,7 @@ struct eg_ctx {
     std::vector<uint8_t> host_tally;        // child of a multi context: its partial tally, host copy
     uint32_t comm_bad = 0;                  // host copy of the combine kernel's flag (comm_combine / comm_check)
     bool comm_pending = false;
+    dev_buf ws[13];                         // scratch of eg_ciphertexts_weighted_sum (api_weighted_sum.inc)
 };
 
 struct eg_dlog_table {
@@ -725,6 +727,7 @@ extern "C" void eg_ctx_destroy(eg_ctx *ctx) {
                        &ctx->adm, &ctx->misc, &ctx->slots, &ctx->consts, &ctx->res_big, &ctx->ring_scratch,
                        &ctx->in2[0], &ctx->in2[1], &ctx->in2[2], &ctx->term, &ctx->gather, &ctx->xtab};
     for (dev_buf *b : bufs) if (b->p) cudaFree(b->p);
+    for (dev_buf &b : ctx->ws) if (b.p) cudaFree(b.p);
     if (ctx->d_table_g) cudaFree(ctx->d_table_g);
     if (ctx->d_table_k) cudaFree(ctx->d_table_k);
     if (ctx->d_table_h) cudaFree(ctx->d_table_h);
@@ -819,5 +822,7 @@ extern "C" eg_status eg_ctx_set_blinding_base(eg_ctx *ctx, const uint8_t base[32
 #include "api_decrypt_side.inc"
 
 #include "api_sigma_provers.inc"
+
+#include "api_weighted_sum.inc"
 
 #include "api_multi.inc"

@@ -224,6 +224,42 @@ class Engine:
         self._check(self.lib.eg_ciphertexts_sum(self.h, n_parts, n_cts, _addr(parts), _addr(out), _addr(ok)))
         return out, bool(ok[0])
 
+    def weighted_sum(self, cts, scalars, verdicts=None, ct_stride=None, n_cts=None):
+        """The weighted tally fold sum_i [scalars[i]] cts[i] over the items with verdicts[i] == 0 (every item when verdicts
+        is None): (out (n_cts, 64), ok).  `cts` is an (n, n_cts, 64) array, or with `ct_stride` an (n, item_stride) record
+        buffer whose ciphertext j sits at byte j * ct_stride of each record (e.g. QV ballots: ct_stride = the vote range-proof
+        record, n_cts = options; n_cts=None: as many as fit).  `scalars` (n, 32) are canonical scalars; a 1-D integer array
+        is taken as u64 weights.  Variable-time in the scalars: weights are public."""
+        n_cts, item_stride, ct_stride, cts, scalars, verdicts = self._weighted_args(cts, scalars, verdicts, ct_stride, n_cts)
+        n = scalars.shape[0]
+        out, ok = np.empty((n_cts, 64), np.uint8), np.zeros(1, np.uint8)
+        self._check(self.lib.eg_ciphertexts_weighted_sum(self.h, n, n_cts, item_stride, ct_stride, _addr(cts), _addr(scalars),
+                                                         _addr(verdicts), _addr(out), _addr(ok)))
+        return out, bool(ok[0])
+
+    @staticmethod
+    def _weighted_args(cts, scalars, verdicts, ct_stride, n_cts=None):
+        scalars = np.asarray(scalars)
+        if scalars.ndim == 1:
+            scalars = np.ascontiguousarray(scalars, dtype="<u8").view(np.uint8).reshape(-1, 8)
+            scalars = np.concatenate([scalars, np.zeros((scalars.shape[0], 24), np.uint8)], axis=1)
+        scalars = _u8(scalars, (-1, 32))
+        n = scalars.shape[0]
+        if ct_stride is None:
+            cts = _u8(cts)
+            n_cts = cts.shape[1] if cts.ndim == 3 else cts.shape[1] // 64
+            cts = cts.reshape(n, n_cts * 64)
+            item_stride, ct_stride = 64 * n_cts, 64
+        else:
+            cts = _u8(cts)
+            cts = cts.reshape(n, -1)
+            item_stride = cts.shape[1]
+            if n_cts is None:
+                n_cts = (item_stride - 64) // ct_stride + 1
+        if verdicts is not None:
+            verdicts = _u8(verdicts, (n,))
+        return n_cts, item_stride, ct_stride, cts, scalars, verdicts
+
     # ---- proofs
     def verify_zero(self, cts, proofs):
         cts, proofs = _u8(cts, (-1, 64)), _u8(proofs, (-1, 64))
@@ -588,6 +624,10 @@ class Engine:
 
     def ciphertexts_sum_dev(self, n_parts, n_cts, d_parts, d_out, d_bad=None):
         self._check(self.lib.eg_ciphertexts_sum_dev(self.h, n_parts, n_cts, d_parts, d_out, d_bad))
+
+    def weighted_sum_dev(self, n, n_cts, item_stride, ct_stride, d_cts, d_scalars, d_verdicts, d_out, d_ok):
+        self._check(self.lib.eg_ciphertexts_weighted_sum_dev(self.h, n, n_cts, item_stride, ct_stride, d_cts, d_scalars, d_verdicts,
+                                                             d_out, d_ok))
 
     def verify_choice_dev(self, n, options, single, d_choices, d_rings, d_sums, d_verdicts, d_tally):
         self._check(self.lib.eg_verify_choice_batch_dev(self.h, n, options, int(single), d_choices, d_rings, d_sums,

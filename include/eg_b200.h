@@ -136,6 +136,21 @@ eg_status eg_ciphertexts_lincomb_batch(eg_ctx *ctx, size_t n, uint32_t terms, co
  * each row = n_cts ciphertexts.  Used to combine per-GPU partial tallies. ok = 0 if any element is malformed. */
 eg_status eg_ciphertexts_sum(eg_ctx *ctx, size_t n_parts, size_t n_cts, const uint8_t *parts /* n_parts*n_cts*64 */,
                              uint8_t *out /* n_cts*64 */, uint8_t *ok /* 1 */);
+/* The weighted tally fold  total[j] += cts[i][j] * scalars[i]  (Ciphertext Mul<&Scalar> src/encryption.rs:197 / Mul<u64> :208,
+ * Add :163) over the items i with verdicts[i] == EG_V_OK; every item when verdicts is NULL.  Ciphertext j of item i is the
+ * 64 bytes at cts + i*item_stride + j*ct_stride, so the `choices` buffer of eg_verify_choice_batch (item_stride = 64*options,
+ * ct_stride = 64) and a QV ballot buffer (item_stride = eg_qv_ballot_size, ct_stride = the vote range-proof record) are
+ * read where they are.  scalars: n canonical 32-byte scalars (Ristretto::serialize_scalar); a u64 weight w is w
+ * little-endian, zero-padded.  out = n_cts ciphertexts (Ciphertext::to_bytes).  ok = 1, or 0 when an included item has a
+ * non-canonical scalar or an element that does not decode (out is then n_cts identity ciphertexts).  Excluded items are
+ * neither decoded nor checked.  No included item, or n = 0: identity ciphertexts (Ciphertext::zero), ok = 1.
+ * n_cts in 1..64; ct_stride >= 64 when n_cts > 1; item_stride >= (n_cts - 1) * ct_stride + 64; else EG_ERR_INVALID_ARG.
+ * Variable-time in the scalars (weights are public): do not pass secret scalars.  Needs no receiver key.
+ * Multi-device context: the batch is sharded and the result is the total over all devices.  With an attached
+ * communicator the call is NOT collective: the result covers this rank's items. */
+eg_status eg_ciphertexts_weighted_sum(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
+                                      const uint8_t *cts, const uint8_t *scalars /* n*32 */, const uint8_t *verdicts /* n or NULL */,
+                                      uint8_t *out /* n_cts*64 */, uint8_t *ok /* 1 */);
 
 /* ---- wire format (src/serde.rs:19-80) ----------------------------------------------------------- */
 
@@ -539,6 +554,11 @@ eg_status eg_encrypt_range_batch_dev(eg_ctx *ctx, const eg_range *range, const c
  * of per-GPU partial tallies.  *d_bad_flag (optional, device) becomes non-zero when a part does not decode. */
 eg_status eg_ciphertexts_sum_dev(eg_ctx *ctx, size_t n_parts, size_t n_cts, const uint8_t *d_parts, uint8_t *d_out,
                                  uint32_t *d_bad_flag);
+/* eg_ciphertexts_weighted_sum on device pointers (single-device context only, EG_ERR_INVALID_ARG otherwise); synchronous
+ * like the other _dev verifiers.  d_ok is one device byte. */
+eg_status eg_ciphertexts_weighted_sum_dev(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
+                                          const uint8_t *d_cts, const uint8_t *d_scalars, const uint8_t *d_verdicts,
+                                          uint8_t *d_out, uint8_t *d_ok);
 
 /* ---- instrumentation --------------------------------------------------------------------------- */
 /* Number of kernels this context has launched since creation (bench.py's `gpu_launches`). */

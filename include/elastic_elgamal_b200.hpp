@@ -194,6 +194,26 @@ class Engine {
         return to_ciphertexts(out);
     }
 
+    // The weighted tally fold total[j] += items[i][j] * scalars[i] (src/encryption.rs:163,197) over the items whose verdict
+    // is 0 (every item when `verdicts` is empty), e.g. the verdicts of verify_choice_batch.  Variable-time in the scalars.
+    std::vector<Ciphertext> weighted_sum(const std::vector<std::vector<Ciphertext>> &items, const std::vector<Scalar> &scalars,
+                                         const std::vector<uint8_t> &verdicts = {}) {
+        const size_t n = items.size(), n_cts = n ? items[0].size() : 1;
+        if (scalars.size() != n || (!verdicts.empty() && verdicts.size() != n))
+            throw Error(EG_ERR_INVALID_ARG, "one scalar and verdict per item");
+        std::vector<uint8_t> s, c, out(n_cts * 64);
+        uint8_t ok = 0;
+        for (size_t i = 0; i < n; i++) {
+            if (items[i].size() != n_cts) throw Error(EG_ERR_INVALID_ARG, "items must have the same number of ciphertexts");
+            s.insert(s.end(), scalars[i].begin(), scalars[i].end());
+            for (const auto &ct : items[i]) append(c, ct);
+        }
+        check(eg_ciphertexts_weighted_sum(ctx_, n, (uint32_t)n_cts, 64 * n_cts, 64, c.data(), s.data(),
+                                          verdicts.empty() ? nullptr : verdicts.data(), out.data(), &ok));
+        if (!ok) throw Error(EG_ERR_INVALID_ARG, "malformed element or scalar in a weighted sum");
+        return to_ciphertexts(out);
+    }
+
     ChoiceBatchResult verify_qv_batch(uint32_t options, uint64_t credits, const std::vector<QuadraticVotingBallot> &ballots) {
         eg_qv_params qp;
         check(eg_qv_params_new(options, credits, &qp));

@@ -151,6 +151,10 @@ extern "C" {
     pub fn eg_encrypt_range_batch_dev(ctx: *mut eg_ctx, range: *const eg_range, transcript_label: *const c_char, n: usize, d_values: *const u64, d_wide_rand: *const u8, seed: *const u8, counter_base: u64, d_cts: *mut u8, d_partials: *mut u8, d_ring_proofs: *mut u8) -> eg_status;
     pub fn eg_ciphertexts_sum_dev(ctx: *mut eg_ctx, n_parts: usize, n_cts: usize, d_parts: *const u8, d_out: *mut u8,
                                   d_bad: *mut u32) -> eg_status;
+    pub fn eg_ciphertexts_weighted_sum(ctx: *mut eg_ctx, n: usize, n_cts: u32, item_stride: usize, ct_stride: usize, cts: *const u8,
+                                       scalars: *const u8, verdicts: *const u8, out: *mut u8, ok: *mut u8) -> eg_status;
+    pub fn eg_ciphertexts_weighted_sum_dev(ctx: *mut eg_ctx, n: usize, n_cts: u32, item_stride: usize, ct_stride: usize, d_cts: *const u8,
+                                           d_scalars: *const u8, d_verdicts: *const u8, d_out: *mut u8, d_ok: *mut u8) -> eg_status;
 
     pub fn eg_base64url_chars(bytes_per_item: usize) -> usize;
     pub fn eg_base64url_decode_batch(ctx: *mut eg_ctx, n: usize, bytes_per_item: usize, text: *const c_char, raw: *mut u8,

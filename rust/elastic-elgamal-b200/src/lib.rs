@@ -768,6 +768,32 @@ impl Engine {
         Ok(ciphertexts(&out))
     }
 
+    /// The weighted tally fold `total[j] += items[i][j] * scalars[i]` (encryption.rs:163,197) over the items whose verdict is
+    /// 0 (every item with `None`), e.g. the verdicts of `verify_choices`.  Every item has the same number of ciphertexts
+    /// (1..=64).  Variable-time in the scalars: weights are public.
+    pub fn weighted_sum(&self, items: &[Vec<Ciphertext<Ristretto>>], scalars: &[Scalar], verdicts: Option<&[u8]>) -> Result<Vec<Ciphertext<Ristretto>>, EngineError> {
+        let n = items.len();
+        assert!(scalars.len() == n && verdicts.map_or(true, |v| v.len() == n), "one scalar and verdict per item");
+        let n_cts = items.first().map_or(1, |r| r.len());
+        let (mut s, mut c) = (Vec::with_capacity(n * 32), Vec::with_capacity(n * n_cts * 64));
+        for (row, k) in items.iter().zip(scalars) {
+            assert!(row.len() == n_cts, "items must have the same number of ciphertexts");
+            let mut b = [0_u8; 32];
+            Ristretto::serialize_scalar(k, &mut b);
+            s.extend_from_slice(&b);
+            for ct in row {
+                c.extend_from_slice(&ct.to_bytes());
+            }
+        }
+        let (mut out, mut ok) = (vec![0_u8; n_cts * 64], [0_u8; 1]);
+        let v = verdicts.map_or(std::ptr::null(), |v| v.as_ptr());
+        self.check(unsafe {
+            sys::eg_ciphertexts_weighted_sum(self.ctx, n, n_cts as u32, 64 * n_cts, 64, c.as_ptr(), s.as_ptr(), v, out.as_mut_ptr(), ok.as_mut_ptr())
+        })?;
+        debug_assert!(ok[0] == 1, "typed inputs are canonical");
+        Ok(ciphertexts(&out))
+    }
+
     // ------------------------------------------------------------------ creation side
 
     /// `key.encrypt(value, rng)` over a batch (keys/impls.rs:16-23).
