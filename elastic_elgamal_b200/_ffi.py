@@ -97,6 +97,8 @@ PROTOTYPES = {
     "eg_verify_qv_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(QvParams), C.c_size_t, P8, P8, P8]),
     "eg_verify_shares_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(KeySet), C.c_size_t, C.c_uint32, C.POINTER(C.c_uint32), P8, P8, P8, P8]),
     "eg_combine_decrypt_batch_dev": (C.c_int32, [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_size_t, C.c_uint32, P8, P8, C.c_void_p, P8, P8]),
+    "eg_combine_decrypt_accepted_batch": (C.c_int32, [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32), C.c_size_t, P8, P8, P8, C.c_void_p, P8, P8]),
+    "eg_combine_decrypt_accepted_batch_dev": (C.c_int32, [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32), C.c_size_t, P8, P8, P8, C.c_void_p, P8, P8]),
     "eg_encrypt_bool_batch_dev": (C.c_int32, [C.c_void_p, C.c_size_t, P8, P8, P8, C.c_uint64, P8, P8]),
     "eg_encrypt_choice_batch_dev": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_int, P8, P8, P8, C.c_uint64, P8, P8, P8]),
     "eg_encrypt_range_batch_dev": (C.c_int32, [C.c_void_p, C.POINTER(Range), C.c_char_p, C.c_size_t, P8, P8, P8, C.c_uint64, P8, P8, P8]),

@@ -1737,6 +1737,86 @@ EG_HD void dlog_build_body(const dlog_build_params &P, size_t tid) {
     }
 }
 
+// lagrange_coefficients (sharing/mod.rs:139-170) of t <= EG_MSM_MAXV distinct participant indexes, each folded with the
+// common scale prod_b (i_b + 1):  coeff[a] = scale / ((i_a + 1) prod_{b != a} (i_b - i_a)).  The t denominators share one
+// inversion (Montgomery's trick: prefix products, one sc_invert, back-substitution), as the reference's invert_scalars.
+// The host's batch constants (lagrange_scaled) and k_combine_select's per-tally coefficients both come from here.
+EG_HD void lagrange_scaled_coeffs(uint32_t t, const uint32_t *indexes, sc *coeff) {
+    sc scale = sc_from_u64(1), pre[EG_MSM_MAXV];
+    for (uint32_t a = 0; a < t; a++) {
+        sc e = sc_from_u64((uint64_t)indexes[a] + 1), mag = e;
+        sc_mul(scale, scale, e);
+        bool sign = false;
+        for (uint32_t b = 0; b < t; b++) {
+            if (b == a) continue;
+            if (indexes[a] > indexes[b]) { sign = !sign; e = sc_from_u64(indexes[a] - indexes[b]); }
+            else e = sc_from_u64(indexes[b] - indexes[a]);
+            sc_mul(mag, mag, e);
+        }
+        if (sign) sc_neg(mag, mag);
+        coeff[a] = mag;                                     // the denominator, until the back-substitution below
+        if (a == 0) pre[0] = mag; else sc_mul(pre[a], pre[a - 1], mag);
+    }
+    sc inv;
+    sc_invert(inv, pre[t - 1]);                             // 1 / (denominator 0 ... denominator a), a = t - 1 first
+    for (uint32_t a = t; a-- > 0;) {
+        sc d = coeff[a], c;
+        if (a > 0) sc_mul(c, inv, pre[a - 1]); else c = inv;     // 1 / denominator a
+        sc_mul(inv, inv, d);
+        sc_mul(coeff[a], c, scale);     // (sum lambda_j S_j) * scale == sum (lambda_j * scale) S_j
+    }
+}
+
+// Params::combine_shares (sharing/mod.rs:302-325) on the shares a tallier accepted: tally i has n_shares candidate shares
+// (column j from participant indexes[j]) and combines the first t columns, in column order, whose verdict byte is EG_V_OK.
+// Their encodings go to a compact row of t shares in `sel`, so that the decode reads no other column, and their Lagrange
+// coefficients to the planar scalars `coeff` (k_msm reads them as scalar_src kind 1).  When the selection is columns
+// 0 .. t-1 (every tally of a batch without rejected shares) the batch constants `first_coeff` are copied instead.  A tally
+// with fewer than t accepted shares (combine_shares returns None) gets identity encodings, zero coefficients and flag bit
+// 2u, which dlog_lookup_body turns into found 3.
+struct combine_select_params {
+    size_t n;
+    uint32_t t, n_shares;
+    const uint8_t *shares;          // n x n_shares x 32
+    const uint8_t *verdicts;        // n x n_shares
+    const uint32_t *indexes;        // n_shares distinct participant indexes
+    const uint32_t *first_coeff;    // coefficients of columns 0 .. t-1, 8 words each
+    uint8_t *sel;                   // n x t x 32
+    uint32_t *coeff;                // planar scalars (8 words): t per item
+    uint32_t *flags;                // per item; bit 2u = fewer than t accepted shares
+};
+
+EG_HD void combine_select_body(const combine_select_params &P, size_t item) {
+    uint32_t col[EG_MSM_MAXV], idx[EG_MSM_MAXV], k = 0;
+    bool first = true;
+    const uint8_t *v = P.verdicts + item * P.n_shares;
+    for (uint32_t j = 0; j < P.n_shares && k < P.t; j++)
+        if (v[j] == 0) { first = first && j == k; col[k] = j; idx[k] = P.indexes[j]; k++; }
+    uint8_t *out = P.sel + item * P.t * 32;
+    const uint32_t zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    if (k < P.t) {
+        for (uint32_t j = 0; j < P.t; j++) {
+            store32_bytes(out + 32 * j, zero);
+            planar_store_words(P.coeff, P.n, j, 8, item, zero);
+        }
+        P.flags[item] |= 2u;
+        return;
+    }
+    const uint8_t *row = P.shares + item * P.n_shares * 32;
+    uint32_t w[8];
+    for (uint32_t j = 0; j < P.t; j++) {
+        load32_bytes(w, row + 32 * col[j]);
+        store32_bytes(out + 32 * j, w);
+    }
+    if (first) {
+        for (uint32_t j = 0; j < P.t; j++) planar_store_words(P.coeff, P.n, j, 8, item, P.first_coeff + 8 * j);
+        return;
+    }
+    sc c[EG_MSM_MAXV];
+    lagrange_scaled_coeffs(P.t, idx, c);
+    for (uint32_t j = 0; j < P.t; j++) planar_store_words(P.coeff, P.n, j, 8, item, c[j].v);
+}
+
 // decrypt_to_element (decryption.rs:129-131) + DiscreteLogTable::get (encryption.rs:287-297):
 // M = B - D (D = recombined share, a planar point), identity -> Some(0), else table probe on the encoding
 struct dlog_lookup_params {
@@ -1746,9 +1826,9 @@ struct dlog_lookup_params {
     size_t cap;
     const uint32_t *keys;
     const unsigned long long *vals;
-    const uint32_t *flags;      // malformed inputs
+    const uint32_t *flags;      // 1u: malformed input; 2u: fewer accepted shares than the threshold (k_combine_select)
     unsigned long long *values;
-    uint8_t *found;             // 1 found, 0 absent, 2 malformed input
+    uint8_t *found;             // 1 found, 0 absent, 2 malformed input, 3 not combined
     uint8_t *enc;               // n * 32 or null: the encoding of M (read by the giant-step walk of a BSGS table)
 };
 
@@ -1766,6 +1846,8 @@ EG_HD uint8_t dlog_probe(const uint32_t w[8], size_t cap, const uint32_t *keys, 
 }
 
 EG_HD void dlog_lookup_body(const dlog_lookup_params &P, size_t item) {
+    // combine_shares returned None before anything was decrypted: 3 wins over 2, and found != 0 keeps the walk away
+    if (P.flags[item] & 2u) { P.found[item] = 3; P.values[item] = 0; return; }
     if (P.flags[item] & 1u) { P.found[item] = 2; P.values[item] = 0; return; }
     ge_ext B, D, M;
     planar_load_point(B, P.pts, P.n, P.b_p_index, item);

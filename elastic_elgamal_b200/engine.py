@@ -508,6 +508,20 @@ class Engine:
                                                       _addr(values), _addr(found)))
         return values, found
 
+    def combine_decrypt_accepted(self, threshold, indexes, cts, shares, verdicts, table):
+        """combine_shares on the first `threshold` shares of each tally whose verdict (as verify_shares returns it) is
+        EG_V_OK, in column order, then decrypt: (values, found), found as combine_decrypt, or 3 (value 0) when fewer than
+        `threshold` shares of the tally are accepted.  shares (n, len(indexes), 32), verdicts (n, len(indexes))."""
+        s = len(indexes)
+        cts = _u8(cts, (-1, 64))
+        n = cts.shape[0]
+        shares, verdicts = _u8(shares, (n, s, 32)), _u8(verdicts, (n, s))
+        idx = (C.c_uint32 * s)(*indexes)
+        values, found = np.zeros(n, np.uint64), np.zeros(n, np.uint8)
+        self._check(self.lib.eg_combine_decrypt_accepted_batch(self.h, threshold, s, idx, n, _addr(cts), _addr(shares), _addr(verdicts),
+                                                               table.h, _addr(values), _addr(found)))
+        return values, found
+
     # ---- decryption side (the holder's secret key; randomness as for encrypt_*: `wide_rand` blocks or `seed=`)
     @staticmethod
     def _secret(secret):
@@ -628,6 +642,11 @@ class Engine:
     def weighted_sum_dev(self, n, n_cts, item_stride, ct_stride, d_cts, d_scalars, d_verdicts, d_out, d_ok):
         self._check(self.lib.eg_ciphertexts_weighted_sum_dev(self.h, n, n_cts, item_stride, ct_stride, d_cts, d_scalars, d_verdicts,
                                                              d_out, d_ok))
+
+    def combine_decrypt_accepted_dev(self, threshold, indexes, n, d_cts, d_shares, d_verdicts, table, d_values, d_found):
+        idx = (C.c_uint32 * len(indexes))(*indexes)
+        self._check(self.lib.eg_combine_decrypt_accepted_batch_dev(self.h, threshold, len(indexes), idx, n, d_cts, d_shares, d_verdicts,
+                                                                   table.h, d_values, d_found))
 
     def verify_choice_dev(self, n, options, single, d_choices, d_rings, d_sums, d_verdicts, d_tally):
         self._check(self.lib.eg_verify_choice_batch_dev(self.h, n, options, int(single), d_choices, d_rings, d_sums,

@@ -318,8 +318,9 @@ void      eg_dlog_table_destroy(eg_dlog_table *table);
  * eg_dlog_table_create(lo, hi) would return if it could be built.  When hi - lo <= baby_steps, the result is that range
  * table and no walk ever runs.
  * EG_ERR_INVALID_ARG unless hi >= lo, 256 <= baby_steps <= 2^28 and J <= 2^32.  The table is accepted wherever an
- * eg_dlog_table is: eg_decrypt_batch, eg_combine_decrypt_batch(_dev), eg_dlog_lookup_batch, single- and multi-device
- * contexts (one replica per device), eg_dlog_table_destroy.  A lookup's time depends on the value it finds. */
+ * eg_dlog_table is: eg_decrypt_batch, eg_combine_decrypt_batch(_dev), eg_combine_decrypt_accepted_batch(_dev),
+ * eg_dlog_lookup_batch, single- and multi-device contexts (one replica per device), eg_dlog_table_destroy.  A lookup's
+ * time depends on the value it finds. */
 eg_status eg_dlog_table_create_bsgs(eg_ctx *ctx, uint64_t lo, uint64_t hi, uint64_t baby_steps, eg_dlog_table **out);
 
 /* DiscreteLogTable::get (src/encryption.rs:287-297) over a batch of 32-byte element encodings, for either kind of table:
@@ -336,6 +337,22 @@ eg_status eg_combine_decrypt_batch(eg_ctx *ctx, uint32_t threshold, const uint32
                                    size_t n_tallies, uint32_t share_stride /* shares per tally in `shares` */,
                                    const uint8_t *cts /* n_tallies*64 */, const uint8_t *shares,
                                    const eg_dlog_table *table, uint64_t *values /* n */, uint8_t *found /* n */);
+
+/* Params::combine_shares (src/sharing/mod.rs:302-325) on the shares a tallier accepted, then VerifiableDecryption::decrypt
+ * (src/decryption.rs:138-144) through DiscreteLogTable::get (src/encryption.rs:287-297).  Tally i has n_shares candidate
+ * shares; share j comes from participant indexes[j], and verdicts[i*n_shares + j] is its verdict byte, as
+ * eg_verify_shares_batch writes it.  For every tally, the first `threshold` shares, in column order, whose verdict is EG_V_OK
+ * are combined (the reference's tallier passes the shares it accepted, and combine_shares takes the first t of them).
+ *   found[i] = 1 / 0 / 2 as eg_combine_decrypt_batch (in table / not in table / an element that is used does not decode),
+ *   found[i] = 3 when fewer than `threshold` shares of the tally are accepted (combine_shares returns None); value 0.
+ *   Found 3 wins over 2: a tally that is not combined is not decrypted.
+ * Shares that are rejected, or accepted but beyond the first `threshold`, are never decoded.  indexes need not be ascending.
+ * 1 <= threshold <= 16, threshold <= n_shares <= 64, indexes distinct (all n_shares of them); else EG_ERR_INVALID_ARG.
+ * Multi-device contexts shard the tallies.  The time depends on the verdicts and indexes only, which are public. */
+eg_status eg_combine_decrypt_accepted_batch(eg_ctx *ctx, uint32_t threshold, uint32_t n_shares, const uint32_t *indexes /* n_shares */,
+                                            size_t n_tallies, const uint8_t *cts /* n*64 */,
+                                            const uint8_t *shares /* n*n_shares*32 */, const uint8_t *verdicts /* n*n_shares */,
+                                            const eg_dlog_table *table, uint64_t *values /* n */, uint8_t *found /* n */);
 
 /* ---- encryption side (encrypt_* drop-ins with caller-supplied randomness) ----------------------- */
 
@@ -538,6 +555,11 @@ eg_status eg_verify_shares_batch_dev(eg_ctx *ctx, const eg_keyset *keyset, size_
 eg_status eg_combine_decrypt_batch_dev(eg_ctx *ctx, uint32_t threshold, const uint32_t *indexes, size_t n_tallies, uint32_t share_stride,
                                        const uint8_t *d_cts, const uint8_t *d_shares, const eg_dlog_table *table, uint64_t *d_values,
                                        uint8_t *d_found);
+/* eg_combine_decrypt_accepted_batch on device buffers: the verdicts of eg_verify_shares_batch_dev can be passed as they are */
+eg_status eg_combine_decrypt_accepted_batch_dev(eg_ctx *ctx, uint32_t threshold, uint32_t n_shares, const uint32_t *indexes,
+                                                size_t n_tallies, const uint8_t *d_cts, const uint8_t *d_shares,
+                                                const uint8_t *d_verdicts, const eg_dlog_table *table, uint64_t *d_values,
+                                                uint8_t *d_found);
 /* Provers on device buffers: values in, objects out, all in HBM of the context's device.  Randomness: `seed` (32 bytes, HOST
  * pointer) + counter_base as in the _seeded forms, or -- with seed == NULL -- blocks already resident at d_wide_rand in the
  * layout of the host forms.  The domain checks the host forms make on the values (exactly one option for `single`, value

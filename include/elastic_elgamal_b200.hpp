@@ -322,6 +322,32 @@ class Engine {
         return out;
     }
 
+    // The tallier of examples/voting.rs: combine_shares on the first `threshold` shares of each tally whose verdict (as
+    // verify_shares_batch returns it) is Ok, in the order of `indexes`, then decrypt.  shares / verdicts are tally-major,
+    // indexes.size() per tally.  `enough[i]` (optional) is false when fewer than `threshold` shares were accepted (combine_shares
+    // returns None); such a tally is reported as not found.
+    std::vector<DecryptedValue> combine_decrypt_accepted_batch(uint32_t threshold, const std::vector<uint32_t> &indexes,
+                                                               const std::vector<Ciphertext> &cts, const std::vector<Element> &shares,
+                                                               const std::vector<Verdict> &verdicts, const eg_dlog_table *table,
+                                                               std::vector<bool> *enough = nullptr) {
+        const size_t n = cts.size(), s = indexes.size();
+        if (shares.size() != n * s || verdicts.size() != n * s) throw Error(EG_ERR_LEN_MISMATCH, "batch size mismatch");
+        std::vector<uint8_t> c, sh, v(n * s), found(n);
+        std::vector<uint64_t> values(n);
+        for (const auto &ct : cts) append(c, ct);
+        for (const auto &e : shares) sh.insert(sh.end(), e.begin(), e.end());
+        for (size_t k = 0; k < n * s; k++) v[k] = (uint8_t)verdicts[k];
+        check(eg_combine_decrypt_accepted_batch(ctx_, threshold, (uint32_t)s, indexes.data(), n, c.data(), sh.data(), v.data(), table,
+                                                values.data(), found.data()));
+        std::vector<DecryptedValue> out(n);
+        if (enough) enough->assign(n, true);
+        for (size_t i = 0; i < n; i++) {
+            out[i] = DecryptedValue{found[i] == 1, values[i]};
+            if (enough && found[i] == 3) (*enough)[i] = false;
+        }
+        return out;
+    }
+
     // secret.decrypt(ct, &table) over a batch (keys/impls.rs:160-177); table == nullptr: decrypt_to_element only (found = decoded)
     std::vector<DecryptedValue> decrypt_batch(const Scalar &secret, const std::vector<Ciphertext> &cts, const eg_dlog_table *table,
                                               std::vector<Element> *elements = nullptr) {

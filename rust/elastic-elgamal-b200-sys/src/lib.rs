@@ -126,6 +126,9 @@ extern "C" {
     pub fn eg_combine_decrypt_batch(ctx: *mut eg_ctx, threshold: u32, indexes: *const u32, n_tallies: usize,
                                     share_stride: u32, cts: *const u8, shares: *const u8, table: *const eg_dlog_table,
                                     values: *mut u64, found: *mut u8) -> eg_status;
+    pub fn eg_combine_decrypt_accepted_batch(ctx: *mut eg_ctx, threshold: u32, n_shares: u32, indexes: *const u32, n_tallies: usize,
+                                             cts: *const u8, shares: *const u8, verdicts: *const u8, table: *const eg_dlog_table,
+                                             values: *mut u64, found: *mut u8) -> eg_status;
 
     pub fn eg_verify_bool_batch_dev(ctx: *mut eg_ctx, n: usize, d_cts: *const u8, d_proofs: *const u8, d_verdicts: *mut u8) -> eg_status;
     pub fn eg_verify_choice_batch_dev(ctx: *mut eg_ctx, n: usize, options: u32, single: c_int, d_choices: *const u8,
@@ -146,6 +149,7 @@ extern "C" {
     pub fn eg_verify_qv_batch_dev(ctx: *mut eg_ctx, params: *const eg_qv_params, n: usize, d_ballots: *const u8, d_verdicts: *mut u8, d_tally: *mut u8) -> eg_status;
     pub fn eg_verify_shares_batch_dev(ctx: *mut eg_ctx, keyset: *const eg_keyset, n_tallies: usize, n_shares: u32, indexes: *const u32, d_cts: *const u8, d_shares: *const u8, d_proofs: *const u8, d_verdicts: *mut u8) -> eg_status;
     pub fn eg_combine_decrypt_batch_dev(ctx: *mut eg_ctx, threshold: u32, indexes: *const u32, n_tallies: usize, share_stride: u32, d_cts: *const u8, d_shares: *const u8, table: *const eg_dlog_table, d_values: *mut u64, d_found: *mut u8) -> eg_status;
+    pub fn eg_combine_decrypt_accepted_batch_dev(ctx: *mut eg_ctx, threshold: u32, n_shares: u32, indexes: *const u32, n_tallies: usize, d_cts: *const u8, d_shares: *const u8, d_verdicts: *const u8, table: *const eg_dlog_table, d_values: *mut u64, d_found: *mut u8) -> eg_status;
     pub fn eg_encrypt_bool_batch_dev(ctx: *mut eg_ctx, n: usize, d_values: *const u8, d_wide_rand: *const u8, seed: *const u8, counter_base: u64, d_cts: *mut u8, d_proofs: *mut u8) -> eg_status;
     pub fn eg_encrypt_choice_batch_dev(ctx: *mut eg_ctx, n: usize, options: u32, single: c_int, d_values: *const u8, d_wide_rand: *const u8, seed: *const u8, counter_base: u64, d_choices: *mut u8, d_ring_proofs: *mut u8, d_sum_proofs: *mut u8) -> eg_status;
     pub fn eg_encrypt_range_batch_dev(ctx: *mut eg_ctx, range: *const eg_range, transcript_label: *const c_char, n: usize, d_values: *const u64, d_wide_rand: *const u8, seed: *const u8, counter_base: u64, d_cts: *mut u8, d_partials: *mut u8, d_ring_proofs: *mut u8) -> eg_status;

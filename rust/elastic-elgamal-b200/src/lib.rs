@@ -58,6 +58,13 @@ impl From<flat::FlatError> for EngineError {
     }
 }
 
+/// Why a tally of [`Engine::combine_accepted_and_decrypt`] has no decryption.
+#[derive(Debug, Clone, Copy, PartialEq, Eq)]
+pub enum CombineError {
+    /// Fewer than `threshold` of the tally's shares were accepted: `Params::combine_shares` returns `None`.
+    NotEnoughShares,
+}
+
 /// One context: a single GPU (`new`), all chosen GPUs of the box (`new_multi`), or one rank of a multi-process job
 /// (`new` + `attach_comm`).  `!Sync`: use from one thread at a time; independent across instances.
 pub struct Engine {
@@ -634,6 +641,40 @@ impl Engine {
             sys::eg_combine_decrypt_batch(self.ctx, t as u32, idx.as_ptr(), n, t as u32, c.as_ptr(), sh.as_ptr(), table.table, values.as_mut_ptr(), found.as_mut_ptr())
         })?;
         Ok(values.iter().zip(found).map(|(&v, f)| (f == 1).then_some(v)).collect())
+    }
+
+    /// The tallier of examples/voting.rs: `params.combine_shares(..)` on the shares that `verify_shares` accepted, then
+    /// `decrypt(ct, &table)`, per tally.  `shares` is `verify_shares`' output (tally-major, `indexes.len()` per tally, at
+    /// most 64); each tally combines its first `threshold` accepted shares in that order.  `Ok(Some(value))`, `Ok(None)` when
+    /// the plaintext is outside the table, `Err(CombineError::NotEnoughShares)` when fewer than `threshold` shares were
+    /// accepted (`combine_shares` returns `None`).
+    pub fn combine_accepted_and_decrypt(
+        &self,
+        threshold: usize,
+        indexes: &[usize],
+        cts: &[Ciphertext<Ristretto>],
+        shares: &[Result<VerifiableDecryption<Ristretto>, VerificationError>],
+        table: &DlogTable<'_>,
+    ) -> Result<Vec<Result<Option<u64>, CombineError>>, EngineError> {
+        let (n, s) = (cts.len(), indexes.len());
+        assert_eq!(shares.len(), n * s);
+        let idx: Vec<u32> = indexes.iter().map(|&i| i as u32).collect();
+        let c: Vec<u8> = cts.iter().flat_map(|ct| ct.to_bytes()).collect();
+        let sh: Vec<u8> = shares.iter().flat_map(|share| share.as_ref().map_or_else(|_| vec![0_u8; 32], |d| d.to_bytes().to_vec())).collect();
+        let verdicts: Vec<u8> = shares.iter().map(|share| if share.is_ok() { sys::EG_V_OK } else { sys::EG_V_CHALLENGE_MISMATCH }).collect();
+        let (mut values, mut found) = (vec![0_u64; n], vec![0_u8; n]);
+        self.check(unsafe {
+            sys::eg_combine_decrypt_accepted_batch(self.ctx, threshold as u32, s as u32, idx.as_ptr(), n, c.as_ptr(), sh.as_ptr(), verdicts.as_ptr(),
+                                                   table.table, values.as_mut_ptr(), found.as_mut_ptr())
+        })?;
+        Ok(values
+            .iter()
+            .zip(found)
+            .map(|(&v, f)| {
+                debug_assert!(f != 2, "typed ciphertexts and shares decode");
+                if f == 3 { Err(CombineError::NotEnoughShares) } else { Ok((f == 1).then_some(v)) }
+            })
+            .collect())
     }
 
     // ------------------------------------------------------------------ decryption side (the holder's secret key)
