@@ -102,12 +102,33 @@ void eo_transcript_start_proof(eo_transcript *t, const char *label);
 void eo_transcript_append_element(eo_transcript *t, const char *label, const eo_pt *p);
 void eo_transcript_challenge_scalar(eo_transcript *t, const char *label, eo_sc *out);
 
-/* ------------------------------------------------------------------ ChaCha20 RNG (rand_chacha) */
-typedef struct { uint8_t key[32]; uint64_t block; } eo_rng;
+/* ------------------------------------------------------------------ ChaCha20 RNG (rand_chacha)
+ * or a replay of caller-supplied blocks.  A replaying rng hands out blocks[0], blocks[1], ... in order (`block` counts the
+ * draws) so that a prover runs on exactly the blocks the library's `wide_rand` form takes.  Its state lives in the 32 key
+ * bytes, marked by EO_RNG_REPLAY_TAG, so eo_rng keeps its 40-byte layout: every caller that allocates the struct itself
+ * (the ctypes mirror in tests/oracle.py, checked against eo_rng_size()) stays valid.  A draw past the last block yields a
+ * 0xff block and leaves the rng overrun for good (eo_rng_overrun); tests/oracle.py raises on it, so a wrong draw count can
+ * neither wrap around nor pass as zeros. */
+#define EO_RNG_REPLAY_TAG "eo_rng replay v1"               /* 16 bytes, no terminator stored */
+typedef struct {
+    union {
+        uint8_t key[32];                                    /* ChaCha20 key */
+        struct {
+            uint8_t tag[16];                                /* EO_RNG_REPLAY_TAG */
+            const uint8_t *blocks;                          /* n_blocks * 64 caller-owned bytes */
+            uint64_t n_blocks;
+        } replay;
+    };
+    uint64_t block;                                         /* ChaCha20: next block counter; replay: draws so far */
+} eo_rng;
 
+size_t eo_rng_size(void);                                   /* sizeof(eo_rng) = 40, for the ctypes mirror */
 void eo_rng_from_seed(eo_rng *r, const uint8_t seed[32], uint64_t first_block);
 void eo_rng_seed_from_u64(eo_rng *r, uint64_t seed);        /* rand_core SeedableRng::seed_from_u64 */
-void eo_rng_block(eo_rng *r, uint8_t out[64]);              /* next 64-byte keystream block */
+void eo_rng_from_blocks(eo_rng *r, const uint8_t *blocks, uint64_t n_blocks);   /* replay; `blocks` must outlive r */
+int  eo_rng_overrun(const eo_rng *r);                       /* 1: a replay was asked for more blocks than it holds */
+uint64_t eo_rng_blocks_left(const eo_rng *r);            /* blocks a replay has not handed out yet (0 for ChaCha20) */
+void eo_rng_block(eo_rng *r, uint8_t out[64]);              /* next 64-byte keystream (or replayed) block */
 void eo_rng_scalar(eo_rng *r, eo_sc *out);                  /* Ristretto::generate_scalar, ristretto.rs:28-32 */
 
 /* ------------------------------------------------------------------ verdict codes

@@ -181,9 +181,29 @@ void eo_transcript_challenge_scalar(eo_transcript *t, const char *label, eo_sc *
     a += b; d ^= a; d = ROL32(d, 16); c += d; b ^= c; b = ROL32(b, 12); \
     a += b; d ^= a; d = ROL32(d, 8);  c += d; b ^= c; b = ROL32(b, 7)
 
+_Static_assert(sizeof(eo_rng) == 40, "eo_rng is allocated by callers at 40 bytes (key[32] + block)");
+_Static_assert(sizeof(EO_RNG_REPLAY_TAG) - 1 == 16, "the replay tag fills replay.tag");
+
+size_t eo_rng_size(void) { return sizeof(eo_rng); }
+
 void eo_rng_from_seed(eo_rng *r, const uint8_t seed[32], uint64_t first_block) {
     memcpy(r->key, seed, 32);
     r->block = first_block;
+}
+
+void eo_rng_from_blocks(eo_rng *r, const uint8_t *blocks, uint64_t n_blocks) {
+    memcpy(r->replay.tag, EO_RNG_REPLAY_TAG, 16);
+    r->replay.blocks = blocks;
+    r->replay.n_blocks = n_blocks;
+    r->block = 0;
+}
+
+static int rng_is_replay(const eo_rng *r) { return memcmp(r->replay.tag, EO_RNG_REPLAY_TAG, 16) == 0; }
+
+int eo_rng_overrun(const eo_rng *r) { return rng_is_replay(r) && r->block > r->replay.n_blocks; }
+
+uint64_t eo_rng_blocks_left(const eo_rng *r) {
+    return rng_is_replay(r) && r->block < r->replay.n_blocks ? r->replay.n_blocks - r->block : 0;
 }
 
 void eo_rng_seed_from_u64(eo_rng *r, uint64_t state) {
@@ -201,6 +221,13 @@ void eo_rng_seed_from_u64(eo_rng *r, uint64_t state) {
 }
 
 void eo_rng_block(eo_rng *r, uint8_t out[64]) {
+    if (rng_is_replay(r)) {
+        /* past the end: a 0xff block, and block > n_blocks from now on (eo_rng_overrun) */
+        if (r->block < r->replay.n_blocks) memcpy(out, r->replay.blocks + 64 * r->block, 64);
+        else memset(out, 0xff, 64);
+        if (r->block <= r->replay.n_blocks) r->block++;
+        return;
+    }
     uint32_t s[16], x[16];
     s[0] = 0x61707865; s[1] = 0x3320646e; s[2] = 0x79622d32; s[3] = 0x6b206574;
     for (int i = 0; i < 8; i++)

@@ -2,8 +2,8 @@
 (test_gpu_edges.py).  Random inputs almost never reach the values where integer code goes wrong, so these are chosen by hand:
 discrete-log tables whose ranges do not start at 0 or end next to 2^64, u64 plaintexts at the ends of their range, and secret
 keys and nonces whose recodings sit on the digit limits of the decryption kernels (sc_recode4, sc_wide_digit, sc_half).
-Outputs are compared with the oracle, or -- for proofs on chosen nonces, which the oracle's ChaCha20-driven prover cannot
-take -- checked by algebra with the oracle's point operations."""
+Outputs are compared with the oracle, or -- for proofs on chosen nonces -- checked by algebra with the oracle's point
+operations."""
 import ctypes as C
 import functools
 import random

@@ -19,13 +19,21 @@ QV_VARIANT_BASE = 16
 
 
 def build(force=False):
-    if force or not LIB_PATH.exists():
+    stale = LIB_PATH.exists() and any(p.stat().st_mtime > LIB_PATH.stat().st_mtime
+                                      for p in list(ORACLE_DIR.glob("*.[ch]")) + [ORACLE_DIR / "Makefile"])
+    if force or stale or not LIB_PATH.exists():
         subprocess.run(["make", "-C", str(ORACLE_DIR), "-B" if force else "-s", "liboracle.so"], check=True,
                        stdout=subprocess.DEVNULL)
     return LIB_PATH
 
 
+class RngOverrun(AssertionError):
+    """A replaying oracle rng was asked for more blocks than it was given."""
+
+
 class Rng(C.Structure):
+    """eo_rng (oracle/eg_oracle.h): a replaying rng keeps its state in the key bytes, so the layout is the same for both
+    forms; its size is checked against eo_rng_size() when the library is loaded."""
     _fields_ = [("key", C.c_uint8 * 32), ("block", C.c_uint64)]
 
 
@@ -79,6 +87,13 @@ def lib():
         _lib.eo_range_optimal.argtypes = [C.POINTER(Range), C.c_uint64]
         _lib.eo_rng_seed_from_u64.argtypes = [C.POINTER(Rng), C.c_uint64]
         _lib.eo_rng_from_seed.argtypes = [C.POINTER(Rng), C.c_char_p, C.c_uint64]
+        _lib.eo_rng_from_blocks.argtypes = [C.POINTER(Rng), C.c_void_p, C.c_uint64]
+        _lib.eo_rng_size.restype = C.c_size_t
+        _lib.eo_rng_overrun.argtypes = [C.POINTER(Rng)]
+        _lib.eo_rng_blocks_left.argtypes = [C.POINTER(Rng)]
+        _lib.eo_rng_blocks_left.restype = C.c_uint64
+        # a mirror that disagrees with the C struct would corrupt memory far from the cause
+        assert _lib.eo_rng_size() == C.sizeof(Rng), (_lib.eo_rng_size(), C.sizeof(Rng))
     return _lib
 
 
@@ -104,15 +119,38 @@ def rng_from_seed(seed32, first_block=0):
     return r
 
 
+def rng_from_blocks(blocks):
+    """An rng that replays `blocks` (a multiple of 64 bytes) in order, as the library's `wide_rand` form takes them; every
+    wrapper below raises RngOverrun once a prover has drawn past the end."""
+    blocks = bytes(blocks)
+    assert len(blocks) % 64 == 0
+    r = Rng()
+    r._blocks = C.create_string_buffer(blocks, len(blocks))       # kept alive with the rng
+    lib().eo_rng_from_blocks(C.byref(r), C.addressof(r._blocks), len(blocks) // 64)
+    return r
+
+
+def rng_blocks_left(rng):
+    """Blocks a replaying rng has not handed out yet."""
+    return lib().eo_rng_blocks_left(C.byref(rng))
+
+
+def _drawn(rng):
+    if lib().eo_rng_overrun(C.byref(rng)):
+        raise RngOverrun(f"a prover drew more than the {rng.block - 1} blocks of its replay")
+
+
 def rng_block(rng):
     out = buf(64)
     lib().eo_rng_block(C.byref(rng), out)
+    _drawn(rng)
     return raw(out)
 
 
 def keypair(rng):
     sk, pk = buf(32), buf(32)
     lib().eo_keypair_generate(C.byref(rng), sk, pk)
+    _drawn(rng)
     return raw(sk), raw(pk)
 
 
@@ -212,6 +250,7 @@ class MerlinTranscript:
 def encrypt(pk, value, rng):
     ct = buf(64)
     assert lib().eo_encrypt(pk, C.c_uint64(value), C.byref(rng), ct) == 0
+    _drawn(rng)
     return raw(ct)
 
 
@@ -224,6 +263,7 @@ def decrypt_to_element(sk, ct):
 def encrypt_zero(pk, rng):
     ct, proof = buf(64), buf(64)
     assert lib().eo_encrypt_zero(pk, C.byref(rng), ct, proof) == 0
+    _drawn(rng)
     return raw(ct), raw(proof)
 
 
@@ -234,6 +274,7 @@ def verify_zero(pk, ct, proof):
 def encrypt_bool(pk, value, rng):
     ct, proof = buf(64), buf(96)
     assert lib().eo_encrypt_bool(pk, int(value), C.byref(rng), ct, proof) == 0
+    _drawn(rng)
     return raw(ct), raw(proof)
 
 
@@ -246,6 +287,7 @@ def choice_new(pk, choices, single, rng):
     cts, ring, sm = buf(64 * n), buf(32 * (1 + 2 * n)), buf(64)
     flags = bytes(1 if c else 0 for c in choices)
     assert lib().eo_choice_new(pk, n, flags, int(single), C.byref(rng), cts, ring, sm) == 0
+    _drawn(rng)
     return raw(cts), raw(ring), (raw(sm) if single else None)
 
 
@@ -271,6 +313,7 @@ def range_prove(pk, rng_spec, label, value, rng):
     partial, ring = buf(max(1, 64 * (rng_spec.n_rings - 1))), buf(32 * (1 + total))
     assert lib().eo_range_prove(pk, C.byref(rng_spec), label.encode(), C.c_uint64(value), C.byref(rng), ct, r_out,
                                 partial, ring) == 0
+    _drawn(rng)
     return raw(ct), raw(partial)[:64 * (rng_spec.n_rings - 1)], raw(ring), raw(r_out)
 
 
@@ -283,6 +326,7 @@ def sumsq_prove(pk, cts, values, randomness, sum_ct, sum_randomness, label, rng)
     proof = buf(32 * (2 * n + 2))
     assert lib().eo_sumsq_prove(pk, n, b"".join(cts), b"".join(values), b"".join(randomness), sum_ct, sum_randomness,
                                 label.encode(), C.byref(rng), proof) == 0
+    _drawn(rng)
     return raw(proof)
 
 
@@ -304,6 +348,7 @@ def qv_new(pk, p, votes, rng):
     ballot = buf(qv_ballot_size(p))
     v = (C.c_uint64 * len(votes))(*votes)
     assert lib().eo_qv_new(pk, C.byref(p), v, C.byref(rng), ballot) == 0
+    _drawn(rng)
     return raw(ballot)
 
 
@@ -316,12 +361,14 @@ def dealer_new(shares, threshold, rng):
     secrets = buf(32 * shares)
     assert lib().eo_dealer_new(shares, threshold, C.byref(rng), C.byref(ks), secrets) == 0
     s = raw(secrets)
+    _drawn(rng)
     return ks, [s[32 * i:32 * i + 32] for i in range(shares)]
 
 
 def decrypt_share(ks, index, secret, ct, rng):
     share, proof = buf(32), buf(64)
     assert lib().eo_decrypt_share(C.byref(ks), index, secret, ct, C.byref(rng), share, proof) == 0
+    _drawn(rng)
     return raw(share), raw(proof)
 
 
@@ -332,6 +379,7 @@ def verify_share(ks, index, ct, share, proof):
 def decryption_prove(secret, label, ct, rng):
     dh, proof = buf(32), buf(64)
     assert lib().eo_decryption_prove(bytes(secret), label.encode(), bytes(ct), C.byref(rng), dh, proof) == 0
+    _drawn(rng)
     return raw(dh), raw(proof)
 
 
@@ -469,6 +517,7 @@ def commitment_equiv_prove(pk, value, blinding_base, label, rng):
     ct, commitment, proof, blinding = buf(64), buf(32), buf(128), buf(32)
     assert lib().eo_commitment_equiv_prove(pk, C.c_uint64(value), bytes(blinding_base), label.encode(), C.byref(rng), ct,
                                            commitment, proof, blinding) == 0
+    _drawn(rng)
     return raw(ct), raw(commitment), raw(proof), raw(blinding)
 
 
@@ -500,6 +549,7 @@ def pop_prove(secrets, keys, label, rng):
     k = len(keys)
     proof = buf(32 * (1 + k))
     assert lib().eo_pop_prove(k, b"".join(secrets), b"".join(keys), label.encode(), C.byref(rng), proof) == 0
+    _drawn(rng)
     return raw(proof)
 
 
