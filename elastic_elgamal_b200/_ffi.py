@@ -73,6 +73,9 @@ PROTOTYPES = {
     "eg_ciphertexts_sum_dev": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_size_t, P8, P8, P8]),
     "eg_ciphertexts_weighted_sum": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_size_t, C.c_size_t, P8, P8, P8, P8, P8]),
     "eg_ciphertexts_weighted_sum_dev": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_size_t, C.c_size_t, P8, P8, P8, P8, P8]),
+    "eg_ciphertexts_group_sum": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_size_t, C.c_size_t, P8, P8, C.c_uint32, P8, P8, P8]),
+    "eg_ciphertexts_group_sum_dev": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_size_t, C.c_size_t, P8, P8, C.c_uint32, P8, P8,
+                                                 P8]),
     "eg_verify_zero_batch": (C.c_int32, [C.c_void_p, C.c_size_t, P8, P8, P8]),
     "eg_verify_bool_batch": (C.c_int32, [C.c_void_p, C.c_size_t, P8, P8, P8]),
     "eg_verify_choice_batch": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_int, P8, P8, P8, P8, P8]),

@@ -45,6 +45,7 @@ template <class K> static cudaError_t cudaOccupancyMaxActiveBlocksPerMultiproces
 #include "../../include/eg_b200.h"
 #include "kernels.cuh"
 #include "weighted_sum.cuh"
+#include "group_sum.cuh"
 
 using namespace eg;
 
@@ -106,7 +107,8 @@ struct eg_ctx {
     std::vector<uint8_t> host_tally;        // child of a multi context: its partial tally, host copy
     uint32_t comm_bad = 0;                  // host copy of the combine kernel's flag (comm_combine / comm_check)
     bool comm_pending = false;
-    dev_buf ws[13];                         // scratch of eg_ciphertexts_weighted_sum (api_weighted_sum.inc)
+    dev_buf ws[13];                         // scratch of eg_ciphertexts_weighted_sum and _group_sum (api_weighted_sum.inc,
+                                            // api_group_sum.inc)
 };
 
 struct eg_dlog_table {
@@ -824,5 +826,7 @@ extern "C" eg_status eg_ctx_set_blinding_base(eg_ctx *ctx, const uint8_t base[32
 #include "api_sigma_provers.inc"
 
 #include "api_weighted_sum.inc"
+
+#include "api_group_sum.inc"
 
 #include "api_multi.inc"

@@ -48,6 +48,7 @@ struct ws_params {
     size_t n;                   // items of the chunk
     uint32_t cols;              // 2 n_cts
     uint32_t c, B, wmax, span, S;   // window bits, buckets per window (2^(c-1)), windows of a 253-bit scalar, spans per window
+                                    // (the group sum, group_sum.cuh: B = n_groups, wmax = 1)
     size_t lmax, cap;           // list capacity (wmax n), entries per column of each level buffer
     uint32_t *pts;              // planar Niels points: word w of column col of item i at (col * 24 + w) * n + i
     int32_t *digits;            // digit of window w of item i at w * n + i
@@ -61,9 +62,10 @@ struct ws_params {
     uint32_t *buckets;          // bucket key of column col at (col * wmax B + key) * 32
     uint32_t *rsum;             // per (column, window, span): 64 words (weighted sum, plain sum)
     uint32_t *wsum;             // per (column, window): 32 words
-    uint32_t *running;          // per column: 32 words, the total over the chunks so far
+    uint32_t *running;          // per column: 32 words, the total over the chunks so far (group sum: per group and column)
     uint32_t *ctl;              // [0] largest bit length of the chunk's included scalars, [1] list length
-    uint32_t *bad;              // a non-canonical scalar or an undecodable element in an included item (whole call)
+    uint32_t *bad;              // a non-canonical scalar or an undecodable element in an included item (whole call);
+                                // group sum: a group id out of range in an included item
 };
 
 EG_HD uint32_t ws_atomic_add(uint32_t *p, uint32_t v) {
@@ -124,18 +126,24 @@ EG_HD void ws_scalars_body(const ws_params &P, size_t i) {
     if (bits) ws_atomic_max(P.ctl, bits);
 }
 
-EG_HD void ws_decode_body(const ws_params &P, size_t i, uint32_t col) {
-    if (!ws_included(P, i)) return;
+// element col of item i into column col of P.pts; false (nothing stored) when it does not decode
+EG_HD bool ws_decode_niels(const ws_params &P, size_t i, uint32_t col) {
     uint32_t w[8];
     load32_bytes(w, P.cts + i * P.item_stride + (size_t)(col >> 1) * P.ct_stride + 32 * (col & 1));
     ge_ext p;
-    if (!ge_decode(p, w)) { ws_set_bad(P.bad); return; }
+    if (!ge_decode(p, w)) return false;
     fe t;                                           // Z = 1: (y + x, y - x, 2 d x y)
     uint32_t o[24];
     fe_add(t, p.Y, p.X); fe_towords(o, t);
     fe_sub(t, p.Y, p.X); fe_towords(o + 8, t);
     fe_mul(t, p.T, fe_const_2d()); fe_towords(o + 16, t);
     planar_store_words(P.pts, P.n, col, 24, i, o);
+    return true;
+}
+
+EG_HD void ws_decode_body(const ws_params &P, size_t i, uint32_t col) {
+    if (!ws_included(P, i)) return;
+    if (!ws_decode_niels(P, i, col)) ws_set_bad(P.bad);
 }
 
 // ------------------------------------------------------------------ 2. signed digits and histogram

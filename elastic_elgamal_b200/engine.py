@@ -244,7 +244,12 @@ class Engine:
             scalars = np.ascontiguousarray(scalars, dtype="<u8").view(np.uint8).reshape(-1, 8)
             scalars = np.concatenate([scalars, np.zeros((scalars.shape[0], 24), np.uint8)], axis=1)
         scalars = _u8(scalars, (-1, 32))
-        n = scalars.shape[0]
+        n_cts, item_stride, ct_stride, cts, verdicts = Engine._item_args(scalars.shape[0], cts, verdicts, ct_stride, n_cts)
+        return n_cts, item_stride, ct_stride, cts, scalars, verdicts
+
+    @staticmethod
+    def _item_args(n, cts, verdicts, ct_stride, n_cts):
+        """The (n_cts, item_stride, ct_stride) view of n items of ciphertexts, and the verdict mask (weighted_sum, group_sum)."""
         if ct_stride is None:
             cts = _u8(cts)
             n_cts = cts.shape[1] if cts.ndim == 3 else cts.shape[1] // 64
@@ -258,7 +263,20 @@ class Engine:
                 n_cts = (item_stride - 64) // ct_stride + 1
         if verdicts is not None:
             verdicts = _u8(verdicts, (n,))
-        return n_cts, item_stride, ct_stride, cts, scalars, verdicts
+        return n_cts, item_stride, ct_stride, cts, verdicts
+
+    def group_sum(self, cts, groups, n_groups, verdicts=None, ct_stride=None, n_cts=None):
+        """The tally fold per group: out[g] = sum of cts[i] over the items with groups[i] == g and verdicts[i] == 0 (every
+        item when verdicts is None), as (out (n_groups, n_cts, 64), ok (n_groups,) bool).  `cts`, `ct_stride` and `n_cts` as
+        in weighted_sum; `groups` holds one id below n_groups per item.  A group without included items is the identity
+        with ok True; a group with an undecodable included element is the identity with ok False."""
+        groups = np.ascontiguousarray(groups, dtype=np.uint32).reshape(-1)
+        n = groups.shape[0]
+        n_cts, item_stride, ct_stride, cts, verdicts = self._item_args(n, cts, verdicts, ct_stride, n_cts)
+        out, ok = np.empty((n_groups, n_cts, 64), np.uint8), np.zeros(n_groups, np.uint8)
+        self._check(self.lib.eg_ciphertexts_group_sum(self.h, n, n_cts, item_stride, ct_stride, _addr(cts), _addr(groups), n_groups,
+                                                      _addr(verdicts), _addr(out), _addr(ok)))
+        return out, ok.astype(bool)
 
     # ---- proofs
     def verify_zero(self, cts, proofs):
@@ -647,6 +665,10 @@ class Engine:
         idx = (C.c_uint32 * len(indexes))(*indexes)
         self._check(self.lib.eg_combine_decrypt_accepted_batch_dev(self.h, threshold, len(indexes), idx, n, d_cts, d_shares, d_verdicts,
                                                                    table.h, d_values, d_found))
+
+    def group_sum_dev(self, n, n_cts, item_stride, ct_stride, d_cts, d_groups, n_groups, d_verdicts, d_out, d_ok):
+        self._check(self.lib.eg_ciphertexts_group_sum_dev(self.h, n, n_cts, item_stride, ct_stride, d_cts, d_groups, n_groups, d_verdicts,
+                                                          d_out, d_ok))
 
     def verify_choice_dev(self, n, options, single, d_choices, d_rings, d_sums, d_verdicts, d_tally):
         self._check(self.lib.eg_verify_choice_batch_dev(self.h, n, options, int(single), d_choices, d_rings, d_sums,

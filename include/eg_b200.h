@@ -151,6 +151,24 @@ eg_status eg_ciphertexts_sum(eg_ctx *ctx, size_t n_parts, size_t n_cts, const ui
 eg_status eg_ciphertexts_weighted_sum(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
                                       const uint8_t *cts, const uint8_t *scalars /* n*32 */, const uint8_t *verdicts /* n or NULL */,
                                       uint8_t *out /* n_cts*64 */, uint8_t *ok /* 1 */);
+/* The tally fold of examples/voting.rs:200-203 (Ciphertext Add, src/encryption.rs:163) keyed by a group id per item (a
+ * precinct, district or question):  out[g][j] = sum of cts[i][j] over the included items i with groups[i] == g.
+ * Reading and masking are exactly those of eg_ciphertexts_weighted_sum: ciphertext j of item i is at
+ * cts + i*item_stride + j*ct_stride; item i is included when verdicts[i] == EG_V_OK, every item when verdicts is NULL;
+ * excluded items are neither decoded nor checked, their group ids included; n_cts and the strides follow the same rules.
+ * out = n_groups rows of n_cts ciphertexts (Ciphertext::to_bytes), row g at out + g*n_cts*64.  A group with no included
+ * item gets identity ciphertexts (Ciphertext::zero) and ok[g] = 1.  ok[g] = 0 when an included item of group g has an
+ * element that does not decode; out[g] is then the identity and the other groups are unaffected (unlike the weighted
+ * sum's call-wide ok; items a verifier accepted always decode).  A group id >= n_groups in an included item is
+ * EG_ERR_INVALID_ARG (found on the device; the outputs are then unspecified).  n_groups >= 1 and n_groups*n_cts <= 2^22,
+ * else EG_ERR_INVALID_ARG.  n = 0: identity everywhere, every ok = 1.  Needs no receiver key; time depends on the group
+ * ids and the mask, which are public.  Multi-device context: the batch is sharded, each device's n_groups*n_cts partial
+ * totals are added, and ok[g] is the AND over the devices.  With an attached communicator the call is NOT collective:
+ * the result covers this rank's items. */
+eg_status eg_ciphertexts_group_sum(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
+                                   const uint8_t *cts, const uint32_t *groups /* n */, uint32_t n_groups,
+                                   const uint8_t *verdicts /* n or NULL */, uint8_t *out /* n_groups*n_cts*64 */,
+                                   uint8_t *ok /* n_groups */);
 
 /* ---- wire format (src/serde.rs:19-80) ----------------------------------------------------------- */
 
@@ -581,6 +599,11 @@ eg_status eg_ciphertexts_sum_dev(eg_ctx *ctx, size_t n_parts, size_t n_cts, cons
 eg_status eg_ciphertexts_weighted_sum_dev(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
                                           const uint8_t *d_cts, const uint8_t *d_scalars, const uint8_t *d_verdicts,
                                           uint8_t *d_out, uint8_t *d_ok);
+/* eg_ciphertexts_group_sum on device pointers (single-device context only, EG_ERR_INVALID_ARG otherwise); synchronous,
+ * so that an out-of-range group id can be reported.  d_ok is n_groups device bytes. */
+eg_status eg_ciphertexts_group_sum_dev(eg_ctx *ctx, size_t n, uint32_t n_cts, size_t item_stride, size_t ct_stride,
+                                       const uint8_t *d_cts, const uint32_t *d_groups, uint32_t n_groups,
+                                       const uint8_t *d_verdicts, uint8_t *d_out, uint8_t *d_ok);
 
 /* ---- instrumentation --------------------------------------------------------------------------- */
 /* Number of kernels this context has launched since creation (bench.py's `gpu_launches`). */

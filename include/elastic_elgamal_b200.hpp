@@ -44,6 +44,9 @@ struct ChoiceParams { PublicKey receiver; uint32_t options_count; bool single; }
 struct EncryptedChoice { std::vector<Ciphertext> choices; RingProof range_proof; LogEqualityProof sum_proof; };
 
 struct ChoiceBatchResult { std::vector<Verdict> verdicts; std::vector<Ciphertext> tally; };
+// per group: n_cts totals, and ok = 0 when an included item of the group had an element that does not decode (its totals
+// are then the identity)
+struct GroupSums { std::vector<std::vector<Ciphertext>> totals; std::vector<uint8_t> ok; };
 // src/proofs/mul.rs:86-93
 struct SumOfSquaresProof { Scalar challenge; std::vector<Scalar> ciphertext_responses; Scalar sum_response; };
 // src/app/quadratic_voting.rs:205-217 (CiphertextWithRangeProof = ciphertext + range proof)
@@ -212,6 +215,28 @@ class Engine {
                                           verdicts.empty() ? nullptr : verdicts.data(), out.data(), &ok));
         if (!ok) throw Error(EG_ERR_INVALID_ARG, "malformed element or scalar in a weighted sum");
         return to_ciphertexts(out);
+    }
+
+    // The tally fold per group (src/encryption.rs:163): totals[g][j] = the sum of items[i][j] over the items with
+    // groups[i] == g whose verdict is 0 (every item when `verdicts` is empty).  Groups without included items are the
+    // identity.  A group id >= n_groups of an included item throws EG_ERR_INVALID_ARG.
+    GroupSums group_sum(const std::vector<std::vector<Ciphertext>> &items, const std::vector<uint32_t> &groups, uint32_t n_groups,
+                        const std::vector<uint8_t> &verdicts = {}) {
+        const size_t n = items.size(), n_cts = n ? items[0].size() : 1;
+        if (groups.size() != n || (!verdicts.empty() && verdicts.size() != n))
+            throw Error(EG_ERR_INVALID_ARG, "one group id and verdict per item");
+        std::vector<uint8_t> c, out(n_groups * n_cts * 64);
+        for (size_t i = 0; i < n; i++) {
+            if (items[i].size() != n_cts) throw Error(EG_ERR_INVALID_ARG, "items must have the same number of ciphertexts");
+            for (const auto &ct : items[i]) append(c, ct);
+        }
+        GroupSums r;
+        r.ok.resize(n_groups);
+        check(eg_ciphertexts_group_sum(ctx_, n, (uint32_t)n_cts, 64 * n_cts, 64, c.data(), groups.data(), n_groups,
+                                       verdicts.empty() ? nullptr : verdicts.data(), out.data(), r.ok.data()));
+        const std::vector<Ciphertext> all = to_ciphertexts(out);
+        for (size_t g = 0; g < n_groups; g++) r.totals.emplace_back(all.begin() + g * n_cts, all.begin() + (g + 1) * n_cts);
+        return r;
     }
 
     ChoiceBatchResult verify_qv_batch(uint32_t options, uint64_t credits, const std::vector<QuadraticVotingBallot> &ballots) {

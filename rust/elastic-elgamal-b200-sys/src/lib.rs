@@ -159,6 +159,10 @@ extern "C" {
                                        scalars: *const u8, verdicts: *const u8, out: *mut u8, ok: *mut u8) -> eg_status;
     pub fn eg_ciphertexts_weighted_sum_dev(ctx: *mut eg_ctx, n: usize, n_cts: u32, item_stride: usize, ct_stride: usize, d_cts: *const u8,
                                            d_scalars: *const u8, d_verdicts: *const u8, d_out: *mut u8, d_ok: *mut u8) -> eg_status;
+    pub fn eg_ciphertexts_group_sum(ctx: *mut eg_ctx, n: usize, n_cts: u32, item_stride: usize, ct_stride: usize, cts: *const u8,
+                                    groups: *const u32, n_groups: u32, verdicts: *const u8, out: *mut u8, ok: *mut u8) -> eg_status;
+    pub fn eg_ciphertexts_group_sum_dev(ctx: *mut eg_ctx, n: usize, n_cts: u32, item_stride: usize, ct_stride: usize, d_cts: *const u8,
+                                        d_groups: *const u32, n_groups: u32, d_verdicts: *const u8, d_out: *mut u8, d_ok: *mut u8) -> eg_status;
 
     pub fn eg_base64url_chars(bytes_per_item: usize) -> usize;
     pub fn eg_base64url_decode_batch(ctx: *mut eg_ctx, n: usize, bytes_per_item: usize, text: *const c_char, raw: *mut u8,

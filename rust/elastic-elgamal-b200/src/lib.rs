@@ -835,6 +835,31 @@ impl Engine {
         Ok(ciphertexts(&out))
     }
 
+    /// The tally fold per group (encryption.rs:163): `totals[g][j]` is the sum of `items[i][j]` over the items with
+    /// `groups[i] == g` whose verdict is 0 (every item with `None`), e.g. per-precinct tallies under the verdicts of
+    /// `verify_choices`.  Groups without included items are `Ciphertext::zero()`.  Every item has the same number of
+    /// ciphertexts (1..=64); `n_groups * n_cts <= 2^22`; a group id `>= n_groups` of an included item is an error.
+    pub fn group_sum(&self, items: &[Vec<Ciphertext<Ristretto>>], groups: &[u32], n_groups: u32, verdicts: Option<&[u8]>) -> Result<Vec<Vec<Ciphertext<Ristretto>>>, EngineError> {
+        let n = items.len();
+        assert!(groups.len() == n && verdicts.map_or(true, |v| v.len() == n), "one group id and verdict per item");
+        let n_cts = items.first().map_or(1, |r| r.len());
+        let mut c = Vec::with_capacity(n * n_cts * 64);
+        for row in items {
+            assert!(row.len() == n_cts, "items must have the same number of ciphertexts");
+            for ct in row {
+                c.extend_from_slice(&ct.to_bytes());
+            }
+        }
+        let (mut out, mut ok) = (vec![0_u8; n_groups as usize * n_cts * 64], vec![0_u8; n_groups as usize]);
+        let v = verdicts.map_or(std::ptr::null(), |v| v.as_ptr());
+        self.check(unsafe {
+            sys::eg_ciphertexts_group_sum(self.ctx, n, n_cts as u32, 64 * n_cts, 64, c.as_ptr(), groups.as_ptr(), n_groups, v, out.as_mut_ptr(),
+                                          ok.as_mut_ptr())
+        })?;
+        debug_assert!(ok.iter().all(|&o| o == 1), "typed inputs decode");
+        Ok(out.chunks(n_cts * 64).map(ciphertexts).collect())
+    }
+
     // ------------------------------------------------------------------ creation side
 
     /// `key.encrypt(value, rng)` over a batch (keys/impls.rs:16-23).
